@@ -5,6 +5,7 @@ demodulated Msamples/s summed over all channels, and % of the HBM roofline.
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                     (the reference's own C chain on the host cores)
   python bench.py --config c3|c4|c5 ...                    (default c3, the single-GPU configuration BASELINE names)
+  python bench.py ... --dump-outputs DIR                   (also write the last timed step's audio, sampled, to DIR/audio.npy)
 
 Workloads (minimal-sdr_b200/workloads.py):
   c3  4096 channels x 10 s at 44.1 kHz per GPU (3446 blocks of 128 samples), mode = {AM, USB, LSB, CW}[c mod 4], the sketch's FIR
@@ -33,6 +34,7 @@ import numpy as np  # noqa: E402
 
 BLOCK = 128
 ALGO_BYTES_PER_SAMPLE = 4  # 2 B int16 IF in + 2 B int16 audio out (SURVEY.md 8d)
+DUMP_BYTES = 64_000_000  # --dump-outputs: upper bound of the float32 sample it writes
 LATENCY_BOUND_CYCLES = 18.0  # loop-carried latency of one biquad stage: IMAD.HI 9 + SHF 4 + I2IP 4 (+1), profiles/r01_microbench_lat.txt
 ISSUE_BOUND_CYCLES = 43.5    # a whole stage in one warp, isolated (tools/microbench/bqstep2.cu)
 
@@ -270,6 +272,19 @@ def parity_check(m, w, make_chain, C, ch0, dev_calls, n_updates=2):
             "mismatches": mism, "checker": "oracle/_ref (reference sources)" if lib.prefix == "ref" else "oracle port"}
 
 
+def output_sample(m, dev_calls, C, L):
+    """The audio the timed path left in its output buffers (the last step, every update in stream order) for a fixed, seeded set of
+    channels, gathered on the device right after the timed steps: (int16 [channels, samples] on the device, channel indices).
+    It takes as many whole channels as fit in DUMP_BYTES as float32. If even the fixed edge channels of sample_channels do not fit,
+    it keeps only their leading samples."""
+    import torch
+    chans = m.workloads.sample_channels(C, want=max(1, DUMP_BYTES // (4 * L)))
+    cols = min(L, DUMP_BYTES // (4 * len(chans)))
+    idx = torch.tensor(chans, device=dev_calls[0][1].device)
+    y = torch.cat([yout[idx, :nb * BLOCK] for _, yout, nb, _ in dev_calls], dim=1)
+    return y[:, :cols].clone(), chans
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -293,7 +308,14 @@ def main():
     ap.add_argument("--layout", choices=["updates", "rows"], default="updates",
                     help="device-resident input layout: 'updates' = one contiguous [channels][samples] batch per update (how a streaming "
                          "receiver holds its block batches), 'rows' = one row per channel for the whole step, updates are column windows of it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the audio the last timed step computed as DIR/audio.npy (float32 [channels, samples]: a fixed, "
+                         "seeded sample of rank 0's channels, at most 64 MB) so that two builds can be compared output for output. Where a step "
+                         "alternates two output batches over more updates (c5), every update gets its own output buffer instead, so that the "
+                         "whole step survives: more device memory, and the JSON line's dump_outputs entry says how much")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -353,10 +375,13 @@ def main():
         x = m.synth.torch_batch(C, L, dev, w.fs, ch0=ch0)
         y = torch.empty_like(x)
         dev_calls = [(x[:, b0 * BLOCK:], y[:, b0 * BLOCK:], nb, x.stride(0)) for b0, nb in updates]
+        dump_buffers = {"output_buffers": 1, "without_dump": 1, "extra_bytes": 0}
     else:  # one contiguous batch per update; same samples, same order of processing
         xs = [m.synth.torch_batch(C, nb * BLOCK, dev, w.fs, ch0=ch0, n0=b0 * BLOCK) for b0, nb in updates[:n_bufs]]
-        ys = [torch.empty_like(t) for t in xs]
-        dev_calls = [(xs[i % n_bufs], ys[i % n_bufs], nb, xs[i % n_bufs].stride(0)) for i, (b0, nb) in enumerate(updates)]
+        n_out = len(updates) if args.dump_outputs else n_bufs  # the dump needs every update's audio of the last step
+        ys = [torch.empty_like(xs[i % n_bufs]) for i in range(n_out)]
+        dump_buffers = {"output_buffers": n_out, "without_dump": n_bufs, "extra_bytes": sum(t.nbytes for t in ys[n_bufs:])}
+        dev_calls = [(xs[i % n_bufs], ys[i % n_out], nb, xs[i % n_bufs].stride(0)) for i, (b0, nb) in enumerate(updates)]
     calls = [(a.data_ptr(), b.data_ptr(), nb, st) for a, b, nb, st in dev_calls]
     torch.cuda.synchronize()
 
@@ -425,6 +450,8 @@ def main():
     barrier()
     clocks.t1 = time.time()
     torch.cuda.profiler.stop()
+    # before the cool-down steps and the parity check write the output buffers again
+    dump = output_sample(m, dev_calls, C, L) if args.dump_outputs and rank == 0 else None
     ms_local = e0.elapsed_time(e1)
     launches = g.launch_count() - l0 + ((fe.launch_count() - fe_l0) if fe is not None else 0)
     if clocks.t1 - clocks.t0 < 0.5:  # untimed cool-down under the same load so that the clock sampler sees it
@@ -580,6 +607,13 @@ def main():
         if world == 1 and not args.no_cpu:
             cb = time_cpu(m, w)
             line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "build", "builds", "sample")}
+        if dump is not None:
+            audio, chans = dump
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "audio.npy"), audio.cpu().numpy().astype(np.float32))
+            line["dump_outputs"] = {"dir": args.dump_outputs, "audio": list(audio.shape), "channels": len(chans),
+                                    "what": "int16 audio of the last timed step as float32; channels of workloads.sample_channels, leading samples of each",
+                                    "timed_path": dump_buffers}
         print(json.dumps(line), flush=True)
     g.close()
     if world > 1:

@@ -66,11 +66,33 @@ def test_numa_helper_parsing(msdr):
     assert info["bound"] is False
 
 
+def test_dump_sample_is_the_last_step_in_stream_order(msdr, monkeypatch):
+    """bench.py --dump-outputs: sampled rows of every update's output buffer, in stream order, within DUMP_BYTES as float32."""
+    import torch
+    import bench
+    C, ups = 300, [4, 4, 2]
+    L = sum(ups) * 128
+    ys = [torch.randint(-32768, 32768, (C, nb * 128 + 128), dtype=torch.int16) for nb in ups]  # a buffer may outsize its update
+    calls = [(None, y, nb, y.stride(0)) for y, nb in zip(ys, ups)]
+    full = torch.cat([y[:, :nb * 128] for y, nb in zip(ys, ups)], dim=1)
+    shapes = []
+    for budget in (64_000_000, 4 * L * 40, 4 * L * 2):  # every channel; 40 whole rows; the fixed edge channels, leading samples only
+        monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+        got, chans = bench.output_sample(msdr, calls, C, L)
+        assert chans == msdr.workloads.sample_channels(C, want=max(1, budget // (4 * L)))
+        assert 4 * got.numel() <= budget and torch.equal(got, full[chans, :got.shape[1]])
+        shapes.append(tuple(got.shape))
+    assert shapes[0] == (C, L) and shapes[1] == (40, L) and 20 < shapes[2][0] < 40 and shapes[2][1] < L
+
+
 def test_reference_arm_line_says_what_ran():
+    import oracle_lib as ol
+    # the reference's own sources where they were built (oracle/_ref), else the oracle port of them
+    build, kind = ("gcc -O2", "reference") if ol.have_ref() else ("gcc -O2 (oracle port)", "port")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0", "--config", "c4"],
                        capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     d = json.loads(r.stdout.strip().splitlines()[-1])
     assert d["impl"] == "reference" and d["value"] > 0 and d["config"]["config"] == "c4"
     assert "reference arm:" in d["config"]["ran"] and "256-tap" in d["config"]["ran"]
-    assert set(d["cpu_baseline"]["builds"]) >= {"gcc -O2"} and d["e2e"]["h2d_bytes_per_step"] == 0
+    assert set(d["cpu_baseline"]["builds"]) >= {build} and d["cpu_baseline"]["kind"] == kind and d["e2e"]["h2d_bytes_per_step"] == 0
