@@ -243,6 +243,26 @@ uint64_t msdr_frontend_launch_count(const msdr_frontend *fe);
 int msdr_frontend_set_option(msdr_frontend *fe, const char *key, int value);
 /* AudioAmplifier::gain (mixer.h:75-79): clamp to +-32767, multiplier = (int32_t)(gain * 65536.0f) */
 int32_t msdr_amp_gain_multiplier(float gain);
+
+/* ---- receive chain from raw ADC codes: the front end above per channel of a chain, in front of it ------------------------------
+ * adc1 -> amp_adc -> queue_adc -> demodulation() with AGC(p_adc) on every block (Minimal-SDR.ino:76-78,445-515) as one object.
+ * Output, chain state and front-end state equal msdr_frontend_update followed by msdr_chain_update with the same parameters, however
+ * a stream is cut into updates.  The FIR history holds conditioned IF samples in both input formats, so int16 and ADC updates may be
+ * interleaved on one chain; an int16 update leaves the front-end state alone.  Buffer, alignment and stride rules are those of
+ * msdr_chain_update / msdr_chain_update_device.  msdr_chain_last_kernel names the path: the front end fused into the converters of
+ * the many-channel row-block kernels, or the front-end kernel over the range followed by the int16 path. */
+/* (Re)initialise the per-channel front end of every channel of the chain, like msdr_frontend_create:
+   hpf 0, agc_idx 25, agc_val = agc_start, multiplier = gain(agc_start). */
+int msdr_chain_enable_frontend(msdr_chain *chain, float agc_start, float agc_max, int agc_on);
+int msdr_chain_frontend_preset(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint16_t first_reading); /* input_adc.cpp:59-63 */
+/* MSDR_ERR_NOT_INITIALISED before msdr_chain_enable_frontend */
+int msdr_chain_update_adc(msdr_chain *chain, const uint16_t *adc, int16_t *out, uint32_t n_blocks, size_t stride);  /* host buffers */
+int msdr_chain_update_adc_device(msdr_chain *chain, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks, size_t stride);
+int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint16_t *d_adc, int16_t *d_out,
+                                       uint32_t n_blocks, size_t stride);
+/* agc_idx outside [0, 25] is MSDR_ERR_ARGUMENT */
+int msdr_chain_get_frontend_state(msdr_chain *chain, uint32_t ch, msdr_frontend_state *out);
+int msdr_chain_set_frontend_state(msdr_chain *chain, uint32_t ch, const msdr_frontend_state *in);
 /* AudioAmplifier::update / applyGain (mixer.cpp:34-47,134-159) in place on host rows: SSAT16((multipliers[row] * x) >> 16).
  * Multiplier 65536 leaves the data unchanged and 0 gives zeros (the reference transmits no block at all for 0). */
 int msdr_op_amplifier(int device, const int32_t *multipliers, int16_t *data, uint32_t rows, uint32_t n, size_t stride);

@@ -568,6 +568,23 @@ public:
   }
   // many blocks at once on caller buffers [channels][stride]
   int update(const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride) { return status_ = msdr_chain_update(chain_, in, out, n_blocks, stride); }
+  // adc1 -> amp_adc -> queue_adc -> demodulation() with AGC(p_adc) on every block (Minimal-SDR.ino:76-78,445-515) in this one object:
+  // begin_frontend() sets up every channel's DC block, amplifier and AGC (AGC_start, AGC_Max, AGC_on of .ino:94-100), update_adc()
+  // takes raw uint16 ADC codes [channels][stride] and returns audio, AGC_val(ch) is the sketch's global of that channel
+  int begin_frontend(float agc_start = 0.25f, float agc_max = 40.0f, int agc_on = 1)
+  {
+    return status_ = msdr_chain_enable_frontend(chain_, agc_start, agc_max, agc_on);
+  }
+  int update_adc(const uint16_t *codes, int16_t *out, uint32_t n_blocks, size_t stride)
+  {
+    return status_ = msdr_chain_update_adc(chain_, codes, out, n_blocks, stride);
+  }
+  float AGC_val(uint32_t ch)
+  {
+    msdr_frontend_state s{};
+    status_ = msdr_chain_get_frontend_state(chain_, ch, &s);
+    return s.agc_val;
+  }
   uint32_t channels() const { return n_; }
 private:
   uint32_t cnt(uint32_t ch0, uint32_t nch) const { return nch == ~0u ? n_ - ch0 : nch; }

@@ -103,6 +103,13 @@ SYMBOLS = {
     "msdr_frontend_set_state": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(FrontendState)]),
     "msdr_frontend_launch_count": (C.c_uint64, [C.c_void_p]),
     "msdr_frontend_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int]),
+    "msdr_chain_enable_frontend": (C.c_int, [C.c_void_p, C.c_float, C.c_float, C.c_int]),
+    "msdr_chain_frontend_preset": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint16]),
+    "msdr_chain_update_adc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_update_adc_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_update_adc_range_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_get_frontend_state": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(FrontendState)]),
+    "msdr_chain_set_frontend_state": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(FrontendState)]),
     "msdr_amp_gain_multiplier": (C.c_int32, [C.c_float]),
     "msdr_op_dac_codes": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t]),
     "msdr_op_amplifier": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t]),

@@ -183,6 +183,45 @@ class ReceiveChain:
         return self._ck(self._L.msdr_chain_update_range_device(self.h, int(ch0), int(nch), C.c_void_p(int(d_in)), C.c_void_p(int(d_out)),
                                                                int(n_blocks), int(stride)))
 
+    # -- raw ADC codes in: the front end (frontend.Frontend) per channel in front of the chain -----------------------------------
+    def enable_frontend(self, agc_start=0.25, agc_max=40.0, agc_on=True):
+        """(Re)initialise every channel's front end like frontend.Frontend(...): DC-block state 0, AGC at agc_start."""
+        return self._ck(self._L.msdr_chain_enable_frontend(self.h, float(agc_start), float(agc_max), int(bool(agc_on))))
+
+    def frontend_preset(self, first_reading, ch0=0, nch=None):
+        """AudioInputAnalog::init: hpf_x1 = first ADC reading << 14, hpf_y1 = 0 (input_adc.cpp:59-63)."""
+        ch0, nch = self._rng(ch0, nch)
+        return self._ck(self._L.msdr_chain_frontend_preset(self.h, ch0, nch, int(first_reading)))
+
+    def update_adc(self, adc, out=None):
+        """adc: uint16 raw codes [n_channels, n_blocks*128] in HOST memory -> audio, as frontend.Frontend.update then update()."""
+        adc = np.asarray(adc)
+        assert adc.dtype == np.uint16 and adc.ndim == 2 and adc.shape[0] == self.n_channels and adc.shape[1] % capi.BLOCK == 0
+        assert adc.strides[1] == 2 and adc.strides[0] % 2 == 0
+        if out is None:
+            out = np.empty((self.n_channels, adc.shape[1]), np.int16)
+        assert out.dtype == np.int16 and out.shape == adc.shape and out.strides[1] == 2
+        assert out.strides[0] == adc.strides[0], "in/out must share the row stride"
+        self._ck(self._L.msdr_chain_update_adc(self.h, capi.ptr(adc), capi.ptr(out), adc.shape[1] // capi.BLOCK, adc.strides[0] // 2))
+        return out
+
+    def update_adc_device(self, d_adc, d_out, n_blocks, stride):
+        """Device pointers (ints), asynchronous on the chain's stream."""
+        return self._ck(self._L.msdr_chain_update_adc_device(self.h, C.c_void_p(int(d_adc)), C.c_void_p(int(d_out)), int(n_blocks), int(stride)))
+
+    def update_adc_range_device(self, ch0, nch, d_adc, d_out, n_blocks, stride):
+        """Only channels [ch0, ch0+nch); the buffers hold nch rows."""
+        return self._ck(self._L.msdr_chain_update_adc_range_device(self.h, int(ch0), int(nch), C.c_void_p(int(d_adc)), C.c_void_p(int(d_out)),
+                                                                   int(n_blocks), int(stride)))
+
+    def get_frontend_state(self, ch):
+        st = capi.FrontendState()
+        self._ck(self._L.msdr_chain_get_frontend_state(self.h, int(ch), C.byref(st)))
+        return st
+
+    def set_frontend_state(self, ch, st):
+        return self._ck(self._L.msdr_chain_set_frontend_state(self.h, int(ch), C.byref(st)))
+
     def synchronize(self):
         return self._ck(self._L.msdr_chain_synchronize(self.h))
 

@@ -1,6 +1,7 @@
 // msdr_capi.cu — the C ABI declared in include/msdr.h: chain object, configuration, updates, stage operators.
 // Host-side only plumbing; every computation is a CUDA kernel from msdr_chain_kernel.cu / msdr_stage_kernels.cu.
 #include "../../include/msdr.h"
+#include "msdr_frontend.cuh"
 #include "msdr_internal.h"
 
 #include <algorithm>
@@ -144,6 +145,14 @@ struct msdr_chain {
   } pll;
 
   int16_t *d_set_taps = nullptr;     // [MSDR_MAX_FIR_SETS][2][MSDR_MAX_TAPS] every live table's raw taps (the side lane's FIR launches read them)
+  // ADC-code input (msdr_chain_enable_frontend): per-channel front end, and the conditioned IF samples of the composed path
+  fe::State *d_fe = nullptr;         // [C]
+  float fe_agc_start = 0.25f, fe_agc_max = 40.0f;
+  int fe_agc_on = 1;
+  int16_t *d_fe_if = nullptr;        // [rows][stride] of the largest composed update so far
+  size_t fe_if_samples = 0;
+  bool fe_composed = false;          // the last ADC update ran K4, then the int16 path
+
   int variant = 0;
   uint32_t host_chunk_channels = 0, host_chunk_blocks = 0; // 0 = auto
   uint32_t spare_sms = 0;
@@ -340,6 +349,7 @@ void msdr_chain_destroy(msdr_chain *chain)
   cudaFree(chain->pll.d_If); cudaFree(chain->pll.d_Qf); cudaFree(chain->pll.d_taps); cudaFree(chain->pll.d_defs);
   cudaFree(chain->d_sets); cudaFree(chain->d_set_kp4); cudaFree(chain->d_set_taps); cudaFree(chain->d_ctrl); cudaFree(chain->d_tile_flags);
   cudaFree(chain->d_in); cudaFree(chain->d_out);
+  cudaFree(chain->d_fe); cudaFree(chain->d_fe_if);
   if (chain->pin_in) cudaFreeHost(chain->pin_in);
   if (chain->pin_out) cudaFreeHost(chain->pin_out);
   for (cudaEvent_t ev : chain->pipe_ev) cudaEventDestroy(ev);
@@ -732,6 +742,27 @@ namespace {
 //                             -> demodulation switch or PLL (state per chain channel) -> LMS where it is on
 //                             -> biquad object 1, 2 -> scatter audio and biquad words back
 // The raw-sample history is the fused kernel's to update; it is correct for every channel.
+// every chain channel that the side lane serves, ascending (one scan per configuration change, not per update)
+const std::vector<uint32_t> &side_lane_channels(msdr_chain *chain)
+{
+  msdr_chain::PllLane &ln = chain->pll;
+  if (ln.dirty) {
+    const bool pll_build = !(chain->flags & MSDR_FLAG_AM_Q31);
+    ln.channels.clear();
+    for (uint32_t c = 0; c < chain->C; ++c)
+      if ((pll_build && chain->h_mode[c] == MSDR_MODE_SYNCAM) || (chain->n_anr && chain->h_anr[c] != 0)) ln.channels.push_back(c);
+    ln.dirty = false;
+  }
+  return ln.channels;
+}
+
+bool side_lane_in_range(msdr_chain *chain, uint32_t ch0, uint32_t nch)
+{
+  const std::vector<uint32_t> &ch = side_lane_channels(chain);
+  const auto it = std::lower_bound(ch.begin(), ch.end(), ch0);
+  return it != ch.end() && *it < ch0 + nch;
+}
+
 int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, size_t stride, uint32_t L)
 {
   msdr_chain::PllLane &ln = chain->pll;
@@ -742,12 +773,7 @@ int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int
   if (!hit) {
     ln.rows.clear();
     ln.any_pll = ln.any_anr = false;
-    if (ln.dirty) { // one scan per configuration change, not per update
-      ln.channels.clear();
-      for (uint32_t c = 0; c < chain->C; ++c)
-        if ((pll_build && chain->h_mode[c] == MSDR_MODE_SYNCAM) || (chain->n_anr && chain->h_anr[c] != 0)) ln.channels.push_back(c);
-      ln.dirty = false;
-    }
+    side_lane_channels(chain);
     for (auto it = std::lower_bound(ln.channels.begin(), ln.channels.end(), ch0); it != ln.channels.end() && *it < ch0 + nch; ++it) {
       const uint32_t r = *it - ch0;
       const bool is_pll = pll_build && chain->h_mode[ch0 + r] == MSDR_MODE_SYNCAM;
@@ -829,20 +855,22 @@ int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, int16_t *d_out, size_t s
   return MSDR_OK;
 }
 
-} // namespace
-
-int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
-                                   size_t stride)
+// d_adc != NULL: the rows are raw ADC codes for the chain's front end.  Where the int16 input would run the row-block kernels and no
+// channel of the range is on the side lane (which gathers IF samples from `d_in`), the front end runs inside their converters; in
+// every other case K4 conditions the range into a scratch buffer first and the int16 path follows.  Both are bit-exact.
+int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks, size_t stride,
+                 const uint16_t *d_adc)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
   if (n_blocks == 0 || nch == 0) return MSDR_OK;
   const uint64_t L64 = (uint64_t)n_blocks * MSDR_BLOCK_SAMPLES;
   if (!range_ok(chain, ch0, nch)) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad channel range");
-  if (!d_in || !d_out || L64 > stride || L64 > 0x7FFFFF00ull) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
-  if (((uintptr_t)d_in & 15u) || ((uintptr_t)d_out & 15u) || (stride & 7u))
+  const void *src_rows = d_adc ? static_cast<const void *>(d_adc) : static_cast<const void *>(d_in);
+  if (!src_rows || !d_out || L64 > stride || L64 > 0x7FFFFF00ull) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
+  if (((uintptr_t)src_rows & 15u) || ((uintptr_t)d_out & 15u) || (stride & 7u))
     return fail(chain, MSDR_ERR_ARGUMENT, "update_device: buffers must be 16-byte aligned and stride a multiple of 8 samples");
   if (chain->n_uninit) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update: some channels have no FIR bound (call msdr_fir_init_q15)");
   CK(cudaSetDevice(chain->device));
+  chain->fe_composed = false;
 
   ChainParams p{};
   p.in = d_in; p.out = d_out; p.stride = stride;
@@ -869,7 +897,28 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
   p.tile_flags = chain->d_tile_flags;
   p.epoch = ++chain->epoch;
   CK(cudaMemsetAsync(chain->d_ctrl, 0, (size_t)(1 + NG) * sizeof(int), chain->stream));
+  // ADC codes outside the fused path: K4 over the range into the scratch rows (same stride as `d_out`), then the int16 path reads them
+  auto compose = [&]() -> int {
+    const size_t need = (size_t)nch * stride;
+    if (need > chain->fe_if_samples) {
+      CK(cudaStreamSynchronize(chain->stream));
+      cudaFree(chain->d_fe_if);
+      chain->d_fe_if = nullptr; chain->fe_if_samples = 0;
+      CK(cudaMalloc(&chain->d_fe_if, need * sizeof(int16_t)));
+      chain->fe_if_samples = need;
+    }
+    CK(launch_frontend(d_adc, chain->d_fe_if, stride, nch, n_blocks, chain->d_fe + ch0, chain->fe_agc_max, chain->fe_agc_on, 0, chain->stream));
+    chain->launches++;
+    d_in = chain->d_fe_if; p.in = d_in;
+    d_adc = nullptr;
+    chain->fe_composed = true;
+    return MSDR_OK;
+  };
   bool use_tc = (chain->variant & 64) == 0; // variant bit 6: force the CUDA-core FIR kernel (msdr_chain_v3.cu)
+  if (d_adc && !use_tc) {
+    const int stc = compose();
+    if (stc != MSDR_OK) return stc;
+  }
   if (use_tc) { // tensor-core FIR producers (msdr_chain_v4.cu)
     int sms = 0;
     CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, chain->device));
@@ -905,6 +954,14 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
       p.tc_rowmap = pl.d_rowmap; p.tc_rb = pl.d_rb; p.tc_grp = pl.d_grp; p.tc_wave_rb0 = pl.d_wave_rb0; p.tc_bmat = pl.d_bmat;
       const bool long_window = !pl.ring_v5 || ((chain->variant & 32768) && pl.ring_v5l); // 256 taps: the half-tile form (bit 15: study, any window)
       p.tc_K = pl.K; p.tc_ring = long_window ? pl.ring_v5l : pl.ring_v5;
+      if (d_adc && side_lane_in_range(chain, ch0, nch)) {
+        const int stc = compose();
+        if (stc != MSDR_OK) return stc;
+      }
+      if (d_adc) { // fused: the converters read codes and condition them (msdr_chain_v5_common.cuh: FeRow)
+        p.in = reinterpret_cast<const int16_t *>(d_adc);
+        p.fe = chain->d_fe; p.agc_max = chain->fe_agc_max; p.agc_on = chain->fe_agc_on ? 1u : 0u;
+      }
       if (chain->timed) {
         int stu = usage_resolve(chain);
         if (stu != MSDR_OK) return stu;
@@ -928,6 +985,7 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
         CK(launch_chain_v5(p, chain->stream, chain->variant, sms, &chain->last_info));
         chain->last_kernel = "msdr::v5::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; one CTA per 128-channel row block)";
       }
+      if (p.fe) chain->last_kernel += "; front end fused into the converters";
       {
         int stl = syncam_lane_finish(chain, ch0, d_out, stride, p.L);
         if (stl != MSDR_OK) return stl;
@@ -954,6 +1012,10 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
         }
       }
       return MSDR_OK;
+    }
+    if (d_adc) {
+      const int stc = compose();
+      if (stc != MSDR_OK) return stc;
     }
     st = build_tc_plan(chain, ch0, nch, (uint32_t)sms, want_dual, &plp);
     if (st != MSDR_OK) return st;
@@ -1104,18 +1166,28 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
   return MSDR_OK;
 }
 
+} // namespace
+
+int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
+                                   size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  return update_range(chain, ch0, nch, d_in, d_out, n_blocks, stride, nullptr);
+}
+
 int msdr_chain_update_device(msdr_chain *chain, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks, size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   return msdr_chain_update_range_device(chain, 0, chain->C, d_in, d_out, n_blocks, stride);
 }
 
+namespace {
+
 // Host buffers: channels are cut into chunks that flow through a 3-slot device ring — H2D copy (stream copy_in),
 // fused kernel (chain stream), D2H copy (stream copy_out) — so PCIe traffic in both directions overlaps the kernels.
-int msdr_chain_update(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride)
+// adc: `in` holds uint16 ADC codes (2 bytes a sample like int16 IF samples) for the chain's front end.
+int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride, bool adc)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if (n_blocks == 0) return MSDR_OK;
   const size_t L = (size_t)n_blocks * MSDR_BLOCK_SAMPLES;
   if (!in || !out || L > stride) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
   if (chain->n_uninit) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update: some channels have no FIR bound (call msdr_fir_init_q15)");
@@ -1161,7 +1233,8 @@ int msdr_chain_update(msdr_chain *chain, const int16_t *in, int16_t *out, uint32
       CK(cudaMemcpy2DAsync(din, Lc * 2, in + hoff, stride * 2, w, nc, cudaMemcpyHostToDevice, chain->copy_in));
       CK(cudaEventRecord(ev_h2d[slot], chain->copy_in));
       CK(cudaStreamWaitEvent(chain->stream, ev_h2d[slot], 0));
-      st = msdr_chain_update_range_device(chain, c0, nc, din, dout, nb, Lc);
+      st = adc ? msdr_chain_update_adc_range_device(chain, c0, nc, reinterpret_cast<const uint16_t *>(din), dout, nb, Lc)
+               : msdr_chain_update_range_device(chain, c0, nc, din, dout, nb, Lc);
       if (st != MSDR_OK) return st;
       CK(cudaEventRecord(ev_k[slot], chain->stream));
       CK(cudaStreamWaitEvent(chain->copy_out, ev_k[slot], 0));
@@ -1171,6 +1244,98 @@ int msdr_chain_update(msdr_chain *chain, const int16_t *in, int16_t *out, uint32
   }
   CK(cudaStreamSynchronize(chain->copy_out));
   CK(cudaStreamSynchronize(chain->stream));
+  return MSDR_OK;
+}
+
+} // namespace
+
+int msdr_chain_update(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (n_blocks == 0) return MSDR_OK;
+  return host_pipeline(chain, in, out, n_blocks, stride, false);
+}
+
+// ---- ADC-code input: the front end of msdr_frontend.cu per chain channel, in front of the chain ------------------------------------
+int msdr_chain_enable_frontend(msdr_chain *chain, float agc_start, float agc_max, int agc_on)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  CK(cudaSetDevice(chain->device));
+  CK(cudaStreamSynchronize(chain->stream));
+  if (!chain->d_fe) CK(cudaMalloc(&chain->d_fe, (size_t)chain->C * sizeof(fe::State)));
+  chain->fe_agc_start = agc_start; chain->fe_agc_max = agc_max; chain->fe_agc_on = agc_on ? 1 : 0;
+  fe::State s{};
+  s.agc_idx = fe::kAgcBuf;                // .ino:451
+  s.agc_val = agc_start;                  // .ino:104
+  s.mult = fe::amp_multiplier(agc_start); // .ino:385
+  std::vector<fe::State> h(chain->C, s);
+  CK(cudaMemcpy(chain->d_fe, h.data(), h.size() * sizeof(fe::State), cudaMemcpyHostToDevice));
+  CK(cudaDeviceSynchronize()); // legacy-stream copy vs the chain's non-blocking stream
+  return MSDR_OK;
+}
+
+/* AudioInputAnalog::init (input_adc.cpp:59-63): x1 = first reading << 14, y1 = 0 */
+int msdr_chain_frontend_preset(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint16_t first_reading)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (!range_ok(chain, ch0, nch)) return fail(chain, MSDR_ERR_ARGUMENT, "frontend_preset: bad channel range");
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "frontend_preset: call msdr_chain_enable_frontend first");
+  if (nch == 0) return MSDR_OK;
+  CK(cudaSetDevice(chain->device));
+  CK(cudaStreamSynchronize(chain->stream));
+  std::vector<fe::State> h(nch);
+  CK(cudaMemcpy(h.data(), chain->d_fe + ch0, nch * sizeof(fe::State), cudaMemcpyDeviceToHost));
+  for (auto &s : h) { s.hpf_x1 = (int32_t)((uint32_t)first_reading << 14); s.hpf_y1 = 0; }
+  CK(cudaMemcpy(chain->d_fe + ch0, h.data(), nch * sizeof(fe::State), cudaMemcpyHostToDevice));
+  CK(cudaDeviceSynchronize());
+  return MSDR_OK;
+}
+
+int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks,
+                                       size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
+  const int st = update_range(chain, ch0, nch, nullptr, d_out, n_blocks, stride, d_adc);
+  if (st == MSDR_OK && chain->fe_composed) chain->last_kernel = "msdr::fe::frontend_kernel (front end), then " + chain->last_kernel;
+  return st;
+}
+
+int msdr_chain_update_adc_device(msdr_chain *chain, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks, size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  return msdr_chain_update_adc_range_device(chain, 0, chain->C, d_adc, d_out, n_blocks, stride);
+}
+
+int msdr_chain_update_adc(msdr_chain *chain, const uint16_t *adc, int16_t *out, uint32_t n_blocks, size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (n_blocks == 0) return MSDR_OK;
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
+  return host_pipeline(chain, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true);
+}
+
+int msdr_chain_get_frontend_state(msdr_chain *chain, uint32_t ch, msdr_frontend_state *out)
+{
+  if (!chain || !out || ch >= chain->C) return MSDR_ERR_ARGUMENT;
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "get_frontend_state: call msdr_chain_enable_frontend first");
+  static_assert(sizeof(msdr_frontend_state) == sizeof(fe::State), "public and device state layouts must match");
+  CK(cudaSetDevice(chain->device));
+  CK(cudaStreamSynchronize(chain->stream));
+  CK(cudaMemcpy(out, chain->d_fe + ch, sizeof(*out), cudaMemcpyDeviceToHost));
+  return MSDR_OK;
+}
+
+int msdr_chain_set_frontend_state(msdr_chain *chain, uint32_t ch, const msdr_frontend_state *in)
+{
+  if (!chain || !in || ch >= chain->C) return MSDR_ERR_ARGUMENT;
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "set_frontend_state: call msdr_chain_enable_frontend first");
+  // agc_idx indexes the 25-entry history after a pre-decrement (Minimal-SDR.ino:481): anything outside 0..25 would be an out-of-bounds store
+  if (in->agc_idx < 0 || in->agc_idx > fe::kAgcBuf) return fail(chain, MSDR_ERR_ARGUMENT, "set_frontend_state: agc_idx outside [0, 25]");
+  CK(cudaSetDevice(chain->device));
+  CK(cudaStreamSynchronize(chain->stream));
+  CK(cudaMemcpy(chain->d_fe + ch, in, sizeof(*in), cudaMemcpyHostToDevice));
+  CK(cudaDeviceSynchronize());
   return MSDR_OK;
 }
 

@@ -73,7 +73,8 @@ size_t smem_bytes(uint32_t K, uint32_t ring)
 // FP64 pipe (msdr_device.cuh).  Alone in its sub-partition a warp steps equally fast either way (43 cycles, it is issue-bound);
 // here two biquad warps, two epilogue warps and a converter share a sub-partition and the integer multiplier is the scarce pipe
 // (IMAD.HI occupies it for 5 cycles), so the default moves three of the five products off it.
-template <class BQ>
+// kAdc: `p.in` holds raw ADC codes; the converters run the front end over them (FeRow, msdr_chain_v5_common.cuh)
+template <class BQ, bool kAdc>
 __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -171,6 +172,8 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         __syncwarp();
         if (lane == 0) mbar_arrive(&pc->b_full);
       }
+      FeRow fr;
+      if constexpr (kAdc) fe_row_begin(fr, p, __ldg(p.tc_rowmap + (size_t)rb * M + r));
       for (uint32_t u = 0; u < npairs; ++u, ++pseq) {
         const uint32_t stage = pseq % RS, pos = pseq % ring;
         prof.start();
@@ -180,6 +183,13 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         prof.lap(1);
         if (!(p.ablate & 1u)) {
           const uint32_t a = smem_u32(sRaw + stage * kRawStageBytes) + r * RAWP;
+          if constexpr (kAdc) {
+            if (u >= KS - 1) { // codes of samples 64 j .. 64 j + 63, j = u - (KS - 1); in front of sample 0 the history is conditioned already
+              const uint32_t t0 = (u - (KS - 1)) * N;
+              if (t0 == 0) fe_row_shift_hist(fr, p);
+              fe_row_run<N / 8>(fr, p, a, t0);
+            }
+          }
           uint4 v0[4], v1[4];
 #pragma unroll
           for (int j = 0; j < 4; ++j) { v0[j] = lds128(a + 16u * j); v1[j] = lds128(a + 64u + 16u * j); }
@@ -191,7 +201,9 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         if (lane == 0) { mbar_arrive(&pc->a_full[pos]); mbar_arrive(&pc->raw_free[stage]); }
         prof.lap(2);
       }
-      { // carry the last H raw samples of this thread's row: hist <- tail of (hist || in[0..L)).  The old history was this row
+      if constexpr (kAdc) {
+        fe_row_end(fr); // the history was written as the samples were conditioned
+      } else { // carry the last H raw samples of this thread's row: hist <- tail of (hist || in[0..L)).  The old history was this row
         // block's first staging entries, which this thread converted long ago; nobody else reads or writes the row's history.
         const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + r);
         if (row != kPad) {
@@ -450,7 +462,9 @@ cudaError_t launch_chain_v5(const ChainParams &p_in, cudaStream_t stream, int va
   const size_t smem = smem_bytes(p.tc_K, p.tc_ring);
   // default: the products as IMAD.HI (with the looped epilogue 352 against 339 Gsamples/s at C5 for the IMAD.WIDE form, which was 1.5 %
   // ahead before); study knobs: variant bit 0 = IMAD.WIDE for the four products off the recurrence, bit 1 = feed-forward products as DFMA
-  auto kern = (variant & 12) == 12 ? chain_kernel<BqStageS> : (variant & 1) ? chain_kernel<BqStageW> : (variant & 2) ? chain_kernel<BqStageH> : (variant & 4) ? chain_kernel<BqStageC> : (variant & 8) ? chain_kernel<BqStageE> : chain_kernel<BqStage>;
+  auto kern = p.fe ? chain_kernel<BqStage, true>
+                   : (variant & 12) == 12 ? chain_kernel<BqStageS, false> : (variant & 1) ? chain_kernel<BqStageW, false> : (variant & 2) ? chain_kernel<BqStageH, false>
+                   : (variant & 4) ? chain_kernel<BqStageC, false> : (variant & 8) ? chain_kernel<BqStageE, false> : chain_kernel<BqStage, false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   const uint32_t grid = p.n_items < (uint32_t)sms ? p.n_items : (uint32_t)sms;

@@ -1,7 +1,9 @@
 // msdr_chain_v5_common.cuh — helpers shared by the row-block kernels (msdr_chain_v5.cu: windows up to 128 words, msdr_chain_v5l.cu: the
-// 256-tap window): epilogue drain and demodulation on registers, the biquad tile loop, the developer profile.
+// 256-tap window): epilogue drain and demodulation on registers, the biquad tile loop, the developer profile, the front end of the
+// ADC-code input.
 #pragma once
 #include "msdr_chain_common.cuh"
+#include "msdr_frontend.cuh"
 #include "msdr_tc_common.cuh"
 
 namespace msdr {
@@ -104,6 +106,84 @@ __device__ __forceinline__ void demod_regs(const uint32_t (&iq)[32], int sgn, ui
   }
 }
 
+// ADC-code input (p.fe != NULL): the converter thread of a row owns the row's front end (msdr_frontend.cuh) for the whole row block and
+// runs it over the staged codes in time order, ahead of the fs/4 fold.  Per row: the recurrence and gain state in registers, the AGC's
+// 25-entry history in the chain's state array in global memory (the long window leaves no shared memory for it), touched once per
+// 128-sample block through an exact running sum of its entries; the slot a block overwrites is read when the block starts.
+struct FeRow {
+  fe::State *s;    // this row's state; NULL for a padded row
+  int x1, y1, mult, idx, sum, old;
+  float val;
+  uint32_t maxv, minv;
+};
+
+__device__ __forceinline__ void fe_row_begin(FeRow &f, const ChainParams &p, uint32_t row)
+{
+  f.s = nullptr;
+  if (row == kPad) return;
+  const size_t ch = (size_t)p.ch0 + row;
+  fe::State *s = p.fe + ch;
+  f.s = s;
+  f.x1 = s->hpf_x1; f.y1 = s->hpf_y1; f.mult = s->mult; f.idx = s->agc_idx; f.val = s->agc_val;
+  f.sum = 0;
+#pragma unroll 5
+  for (int k = 0; k < fe::kAgcBuf; ++k) f.sum += s->agc_buf[k];
+  f.old = 0;
+  f.maxv = fe::kMaxInit; f.minv = fe::kMinInit;
+}
+
+// The history rows hold conditioned IF samples in both input formats; here the converter writes them as it produces them.  For an
+// update shorter than the history (L < H) part of the old history survives and moves down first, in increasing order.  Call this only
+// once the converter has consumed the row block's history stages (j < 0): from then on the loader reads no history of this row, so
+// neither the move nor the new samples can race its copies.
+__device__ __forceinline__ uint4 *fe_row_hist(const FeRow &f, const ChainParams &p)
+{
+  return reinterpret_cast<uint4 *>(p.hist + (size_t)(f.s - p.fe) * p.H);
+}
+__device__ __forceinline__ void fe_row_shift_hist(const FeRow &f, const ChainParams &p)
+{
+  if (!f.s || p.L >= p.H) return;
+  uint4 *hrow = fe_row_hist(f, p);
+  const uint32_t lq = p.L >> 3, keep = (p.H >> 3) - lq;
+  for (uint32_t i = 0; i < keep; ++i) hrow[i] = __ldcg(hrow + i + lq);
+}
+
+// The 8 NQ staged codes of this thread's row at shared address `a`, samples t0 .. t0 + 8 NQ - 1 of the update (8 NQ divides 128), are
+// conditioned in place, one 16-byte word at a time: the fs/4 fold then reads IF samples as in the int16 form, and the conversion's
+// operands and the front end's state are never live together (the 736-thread CTA leaves 80 registers a thread).
+template <int NQ>
+__device__ __forceinline__ void fe_row_run(FeRow &f, const ChainParams &p, uint32_t a, uint32_t t0)
+{
+  if (!f.s) return;
+  if ((t0 & (fe::kBlock - 1)) == 0 && p.agc_on) f.old = f.idx > 0 ? f.s->agc_buf[f.idx - 1] : 0; // the slot this block's maximum takes
+  // the last H samples of hist || in become the history (sample t lands at t + H - L; L and H are multiples of 8)
+  uint4 *hrow = fe_row_hist(f, p) + (((int)t0 + (int)p.H - (int)p.L) >> 3);
+#pragma unroll 2
+  for (int q = 0; q < NQ; ++q) {
+    uint4 v = lds128(a + 16u * q);
+    v.x = fe::condition2(v.x, f.x1, f.y1, f.mult, f.maxv, f.minv);
+    v.y = fe::condition2(v.y, f.x1, f.y1, f.mult, f.maxv, f.minv);
+    v.z = fe::condition2(v.z, f.x1, f.y1, f.mult, f.maxv, f.minv);
+    v.w = fe::condition2(v.w, f.x1, f.y1, f.mult, f.maxv, f.minv);
+    sts128(a + 16u * q, v);
+    if ((int)(t0 + 8u * q) + (int)p.H >= (int)p.L) hrow[q] = v;
+  }
+  if (((t0 + 8u * NQ) & (fe::kBlock - 1)) == 0) { // an audio block is complete
+    if (p.agc_on) {
+      const int16_t m = (int16_t)fe::block_absmax(f.maxv, f.minv);
+      const int i = fe::agc_slot(f.idx);
+      if (i >= 0) { f.sum += (int)m - f.old; f.s->agc_buf[i] = m; }
+      fe::agc_law(f.val, f.mult, f.sum, p.agc_max);
+    }
+    f.maxv = fe::kMaxInit; f.minv = fe::kMinInit;
+  }
+}
+
+__device__ __forceinline__ void fe_row_end(const FeRow &f)
+{
+  if (!f.s) return;
+  f.s->hpf_x1 = f.x1; f.s->hpf_y1 = f.y1; f.s->mult = f.mult; f.s->agc_idx = f.idx; f.s->agc_val = f.val;
+}
 
 } // namespace v5
 } // namespace msdr

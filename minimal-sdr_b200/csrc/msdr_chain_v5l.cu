@@ -50,7 +50,8 @@ size_t smem_bytes(uint32_t K, uint32_t ring)
   return (size_t)kCtrlBytes + 4u * a_plane_bytes(ring) + 4u * N * K + (size_t)(RSH + NH) * kHalfBytes + 1024u;
 }
 
-template <class BQ>
+// kAdc: `p.in` holds raw ADC codes; the converters run the front end over them (FeRow, msdr_chain_v5_common.cuh)
+template <class BQ, bool kAdc>
 __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -148,6 +149,8 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         __syncwarp();
         if (lane == 0) mbar_arrive(&pc->b_full);
       }
+      FeRow fr;
+      if constexpr (kAdc) fe_row_begin(fr, p, __ldg(p.tc_rowmap + (size_t)rb * M + r));
       for (uint32_t u = 0; u < nhalf; ++u, ++hseq) {
         const uint32_t stage = hseq % RSH, kb = u & 1u, pos = pseq % ring;
         prof.start();
@@ -157,6 +160,13 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         prof.lap(1);
         if (!(p.ablate & 1u)) {
           const uint32_t a = smem_u32(sRaw + stage * kHalfBytes) + r * HP;
+          if constexpr (kAdc) {
+            if (u >= 2 * (KS - 1)) { // codes of samples 32 hh .. 32 hh + 31, hh = u - 2 (KS - 1); in front of sample 0 the history is conditioned already
+              const uint32_t t0 = (u - 2 * (KS - 1)) * HU;
+              if (t0 == 0) fe_row_shift_hist(fr, p);
+              fe_row_run<HU / 8>(fr, p, a, t0);
+            }
+          }
           uint4 v[4];
 #pragma unroll
           for (int j = 0; j < 4; ++j) v[j] = lds128(a + 16u * j);
@@ -171,7 +181,9 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         if (kb) ++pseq;
         prof.lap(2);
       }
-      { // carry the last H raw samples of this thread's row: hist <- tail of (hist || in[0..L)), as in msdr_chain_v5.cu
+      if constexpr (kAdc) {
+        fe_row_end(fr); // the history was written as the samples were conditioned
+      } else { // carry the last H raw samples of this thread's row: hist <- tail of (hist || in[0..L)), as in msdr_chain_v5.cu
         const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + r);
         if (row != kPad) {
           const uint32_t hq = p.H >> 3; // uint4 per history row (<= 33)
@@ -409,7 +421,8 @@ cudaError_t launch_chain_v5l(const ChainParams &p_in, cudaStream_t stream, int v
   ChainParams p = p_in;
   p.ablate = ((uint32_t)variant >> 4) & 3u;
   const size_t smem = smem_bytes(p.tc_K, p.tc_ring);
-  auto kern = (variant & 1) ? chain_kernel<BqStage> : chain_kernel<BqStageW>; // variant bit 0: all five products as IMAD.HI (cross-check)
+  // variant bit 0: all five products as IMAD.HI (cross-check)
+  auto kern = p.fe ? chain_kernel<BqStageW, true> : (variant & 1) ? chain_kernel<BqStage, false> : chain_kernel<BqStageW, false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   const uint32_t grid = p.n_items < (uint32_t)sms ? p.n_items : (uint32_t)sms;

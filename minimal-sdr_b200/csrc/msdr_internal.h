@@ -6,6 +6,8 @@
 
 namespace msdr {
 
+namespace fe { struct State; } // msdr_frontend.cuh
+
 constexpr int kGroup = 32;            // channels per work group (one biquad lane each)
 constexpr int kBqWords = 64;          // 2 objects x 4 stages x 8 words (filter_biquad.h:152)
 
@@ -54,6 +56,10 @@ struct ChainParams {
   uint32_t spare_sms;          // v4: launch this many fewer CTAs than a wave has slots (never fewer than there are chains to pin)
   long long *prof;             // developer profile buffer [grid][64] or NULL
   int *tile_cnt;               // [NG][NU] rows of group g whose unit u is in `out` (zeroed before the launch)
+  // ADC-code input (row-block kernels only): non-NULL = `in` holds raw uint16 codes and the converters run the front end first
+  fe::State *fe;               // [chain channels] front-end state, indexed like hist
+  float agc_max;
+  uint32_t agc_on;
 };
 
 struct ChainLaunchInfo {
@@ -70,7 +76,12 @@ cudaError_t launch_chain_v4(const ChainParams &p, cudaStream_t stream, int varia
 uint32_t chain_v4_span_samples();
 uint32_t chain_v4_unit_samples();
 bool chain_v4_config(uint32_t K, int smem_max, uint32_t rings[4]);
-// row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config (0 = does not fit)
+// K4 (msdr_frontend.cu) over C rows: raw codes -> conditioned int16 IF samples; state = the first row's front-end state.
+// sms > 0 packs the channel groups into about that many CTAs.
+cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, uint32_t C, uint32_t n_blocks, fe::State *state, float agc_max,
+                            int agc_on, int sms, cudaStream_t s);
+// row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config (0 = does not fit);
+// p.fe != NULL selects the ADC-code instantiation (default biquad form only)
 cudaError_t launch_chain_v5(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
 uint32_t chain_v5_config(uint32_t K, int smem_max);
 // pinned 32-channel group blocks with the tile rows folded over time (msdr_chain_v6.cu): p.tc_rowmap = [n_items][32] rows of one table,
