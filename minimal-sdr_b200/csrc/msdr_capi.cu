@@ -252,6 +252,22 @@ int assign_set(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t id)
   return MSDR_OK;
 }
 
+// Before channels are bound to a new table, a table used by none but them gives its slot back (its channels stay unbound until the
+// caller binds them): re-tuning a full chain (MSDR_MAX_FIR_SETS live tables) then does not fail for want of the slot it frees itself.
+// A table that keeps another user keeps its slot, and nothing changes when no table is freed, so a refused table leaves the chain as
+// it was.  Used by both FIR setters.  `each(f)` calls f(channel) for every channel to be re-bound, each channel once.
+template <class Each> void release_sole_sets(msdr_chain *chain, Each each)
+{
+  uint32_t n[MSDR_MAX_FIR_SETS] = {0};
+  each([&](uint32_t c) { if (chain->h_set[c] != 0xFF) n[chain->h_set[c]]++; });
+  auto sole = [&](uint32_t sid) { return n[sid] && n[sid] == chain->sets[sid].users; };
+  each([&](uint32_t c) {
+    if (chain->h_set[c] != 0xFF && sole(chain->h_set[c])) { chain->h_set[c] = 0xFF; chain->n_uninit++; }
+  });
+  for (uint32_t sid = 0; sid < chain->sets.size(); ++sid)
+    if (sole(sid)) chain->sets[sid].users = 0;
+}
+
 int ensure_stage(msdr_chain *chain, size_t samples)
 {
   if (chain->stage_samples >= samples) return MSDR_OK;
@@ -467,19 +483,7 @@ int msdr_fir_init_q15(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint16_t nu
   if (numTaps < 4 || numTaps > chain->max_taps) return fail(chain, MSDR_ERR_LENGTH, "fir_init: numTaps outside [4, max_taps of this chain]");
   if (nch == 0) return MSDR_OK;
   CK(cudaSetDevice(chain->device));
-  // a table used by nobody but this range is about to lose its last user: give its slot back first, so re-tuning a full chain
-  // (MSDR_MAX_FIR_SETS live tables) does not fail for want of the slot it is freeing itself
-  {
-    uint32_t in_range[MSDR_MAX_FIR_SETS] = {0};
-    for (uint32_t c = ch0; c < ch0 + nch; ++c)
-      if (chain->h_set[c] != 0xFF) in_range[chain->h_set[c]]++;
-    for (uint32_t sid = 0; sid < chain->sets.size(); ++sid)
-      if (in_range[sid] && in_range[sid] == chain->sets[sid].users) {
-        for (uint32_t c = ch0; c < ch0 + nch; ++c)
-          if (chain->h_set[c] == sid) { chain->h_set[c] = 0xFF; chain->n_uninit++; }
-        chain->sets[sid].users = 0;
-      }
-  }
+  release_sole_sets(chain, [&](auto &&f) { for (uint32_t c = ch0; c < ch0 + nch; ++c) f(c); });
   const int id = intern_set(chain, numTaps, cI, cQ);
   if (id < 0) return id;
   int st = assign_set(chain, ch0, nch, (uint32_t)id);
@@ -521,6 +525,12 @@ int msdr_fir_init_q15_list(msdr_chain *chain, const uint32_t *channels, uint32_t
     lo = std::min(lo, channels[i]); hi = std::max(hi, channels[i]);
   }
   CK(cudaSetDevice(chain->device));
+  {
+    std::vector<uint32_t> uniq(channels, channels + n); // a channel listed twice is one user
+    std::sort(uniq.begin(), uniq.end());
+    uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
+    release_sole_sets(chain, [&](auto &&f) { for (uint32_t c : uniq) f(c); });
+  }
   const int id = intern_set(chain, numTaps, cI, cQ);
   if (id < 0) return id;
   uint32_t added = 0;
