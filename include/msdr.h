@@ -147,6 +147,36 @@ const char *msdr_chain_last_kernel(const msdr_chain *chain);
 int msdr_chain_get_state(msdr_chain *chain, uint32_t ch, msdr_channel_state *out);
 int msdr_chain_set_state(msdr_chain *chain, uint32_t ch, const msdr_channel_state *in);
 
+/* ---- snapshots: checkpoint / resume / migration / re-sharding of channel ranges ----
+ * A snapshot of channels [ch0, ch0+nch) holds everything they carry: their FIR tables (renumbered densely), modes and ANR switches, the
+ * FIR history, both biquad objects, the SYNCAM PLL, and the front-end and LMS state when the chain has them.  The format is versioned and
+ * little-endian, every section starts on a 256-byte boundary (DESIGN.md 7); state sections are plain strided copies of the chain's arrays.
+ * msdr_chain_restore(chain, ch0, buf, bytes, first, n) gives chain channels [ch0, ch0+n) the state of snapshot channels [first, first+n)
+ * (restoring a whole snapshot into the range it came from gives back exactly the chain that was saved), into any chain on any device
+ * whose flags equal the snapshot's and whose max_taps covers the tables used.  A different FIR history length (max_taps) keeps the last
+ * min(H, H') samples, like msdr_chain_set_state.  Restore is all or nothing: MSDR_ERR_ARGUMENT for a bad magic, a truncated buffer, bad
+ * offsets, ranges outside the snapshot or the chain, other flags, a table longer than max_taps or other AGC parameters than the chain's
+ * front end; MSDR_ERR_UNSUPPORTED for another format version; MSDR_ERR_NOMEM when the range would need more than MSDR_MAX_FIR_SETS live
+ * tables (tables only the range used give their slots back first).  A refused restore changes nothing.
+ *   - front end: a snapshot with one enables it on a chain without one (its AGC parameters; other channels start as after
+ *     msdr_chain_enable_frontend); a chain with one and a snapshot without gives the restored channels the initial front-end state.
+ *   - ANR: a snapshot of a chain that ever switched ANR on allocates the LMS arrays; one without gives restored channels the initial state.
+ *   - a restore is one configuration change: the next update over a range builds at most one row plan.
+ * The host calls return when the buffer is written / may be freed; pinned buffers (msdr_host_alloc) move at PCIe rate.  The device
+ * calls take a buffer on the chain's device and are asynchronous on the chain's stream, ordered after every earlier update; keep d_buf
+ * alive until the stream has passed.  restore_device reads header, tables and meta with one small synchronous copy, and trusts the
+ * state sections (a host restore also checks the front-end agc_idx and ANR in_idx of every restored channel). */
+size_t msdr_chain_snapshot_bytes(const msdr_chain *chain, uint32_t nch);
+int msdr_chain_snapshot(msdr_chain *chain, uint32_t ch0, uint32_t nch, void *buf, size_t bytes);          /* host buffer, returns when written */
+int msdr_chain_snapshot_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, void *d_buf, size_t bytes); /* device buffer on the chain's device, asynchronous on its stream */
+int msdr_chain_restore(msdr_chain *chain, uint32_t ch0, const void *buf, size_t bytes, uint32_t first, uint32_t n);
+int msdr_chain_restore_device(msdr_chain *chain, uint32_t ch0, const void *d_buf, size_t bytes, uint32_t first, uint32_t n);
+/* host-only, no device needed: validates a snapshot header (host copy of at least its first 256 bytes).  flags = the chain flags of the
+ * snapshot, plus MSDR_SNAPSHOT_FRONTEND / MSDR_SNAPSHOT_ANR for the sections it has; max_taps_needed = the longest table it holds. */
+#define MSDR_SNAPSHOT_FRONTEND (1u << 16)
+#define MSDR_SNAPSHOT_ANR (1u << 17)
+int msdr_snapshot_info(const void *header, size_t bytes, uint32_t *n_channels, uint32_t *max_taps_needed, uint32_t *flags);
+
 /* Options.  "variant" selects the shape of the fused kernel for studies and cross-checks (all shapes are bit-exact, DESIGN.md 6):
  *   0    default, by channel count: the time-folded kernel (msdr_chain_v6.cu) up to one 32-channel group block per SM; tensor-core
  *        FIR producers (tcgen05 kind::i8) + pinned biquad chains (msdr_chain_v4.cu: feed-forward helper warps up to 148 channel

@@ -585,6 +585,22 @@ public:
     status_ = msdr_chain_get_frontend_state(chain_, ch, &s);
     return s.agc_val;
   }
+  // checkpoint / resume of a channel range (msdr_chain_snapshot / msdr_chain_restore): snapshot() fills `blob` with everything channels
+  // [ch0, ch0+nch) carry, restore() gives channels [ch0, ch0+n) the state of snapshot channels [first, first+n) (n = ~0u: the rest)
+  int snapshot(std::vector<uint8_t> &blob, uint32_t ch0 = 0, uint32_t nch = ~0u)
+  {
+    blob.resize(msdr_chain_snapshot_bytes(chain_, cnt(ch0, nch)));
+    return status_ = msdr_chain_snapshot(chain_, ch0, cnt(ch0, nch), blob.data(), blob.size());
+  }
+  int restore(const std::vector<uint8_t> &blob, uint32_t ch0 = 0, uint32_t first = 0, uint32_t n = ~0u)
+  {
+    if (n == ~0u) {
+      uint32_t total = 0;
+      if ((status_ = msdr_snapshot_info(blob.data(), blob.size(), &total, nullptr, nullptr)) != MSDR_OK) return status_;
+      n = total - first;
+    }
+    return status_ = msdr_chain_restore(chain_, ch0, blob.data(), blob.size(), first, n);
+  }
   uint32_t channels() const { return n_; }
 private:
   uint32_t cnt(uint32_t ch0, uint32_t nch) const { return nch == ~0u ? n_ - ch0 : nch; }

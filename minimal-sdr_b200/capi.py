@@ -9,6 +9,7 @@ BLOCK = 128
 MAX_TAPS = 256
 MODE_SYNCAM, MODE_AM, MODE_LSB, MODE_USB, MODE_CW = 0, 1, 2, 3, 4  # stations.h:4
 FLAG_AM_Q31 = 1
+SNAPSHOT_FRONTEND, SNAPSHOT_ANR = 1 << 16, 1 << 17  # msdr_snapshot_info flags: sections the snapshot has
 OK, ERR_ARGUMENT, ERR_LENGTH, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOMEM, ERR_NOT_INITIALISED = 0, -1, -2, -100, -101, -102, -103
 
 
@@ -136,6 +137,12 @@ SYMBOLS = {
     "msdr_syncam_set_state": (C.c_int, [C.c_void_p, C.c_uint32, C.c_float, C.c_float, C.c_float]),
     "msdr_syncam_constants": (C.c_int, [C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "msdr_syncam_launch_count": (C.c_uint64, [C.c_void_p]),
+    "msdr_chain_snapshot_bytes": (C.c_size_t, [C.c_void_p, C.c_uint32]),
+    "msdr_chain_snapshot": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_size_t]),
+    "msdr_chain_snapshot_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_size_t]),
+    "msdr_chain_restore": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_size_t, C.c_uint32, C.c_uint32]),
+    "msdr_chain_restore_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_size_t, C.c_uint32, C.c_uint32]),
+    "msdr_snapshot_info": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "msdr_version": (C.c_char_p, []),
 }
 
@@ -170,6 +177,17 @@ def check(status, handle=None):
         msg = lib().msdr_last_error(handle)
         raise MsdrError(status, msg.decode() if msg else "")
     return status
+
+
+def snapshot_info(blob):
+    """msdr_snapshot_info on a host copy of (at least the first 256 bytes of) a snapshot: {n_channels, max_taps_needed, flags}.
+    Needs no device; raises MsdrError for a bad magic, a short header or another format version."""
+    b = np.ascontiguousarray(blob, np.uint8).reshape(-1)
+    n, t, f = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+    st = lib().msdr_snapshot_info(ptr(b), b.size, C.byref(n), C.byref(t), C.byref(f))
+    if st != OK:
+        raise MsdrError(st, "msdr_snapshot_info")
+    return {"n_channels": n.value, "max_taps_needed": t.value, "flags": f.value}
 
 
 class PinnedBuffer:

@@ -256,3 +256,42 @@ class ReceiveChain:
 
     def set_state(self, ch, st):
         return self._ck(self._L.msdr_chain_set_state(self.h, int(ch), C.byref(st)))
+
+    # -- snapshots: checkpoint / resume / migration / re-sharding of channel ranges (include/msdr.h, DESIGN.md 7) -----------------
+    def snapshot_bytes(self, nch=None):
+        return int(self._L.msdr_chain_snapshot_bytes(self.h, int(self.n_channels if nch is None else nch)))
+
+    def snapshot(self, ch0=0, nch=None, out=None):
+        """Channels [ch0, ch0+nch) as a uint8 array (tables, modes, ANR switches and all device state).  `out`: a host uint8 array of at
+        least snapshot_bytes(nch) bytes to write into, e.g. capi.PinnedBuffer(...).array for PCIe-rate copies."""
+        ch0, nch = self._rng(ch0, nch)
+        size = self.snapshot_bytes(nch)
+        if out is None:
+            out = np.empty(size, np.uint8)
+        assert out.dtype == np.uint8 and out.flags.c_contiguous and out.size >= size
+        self._ck(self._L.msdr_chain_snapshot(self.h, ch0, nch, capi.ptr(out), out.size))
+        return out[:size]
+
+    def restore(self, blob, ch0=0, first=0, n=None):
+        """Chain channels [ch0, ch0+n) take the state of snapshot channels [first, first+n) (n = None: the rest of the snapshot)."""
+        blob = np.ascontiguousarray(blob, np.uint8).reshape(-1)
+        if n is None:
+            n = capi.snapshot_info(blob)["n_channels"] - int(first)
+        return self._ck(self._L.msdr_chain_restore(self.h, int(ch0), capi.ptr(blob), blob.size, int(first), int(n)))
+
+    @staticmethod
+    def _device_bytes(tensor):
+        assert tensor.is_cuda and str(tensor.dtype) == "torch.uint8" and tensor.is_contiguous(), "a contiguous CUDA uint8 tensor"
+        return C.c_void_p(tensor.data_ptr()), tensor.numel()
+
+    def snapshot_device(self, ch0, nch, tensor):
+        """Into a CUDA uint8 tensor on the chain's device, asynchronous on the chain's stream (after every earlier update)."""
+        p, size = self._device_bytes(tensor)
+        return self._ck(self._L.msdr_chain_snapshot_device(self.h, int(ch0), int(nch), p, size))
+
+    def restore_device(self, tensor, ch0=0, first=0, n=None):
+        """From a CUDA uint8 tensor on the chain's device; keep the tensor alive until the chain's stream has passed."""
+        p, size = self._device_bytes(tensor)
+        if n is None:
+            n = capi.snapshot_info(tensor[:256].cpu().numpy())["n_channels"] - int(first)
+        return self._ck(self._L.msdr_chain_restore_device(self.h, int(ch0), p, size, int(first), int(n)))

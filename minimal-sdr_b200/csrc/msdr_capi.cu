@@ -153,6 +153,16 @@ struct msdr_chain {
   size_t fe_if_samples = 0;
   bool fe_composed = false;          // the last ADC update ran K4, then the int16 path
 
+  // snapshots (msdr_chain_snapshot* / msdr_chain_restore*): host vectors their asynchronous uploads read from; `snap_ev` marks the
+  // last such upload, and the next snapshot or restore waits for it before it writes them again
+  std::vector<uint8_t> snap_host;
+  std::vector<int32_t> snap_ex;
+  std::vector<uint32_t> snap_kp4;
+  std::vector<int16_t> snap_taps;
+  fe::State snap_fe0{};
+  cudaEvent_t snap_ev = nullptr;
+  bool snap_pending = false;
+
   int variant = 0;
   uint32_t host_chunk_channels = 0, host_chunk_blocks = 0; // 0 = auto
   uint32_t spare_sms = 0;
@@ -371,6 +381,7 @@ void msdr_chain_destroy(msdr_chain *chain)
   for (cudaEvent_t ev : chain->pipe_ev) cudaEventDestroy(ev);
   if (chain->ev0) cudaEventDestroy(chain->ev0);
   if (chain->ev1) cudaEventDestroy(chain->ev1);
+  if (chain->snap_ev) cudaEventDestroy(chain->snap_ev);
   if (chain->own_stream) cudaStreamDestroy(chain->own_stream);
   if (chain->copy_in) cudaStreamDestroy(chain->copy_in);
   if (chain->copy_out) cudaStreamDestroy(chain->copy_out);
@@ -1434,6 +1445,437 @@ int msdr_chain_set_state(msdr_chain *chain, uint32_t ch, const msdr_channel_stat
                   cudaMemcpyHostToDevice));
   CK(cudaMemcpy2D(chain->d_pll + ch, (size_t)chain->Cpad * sizeof(float), in->syncam_pll, sizeof(float), sizeof(float), 3, cudaMemcpyHostToDevice));
   CK(cudaDeviceSynchronize()); // legacy-stream copies vs the chain's non-blocking stream
+  return MSDR_OK;
+}
+
+// ---- snapshots of channel ranges: checkpoint, resume, migration, re-sharding (format: DESIGN.md 7) ------------------------------
+// Every state section is a plain (2D) copy of one SoA array of the chain; the copy engines do the work, no kernel is involved.
+namespace {
+
+constexpr char kSnapMagic[8] = {'M', 'S', 'D', 'R', 'S', 'N', 'A', 'P'};
+constexpr uint32_t kSnapVersion = 1;
+constexpr uint32_t kSnapHeaderBytes = 256;
+constexpr uint32_t kSnapFrontend = 1u, kSnapAnr = 2u; // header `sections`
+constexpr uint8_t kNoTable = 0xFF;
+
+struct SnapTable {
+  uint32_t T;
+  int16_t cI[MSDR_MAX_TAPS], cQ[MSDR_MAX_TAPS];
+};
+static_assert(sizeof(SnapTable) == 1028, "snapshot table entry layout");
+
+enum { kOffTables, kOffMeta, kOffHist, kOffBq, kOffPll, kOffFe, kOffAnrD, kOffAnrW, kOffAnrLidx, kOffAnrNgamma, kOffAnrIdx, kNumOff };
+
+struct SnapHeader {
+  char magic[8];
+  uint32_t version, header_bytes;
+  uint64_t total_bytes;
+  uint32_t nch, flags, hist_len, sections;
+  float agc_start, agc_max;
+  int32_t agc_on;
+  uint32_t n_tables, max_taps_needed, reserved;
+  uint64_t off[kNumOff]; // 0 = section absent
+  uint8_t zero[kSnapHeaderBytes - 64 - 8 * kNumOff];
+};
+static_assert(sizeof(SnapHeader) == kSnapHeaderBytes, "snapshot header is 256 bytes");
+
+struct SnapLayout {
+  uint64_t off[kNumOff], size[kNumOff];
+  uint64_t total;
+};
+
+// the whole layout follows from (nch, hist_len, sections): every section starts on a 256-byte boundary, absent sections have offset 0
+SnapLayout snap_layout(uint64_t nch, uint32_t hist_len, uint32_t sections)
+{
+  SnapLayout l{};
+  uint64_t p = kSnapHeaderBytes;
+  auto put = [&](int k, uint64_t bytes) { l.off[k] = p; l.size[k] = bytes; p = (p + bytes + 255u) & ~(uint64_t)255u; };
+  put(kOffTables, (uint64_t)MSDR_MAX_FIR_SETS * sizeof(SnapTable));
+  put(kOffMeta, 4 * nch);
+  put(kOffHist, 2 * nch * hist_len);
+  put(kOffBq, 4 * kBqWords * nch);
+  put(kOffPll, 4 * 3 * nch);
+  if (sections & kSnapFrontend) put(kOffFe, sizeof(fe::State) * nch);
+  if (sections & kSnapAnr) {
+    put(kOffAnrD, 4 * 512 * nch); put(kOffAnrW, 4 * 64 * nch);
+    put(kOffAnrLidx, 4 * nch); put(kOffAnrNgamma, 4 * nch); put(kOffAnrIdx, 4 * nch);
+  }
+  l.total = p;
+  return l;
+}
+
+uint32_t chain_sections(const msdr_chain *c) { return (c->d_fe ? kSnapFrontend : 0u) | (c->d_anr_d ? kSnapAnr : 0u); }
+
+// header checks that need no device: 0, or a status with `why` set
+int snap_parse_header(const void *buf, size_t bytes, SnapHeader &h, const char *&why)
+{
+  why = "";
+  if (!buf || bytes < kSnapHeaderBytes) { why = "snapshot: buffer shorter than the 256-byte header"; return MSDR_ERR_ARGUMENT; }
+  memcpy(&h, buf, sizeof(h));
+  if (memcmp(h.magic, kSnapMagic, sizeof(kSnapMagic))) { why = "snapshot: bad magic"; return MSDR_ERR_ARGUMENT; }
+  if (h.version != kSnapVersion) { why = "snapshot: format version not supported by this library"; return MSDR_ERR_UNSUPPORTED; }
+  const uint32_t hist_max = hist_of_kp(kp_of_taps(MSDR_MAX_TAPS));
+  if (h.header_bytes != kSnapHeaderBytes || h.nch == 0 || h.hist_len == 0 || h.hist_len > hist_max || (h.sections & ~(kSnapFrontend | kSnapAnr)) ||
+      (h.flags & ~MSDR_FLAG_AM_Q31) || h.n_tables > MSDR_MAX_FIR_SETS || h.max_taps_needed > MSDR_MAX_TAPS) {
+    why = "snapshot: header field out of range";
+    return MSDR_ERR_ARGUMENT;
+  }
+  const SnapLayout l = snap_layout(h.nch, h.hist_len, h.sections);
+  if (h.total_bytes != l.total || memcmp(h.off, l.off, sizeof(l.off))) { why = "snapshot: section offsets or total size do not match the layout"; return MSDR_ERR_ARGUMENT; }
+  return MSDR_OK;
+}
+
+// before writing the staging vectors again, the uploads that read them must have run
+int snap_wait(msdr_chain *chain)
+{
+  if (!chain->snap_ev) CK(cudaEventCreateWithFlags(&chain->snap_ev, cudaEventDisableTiming));
+  if (chain->snap_pending) CK(cudaEventSynchronize(chain->snap_ev));
+  chain->snap_pending = false;
+  return MSDR_OK;
+}
+
+int snap_uploaded(msdr_chain *chain)
+{
+  CK(cudaEventRecord(chain->snap_ev, chain->stream));
+  chain->snap_pending = true;
+  return MSDR_OK;
+}
+
+// header, tables and meta of channels [ch0, ch0+nch) into chain->snap_host (the first l.off[kOffHist] bytes of the snapshot)
+void snap_build_prefix(msdr_chain *chain, uint32_t ch0, uint32_t nch, const SnapLayout &l)
+{
+  std::vector<uint8_t> &b = chain->snap_host;
+  b.assign(l.off[kOffHist], 0);
+  SnapHeader h{};
+  memcpy(h.magic, kSnapMagic, sizeof(h.magic));
+  h.version = kSnapVersion; h.header_bytes = kSnapHeaderBytes; h.total_bytes = l.total;
+  h.nch = nch; h.flags = chain->flags; h.hist_len = chain->H; h.sections = chain_sections(chain);
+  if (chain->d_fe) { h.agc_start = chain->fe_agc_start; h.agc_max = chain->fe_agc_max; h.agc_on = chain->fe_agc_on; }
+  memcpy(h.off, l.off, sizeof(h.off));
+  uint8_t dense[MSDR_MAX_FIR_SETS];
+  memset(dense, kNoTable, sizeof(dense));
+  SnapTable *tab = reinterpret_cast<SnapTable *>(b.data() + l.off[kOffTables]);
+  uint8_t *meta = b.data() + l.off[kOffMeta];
+  for (uint32_t i = 0; i < nch; ++i) {
+    const uint32_t c = ch0 + i;
+    const uint8_t sid = chain->h_set[c];
+    if (sid != kNoTable && dense[sid] == kNoTable) { // tables renumbered densely, in order of first use
+      const FirSet &fs = chain->sets[sid];
+      SnapTable &t = tab[h.n_tables];
+      t.T = fs.T;
+      memcpy(t.cI, fs.cI.data(), fs.T * 2);
+      memcpy(t.cQ, fs.cQ.data(), fs.T * 2);
+      h.max_taps_needed = std::max(h.max_taps_needed, fs.T);
+      dense[sid] = (uint8_t)h.n_tables++;
+    }
+    meta[4 * i + 0] = chain->h_mode[c];
+    meta[4 * i + 1] = sid == kNoTable ? kNoTable : dense[sid];
+    meta[4 * i + 2] = chain->h_anr.empty() ? 0 : chain->h_anr[c];
+  }
+  memcpy(b.data(), &h, sizeof(h));
+}
+
+// the state sections of channels [ch0, ch0+nch) into dst (host or device), on the chain's stream
+int snap_copy_state_out(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint8_t *dst, const SnapLayout &l, cudaMemcpyKind kind)
+{
+  cudaStream_t s = chain->stream;
+  const size_t cp = (size_t)chain->Cpad * 4, w = (size_t)nch * 4;
+  CK(cudaMemcpyAsync(dst + l.off[kOffHist], chain->d_hist + (size_t)ch0 * chain->H, (size_t)nch * chain->H * 2, kind, s));
+  CK(cudaMemcpy2DAsync(dst + l.off[kOffBq], w, chain->d_bq + ch0, cp, w, kBqWords, kind, s));
+  CK(cudaMemcpy2DAsync(dst + l.off[kOffPll], w, chain->d_pll + ch0, cp, w, 3, kind, s));
+  if (chain->d_fe) CK(cudaMemcpyAsync(dst + l.off[kOffFe], chain->d_fe + ch0, (size_t)nch * sizeof(fe::State), kind, s));
+  for (int k = kOffHist; k < kNumOff; ++k) { // the alignment padding after each state section is zero: equal chains give equal snapshots
+    if (!l.off[k]) continue;
+    const uint64_t end = l.off[k] + l.size[k], pad = ((end + 255u) & ~(uint64_t)255u) - end;
+    if (!pad) continue;
+    if (kind == cudaMemcpyDeviceToHost) memset(dst + end, 0, pad);
+    else CK(cudaMemsetAsync(dst + end, 0, pad, s));
+  }
+  if (chain->d_anr_d) {
+    CK(cudaMemcpy2DAsync(dst + l.off[kOffAnrD], w, chain->d_anr_d + ch0, cp, w, 512, kind, s));
+    CK(cudaMemcpy2DAsync(dst + l.off[kOffAnrW], w, chain->d_anr_w + ch0, cp, w, 64, kind, s));
+    CK(cudaMemcpyAsync(dst + l.off[kOffAnrLidx], chain->d_anr_lidx + ch0, w, kind, s));
+    CK(cudaMemcpyAsync(dst + l.off[kOffAnrNgamma], chain->d_anr_ngamma + ch0, w, kind, s));
+    CK(cudaMemcpyAsync(dst + l.off[kOffAnrIdx], chain->d_anr_idx + ch0, w, kind, s));
+  }
+  return MSDR_OK;
+}
+
+int snap_begin(msdr_chain *chain, uint32_t ch0, uint32_t nch, size_t bytes, const void *buf, SnapLayout &l)
+{
+  if (!buf || nch == 0 || !range_ok(chain, ch0, nch)) return fail(chain, MSDR_ERR_ARGUMENT, "snapshot: bad buffer or channel range");
+  l = snap_layout(nch, chain->H, chain_sections(chain));
+  if (bytes < l.total) return fail(chain, MSDR_ERR_ARGUMENT, "snapshot: buffer smaller than msdr_chain_snapshot_bytes");
+  CK(cudaSetDevice(chain->device));
+  return snap_wait(chain);
+}
+
+// `count` copies of the element at host address `elem` (which outlives the copies) from d on: one upload, then doubling copies
+int replicate(msdr_chain *chain, void *d, size_t elem_bytes, size_t count, const void *elem)
+{
+  if (!count) return MSDR_OK;
+  uint8_t *p = static_cast<uint8_t *>(d);
+  CK(cudaMemcpyAsync(p, elem, elem_bytes, cudaMemcpyHostToDevice, chain->stream));
+  for (size_t done = 1; done < count; done *= 2)
+    CK(cudaMemcpyAsync(p + done * elem_bytes, p, std::min(done, count - done) * elem_bytes, cudaMemcpyDeviceToDevice, chain->stream));
+  return MSDR_OK;
+}
+
+const float kAnrLidx0 = 120.0f, kAnrNgamma0 = 0.001f; // Minimal-SDR.ino:715,718
+
+// initial LMS state (msdr_chain_set_anr's) for channels [ch0, ch0+n)
+int anr_initial(msdr_chain *chain, uint32_t ch0, uint32_t n)
+{
+  const size_t cp = (size_t)chain->Cpad * 4, w = (size_t)n * 4;
+  CK(cudaMemset2DAsync(chain->d_anr_d + ch0, cp, 0, w, 512, chain->stream));
+  CK(cudaMemset2DAsync(chain->d_anr_w + ch0, cp, 0, w, 64, chain->stream));
+  CK(cudaMemsetAsync(chain->d_anr_idx + ch0, 0, w, chain->stream));
+  int st = replicate(chain, chain->d_anr_lidx + ch0, 4, n, &kAnrLidx0);
+  if (st == MSDR_OK) st = replicate(chain, chain->d_anr_ngamma + ch0, 4, n, &kAnrNgamma0);
+  return st;
+}
+
+// Restore channels [ch0, ch0+n) from snapshot channels [first, first+n).  `pre` is a host copy of the snapshot from byte 0 through
+// the meta of channel first+n-1; `src` is the whole snapshot (host or device, `kind`).  Every check runs before anything changes.
+int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre_bytes, const uint8_t *src, size_t bytes, uint32_t first, uint32_t n,
+                 cudaMemcpyKind kind)
+{
+  SnapHeader h;
+  const char *why;
+  int st = snap_parse_header(pre, pre_bytes, h, why);
+  if (st != MSDR_OK) return fail(chain, st, why);
+  if (bytes < h.total_bytes) return fail(chain, MSDR_ERR_ARGUMENT, "restore: buffer shorter than the snapshot's total size");
+  if ((uint64_t)first + n > h.nch || !range_ok(chain, ch0, n)) return fail(chain, MSDR_ERR_ARGUMENT, "restore: channel range outside the snapshot or the chain");
+  if (h.flags != chain->flags) return fail(chain, MSDR_ERR_ARGUMENT, "restore: the snapshot's chain flags (MSDR_FLAG_AM_Q31) differ from this chain's");
+  const bool has_fe = h.sections & kSnapFrontend, has_anr = h.sections & kSnapAnr;
+  if (has_fe && chain->d_fe && (h.agc_start != chain->fe_agc_start || h.agc_max != chain->fe_agc_max || (h.agc_on != 0) != (chain->fe_agc_on != 0)))
+    return fail(chain, MSDR_ERR_ARGUMENT, "restore: the snapshot's AGC parameters differ from this chain's front end");
+  if (n == 0) return MSDR_OK;
+  const SnapTable *tab = reinterpret_cast<const SnapTable *>(pre + h.off[kOffTables]);
+  const uint8_t *meta = pre + h.off[kOffMeta] + 4 * (size_t)first;
+  uint32_t used[MSDR_MAX_FIR_SETS] = {0};
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint8_t *m = meta + 4 * i;
+    if (m[0] > MSDR_MODE_CW || (m[1] != kNoTable && m[1] >= h.n_tables) || m[2] > 2 || (m[2] && !has_anr))
+      return fail(chain, MSDR_ERR_ARGUMENT, "restore: bad channel entry in the snapshot's meta section");
+    if (m[1] != kNoTable) used[m[1]]++;
+  }
+  for (uint32_t k = 0; k < h.n_tables; ++k)
+    if (used[k] && (tab[k].T < 4 || (tab[k].T & 1u) || tab[k].T > chain->max_taps))
+      return fail(chain, MSDR_ERR_ARGUMENT, "restore: a table of the snapshot is longer than this chain's max_taps (or malformed)");
+  if (kind == cudaMemcpyHostToDevice) { // host snapshots: the indices the kernels use are checked like the per-channel setters check them
+    for (uint32_t i = 0; has_fe && i < n; ++i) {
+      int32_t idx;
+      memcpy(&idx, src + h.off[kOffFe] + ((size_t)first + i) * sizeof(fe::State) + offsetof(fe::State, agc_idx), 4);
+      if (idx < 0 || idx > fe::kAgcBuf) return fail(chain, MSDR_ERR_ARGUMENT, "restore: front-end agc_idx outside [0, 25]");
+    }
+    for (uint32_t i = 0; has_anr && i < n; ++i) {
+      int32_t idx;
+      memcpy(&idx, src + h.off[kOffAnrIdx] + ((size_t)first + i) * 4, 4);
+      if (idx < 0 || idx >= 512) return fail(chain, MSDR_ERR_ARGUMENT, "restore: ANR in_idx outside [0, 512)");
+    }
+  }
+  // table slots: the range gives its bindings back (release_sole_sets frees tables only it used), then the snapshot's tables are
+  // interned; count the live tables that would need before anything changes
+  auto same = [&](const FirSet &s, const SnapTable &t) {
+    return s.T == t.T && !memcmp(s.cI.data(), t.cI, t.T * 2) && !memcmp(s.cQ.data(), t.cQ, t.T * 2);
+  };
+  auto same_tab = [](const SnapTable &a, const SnapTable &b) { return a.T == b.T && !memcmp(a.cI, b.cI, a.T * 2) && !memcmp(a.cQ, b.cQ, a.T * 2); };
+  {
+    uint32_t left[MSDR_MAX_FIR_SETS] = {0};
+    for (size_t s = 0; s < chain->sets.size(); ++s) left[s] = chain->sets[s].users;
+    for (uint32_t c = ch0; c < ch0 + n; ++c)
+      if (chain->h_set[c] != kNoTable) left[chain->h_set[c]]--;
+    uint32_t live = 0;
+    for (size_t s = 0; s < chain->sets.size(); ++s) live += left[s] > 0;
+    for (uint32_t k = 0; k < h.n_tables; ++k) {
+      if (!used[k]) continue;
+      bool found = false;
+      for (size_t s = 0; s < chain->sets.size() && !found; ++s) found = left[s] > 0 && same(chain->sets[s], tab[k]);
+      for (uint32_t j = 0; j < k && !found; ++j) found = used[j] && same_tab(tab[j], tab[k]);
+      live += !found;
+    }
+    if (live > MSDR_MAX_FIR_SETS) return fail(chain, MSDR_ERR_NOMEM, "restore: more than MSDR_MAX_FIR_SETS distinct FIR tables in one chain");
+  }
+
+  // ---- from here on the chain changes
+  CK(cudaSetDevice(chain->device));
+  if ((st = snap_wait(chain)) != MSDR_OK) return st;
+  release_sole_sets(chain, [&](auto &&f) { for (uint32_t c = ch0; c < ch0 + n; ++c) f(c); });
+  for (uint32_t c = ch0; c < ch0 + n; ++c)
+    if (chain->h_set[c] != kNoTable) { chain->sets[chain->h_set[c]].users--; chain->h_set[c] = kNoTable; chain->n_uninit++; }
+  uint8_t map[MSDR_MAX_FIR_SETS];
+  chain->snap_ex.resize((size_t)MSDR_MAX_FIR_SETS * chain->set_stride_words);
+  chain->snap_kp4.resize(MSDR_MAX_FIR_SETS);
+  chain->snap_taps.resize((size_t)MSDR_MAX_FIR_SETS * 2 * MSDR_MAX_TAPS);
+  for (uint32_t k = 0; k < h.n_tables; ++k) {
+    if (!used[k]) continue;
+    const SnapTable &t = tab[k];
+    size_t slot = chain->sets.size();
+    for (size_t s = 0; s < chain->sets.size() && slot == chain->sets.size(); ++s)
+      if (chain->sets[s].users > 0 && same(chain->sets[s], t)) slot = s;
+    if (slot == chain->sets.size()) { // a new table: first free slot, uploaded from the staging vectors
+      for (size_t s = 0; s < chain->sets.size(); ++s)
+        if (chain->sets[s].users == 0) { slot = s; break; }
+      if (slot == chain->sets.size()) chain->sets.emplace_back();
+      FirSet &fs = chain->sets[slot];
+      fs.T = t.T;
+      fs.cI.assign(t.cI, t.cI + t.T);
+      fs.cQ.assign(t.cQ, t.cQ + t.T);
+      std::vector<int32_t> ex;
+      expand_set(fs, ex, chain->set_stride_words);
+      int32_t *sx = chain->snap_ex.data() + slot * chain->set_stride_words;
+      std::copy(ex.begin(), ex.end(), sx);
+      chain->snap_kp4[slot] = kp_of_taps(t.T) / 4;
+      int16_t *tp = chain->snap_taps.data() + slot * 2 * MSDR_MAX_TAPS;
+      std::copy(t.cI, t.cI + t.T, tp);
+      std::copy(t.cQ, t.cQ + t.T, tp + MSDR_MAX_TAPS);
+      CK(cudaMemcpyAsync(chain->d_sets + slot * chain->set_stride_words, sx, ex.size() * 4, cudaMemcpyHostToDevice, chain->stream));
+      CK(cudaMemcpyAsync(chain->d_set_kp4 + slot, &chain->snap_kp4[slot], 4, cudaMemcpyHostToDevice, chain->stream));
+      CK(cudaMemcpyAsync(chain->d_set_taps + slot * 2 * MSDR_MAX_TAPS, tp, 2 * MSDR_MAX_TAPS * 2, cudaMemcpyHostToDevice, chain->stream));
+    }
+    chain->sets[slot].users += used[k]; // counted at once: an identical later entry finds this slot
+    map[k] = (uint8_t)slot;
+  }
+  // host mirrors, then the device copies of mode and table id
+  if (has_anr && chain->h_anr.empty()) chain->h_anr.assign(chain->C, 0);
+  std::vector<uint8_t> &hb = chain->snap_host;
+  hb.resize(2 * (size_t)n);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint8_t *m = meta + 4 * i;
+    const uint32_t c = ch0 + i;
+    chain->h_mode[c] = m[0];
+    if (m[1] != kNoTable) { chain->h_set[c] = map[m[1]]; chain->n_uninit--; }
+    if (!chain->h_anr.empty()) { chain->n_anr += (m[2] != 0) - (chain->h_anr[c] != 0); chain->h_anr[c] = m[2]; }
+    hb[i] = chain->h_mode[c];
+    hb[n + i] = chain->h_set[c];
+  }
+  chain->meta_version++;
+  chain->pll.dirty = true; chain->pll.epoch++;
+  cudaStream_t s = chain->stream;
+  CK(cudaMemcpyAsync(chain->d_mode + ch0, hb.data(), n, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(chain->d_set + ch0, hb.data() + n, n, cudaMemcpyHostToDevice, s));
+
+  // state sections: one (2D) copy each; the snapshot side has pitch nch, the chain side Cpad
+  const size_t H = chain->H, Hs = h.hist_len, m = std::min(H, Hs), cp = (size_t)chain->Cpad * 4, sp = (size_t)h.nch * 4, w = (size_t)n * 4;
+  if (Hs == H) {
+    CK(cudaMemcpyAsync(chain->d_hist + (size_t)ch0 * H, src + h.off[kOffHist] + (size_t)first * Hs * 2, (size_t)n * H * 2, kind, s));
+  } else { // the last min(H, hist_len) samples of each row go to the end of the row, the front is zero (msdr_chain_set_state)
+    CK(cudaMemcpy2DAsync(chain->d_hist + (size_t)ch0 * H + (H - m), H * 2, src + h.off[kOffHist] + ((size_t)first * Hs + (Hs - m)) * 2, Hs * 2, m * 2, n,
+                         kind, s));
+    if (H > m) CK(cudaMemset2DAsync(chain->d_hist + (size_t)ch0 * H, H * 2, 0, (H - m) * 2, n, s));
+  }
+  CK(cudaMemcpy2DAsync(chain->d_bq + ch0, cp, src + h.off[kOffBq] + 4 * (size_t)first, sp, w, kBqWords, kind, s));
+  CK(cudaMemcpy2DAsync(chain->d_pll + ch0, cp, src + h.off[kOffPll] + 4 * (size_t)first, sp, w, 3, kind, s));
+
+  if (has_fe || chain->d_fe) {
+    const bool fe_new = !chain->d_fe;
+    if (fe_new) { // the snapshot brings a front end: enable it with its parameters, every other channel starts as enable_frontend starts it
+      CK(cudaMalloc(&chain->d_fe, (size_t)chain->C * sizeof(fe::State)));
+      chain->fe_agc_start = h.agc_start; chain->fe_agc_max = h.agc_max; chain->fe_agc_on = h.agc_on ? 1 : 0;
+    }
+    fe::State &s0 = chain->snap_fe0;
+    s0 = fe::State{};
+    s0.agc_idx = fe::kAgcBuf;                          // .ino:451
+    s0.agc_val = chain->fe_agc_start;                  // .ino:104
+    s0.mult = fe::amp_multiplier(chain->fe_agc_start); // .ino:385
+    if (fe_new) st = replicate(chain, chain->d_fe, sizeof(fe::State), chain->C, &s0);
+    if (st == MSDR_OK && has_fe)
+      CK(cudaMemcpyAsync(chain->d_fe + ch0, src + h.off[kOffFe] + (size_t)first * sizeof(fe::State), (size_t)n * sizeof(fe::State), kind, s));
+    else if (st == MSDR_OK)
+      st = replicate(chain, chain->d_fe + ch0, sizeof(fe::State), n, &s0); // the snapshot has no front end: restored channels start fresh
+    if (st != MSDR_OK) return st;
+  }
+
+  if (has_anr && !chain->d_anr_d) { // LMS arrays on first need, as msdr_chain_set_anr allocates them; every channel starts at the initial state
+    const size_t cpb = (size_t)chain->Cpad * 4;
+    CK(cudaMalloc(&chain->d_anr_d, 512 * cpb)); CK(cudaMalloc(&chain->d_anr_w, 64 * cpb));
+    CK(cudaMalloc(&chain->d_anr_lidx, cpb)); CK(cudaMalloc(&chain->d_anr_ngamma, cpb)); CK(cudaMalloc(&chain->d_anr_idx, cpb));
+    if ((st = anr_initial(chain, 0, chain->Cpad)) != MSDR_OK) return st;
+  }
+  if (has_anr) {
+    CK(cudaMemcpy2DAsync(chain->d_anr_d + ch0, cp, src + h.off[kOffAnrD] + 4 * (size_t)first, sp, w, 512, kind, s));
+    CK(cudaMemcpy2DAsync(chain->d_anr_w + ch0, cp, src + h.off[kOffAnrW] + 4 * (size_t)first, sp, w, 64, kind, s));
+    CK(cudaMemcpyAsync(chain->d_anr_lidx + ch0, src + h.off[kOffAnrLidx] + 4 * (size_t)first, w, kind, s));
+    CK(cudaMemcpyAsync(chain->d_anr_ngamma + ch0, src + h.off[kOffAnrNgamma] + 4 * (size_t)first, w, kind, s));
+    CK(cudaMemcpyAsync(chain->d_anr_idx + ch0, src + h.off[kOffAnrIdx] + 4 * (size_t)first, w, kind, s));
+  } else if (chain->d_anr_d) {
+    if ((st = anr_initial(chain, ch0, n)) != MSDR_OK) return st;
+  }
+  return snap_uploaded(chain);
+}
+
+} // namespace
+
+size_t msdr_chain_snapshot_bytes(const msdr_chain *chain, uint32_t nch)
+{
+  if (!chain || nch == 0) return 0;
+  return snap_layout(nch, chain->H, chain_sections(chain)).total;
+}
+
+int msdr_chain_snapshot(msdr_chain *chain, uint32_t ch0, uint32_t nch, void *buf, size_t bytes)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  SnapLayout l;
+  int st = snap_begin(chain, ch0, nch, bytes, buf, l);
+  if (st != MSDR_OK) return st;
+  snap_build_prefix(chain, ch0, nch, l);
+  memcpy(buf, chain->snap_host.data(), chain->snap_host.size());
+  if ((st = snap_copy_state_out(chain, ch0, nch, static_cast<uint8_t *>(buf), l, cudaMemcpyDeviceToHost)) != MSDR_OK) return st;
+  CK(cudaStreamSynchronize(chain->stream));
+  return MSDR_OK;
+}
+
+int msdr_chain_snapshot_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, void *d_buf, size_t bytes)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  SnapLayout l;
+  int st = snap_begin(chain, ch0, nch, bytes, d_buf, l);
+  if (st != MSDR_OK) return st;
+  snap_build_prefix(chain, ch0, nch, l);
+  uint8_t *d = static_cast<uint8_t *>(d_buf);
+  CK(cudaMemcpyAsync(d, chain->snap_host.data(), chain->snap_host.size(), cudaMemcpyHostToDevice, chain->stream));
+  if ((st = snap_copy_state_out(chain, ch0, nch, d, l, cudaMemcpyDeviceToDevice)) != MSDR_OK) return st;
+  return snap_uploaded(chain);
+}
+
+int msdr_chain_restore(msdr_chain *chain, uint32_t ch0, const void *buf, size_t bytes, uint32_t first, uint32_t n)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (!buf) return fail(chain, MSDR_ERR_ARGUMENT, "restore: buf == NULL");
+  const uint8_t *b = static_cast<const uint8_t *>(buf);
+  // the meta of snapshot channels [first, first+n) must lie inside `bytes` before the header is trusted with anything
+  const uint64_t need = snap_layout(0, 8, 0).off[kOffMeta] + 4 * ((uint64_t)first + n);
+  int st = snap_restore(chain, ch0, b, (size_t)std::min<uint64_t>(bytes, need), b, bytes, first, n, cudaMemcpyHostToDevice);
+  if (st != MSDR_OK) return st;
+  CK(cudaStreamSynchronize(chain->stream)); // the caller may free the blob on return
+  return MSDR_OK;
+}
+
+int msdr_chain_restore_device(msdr_chain *chain, uint32_t ch0, const void *d_buf, size_t bytes, uint32_t first, uint32_t n)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (!d_buf) return fail(chain, MSDR_ERR_ARGUMENT, "restore_device: d_buf == NULL");
+  // header, tables and the meta of the restored channels: one small synchronous read (stream-ordered after the chain's earlier work)
+  const uint64_t need = snap_layout(0, 8, 0).off[kOffMeta] + 4 * ((uint64_t)first + n);
+  const size_t pre = (size_t)std::min<uint64_t>(bytes, need);
+  if (pre < kSnapHeaderBytes) return fail(chain, MSDR_ERR_ARGUMENT, "snapshot: buffer shorter than the 256-byte header");
+  CK(cudaSetDevice(chain->device));
+  std::vector<uint8_t> h(pre);
+  CK(cudaMemcpyAsync(h.data(), d_buf, pre, cudaMemcpyDeviceToHost, chain->stream));
+  CK(cudaStreamSynchronize(chain->stream));
+  return snap_restore(chain, ch0, h.data(), pre, static_cast<const uint8_t *>(d_buf), bytes, first, n, cudaMemcpyDeviceToDevice);
+}
+
+int msdr_snapshot_info(const void *header, size_t bytes, uint32_t *n_channels, uint32_t *max_taps_needed, uint32_t *flags)
+{
+  SnapHeader h;
+  const char *why;
+  const int st = snap_parse_header(header, bytes, h, why);
+  if (st != MSDR_OK) return st;
+  if (n_channels) *n_channels = h.nch;
+  if (max_taps_needed) *max_taps_needed = h.max_taps_needed;
+  if (flags) *flags = h.flags | (h.sections & kSnapFrontend ? MSDR_SNAPSHOT_FRONTEND : 0u) | (h.sections & kSnapAnr ? MSDR_SNAPSHOT_ANR : 0u);
   return MSDR_OK;
 }
 

@@ -6,6 +6,7 @@ chain object; there is NO collective on the data path.  torch.distributed is onl
 and, if asked, to gather results or checksums.
 """
 from dataclasses import dataclass
+from typing import NamedTuple
 
 
 @dataclass(frozen=True)
@@ -31,6 +32,28 @@ def plan(total_channels, world, rank=None, granule=32):
         shards.append(Shard(r, world, ch0, ch1 - ch0))
         g0 += g
     return shards if rank is None else shards[rank]
+
+
+class Piece(NamedTuple):
+    old_rank: int
+    first: int     # first channel of the piece inside old_rank's chain (and snapshot of its whole range)
+    n: int
+    new_rank: int
+    dst_ch0: int   # where the piece goes inside new_rank's chain
+
+
+def reshard(total_channels, old_world, new_world, granule=32):
+    """The pieces that move a plan(total, old_world) layout to plan(total, new_world): every channel in exactly one piece, in global
+    channel order.  Rank r of the new layout restores each piece with new_rank == r from old_rank's snapshot:
+    chain.restore(snapshots[p.old_rank], ch0=p.dst_ch0, first=p.first, n=p.n)."""
+    old, new = plan(total_channels, old_world, granule=granule), plan(total_channels, new_world, granule=granule)
+    pieces = []
+    for o in old:
+        for s in new:
+            lo, hi = max(o.ch0, s.ch0), min(o.ch0 + o.n, s.ch0 + s.n)
+            if hi > lo:
+                pieces.append(Piece(o.rank, lo - o.ch0, hi - lo, s.rank, lo - s.ch0))
+    return pieces
 
 
 def weak_scaling_shard(channels_per_rank, world, rank):
