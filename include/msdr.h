@@ -186,7 +186,6 @@ int msdr_snapshot_info(const void *header, size_t bytes, uint32_t *n_channels, u
  *   8192   never the row-block kernel;    4096   the row-block kernel for any channel count;    32768  its half-tile form for any window
  *          (+1, +2, +4, +8, +12 there: the stage's products as IMAD.WIDE instead of IMAD.HI (the half-tile form: the other way round) /
  *          DFMA feed-forward / chained DFMA / all DFMA / split 16 x 16 bit)
- *   64   CUDA-core FIR kernel (msdr_chain_v3.cu); +1: biquad products on the FP64 pipe; +8: two channels per chain lane
  *   128  helper-warp shape even beyond 148 groups;  2048: post-warp shape (whole stages in the chain warps);
  *   256  classic shape (neither helper nor post warps)
  *   512  never run two chain sets per SM

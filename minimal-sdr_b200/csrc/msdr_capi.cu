@@ -1,5 +1,5 @@
 // msdr_capi.cu — the C ABI declared in include/msdr.h: chain object, configuration, updates, stage operators.
-// Host-side only plumbing; every computation is a CUDA kernel from msdr_chain_kernel.cu / msdr_stage_kernels.cu.
+// Host-side only plumbing; every computation is a CUDA kernel from the msdr_chain_v*.cu / msdr_stage_kernels.cu files.
 #include "../../include/msdr.h"
 #include "msdr_frontend.cuh"
 #include "msdr_internal.h"
@@ -23,31 +23,9 @@ struct FirSet {
   uint32_t users = 0;
 };
 
-// Expand one (cI, cQ) table into the four polyphase sub-filters the fused kernel consumes.
-// Output layout: [kp4 chunks][24 words]: A[4], B[4] as int32 (I branch, IMAD pipe), C[4], D[4] as double (Q branch, DFMA pipe);
-// KP = 4*kp4 = roundup4(T/2 + 1).
+// Split one (cI, cQ) table into the four polyphase sub-filters of the fs/4 mix + FIR pair; KP = roundup4(T/2 + 1).
 // With k' = d - (KP - T/2):  A[d] = cI[2k'], B[d] = cI[2k'+1], C[d] = cQ[2k'+1], D[d] = cQ[2(k'+1)], zero outside.
-// Derivation in DESIGN.md ("Polyphase form of the fs/4 mix + FIR").
-void expand_set(const FirSet &s, std::vector<int32_t> &out, uint32_t stride_words)
-{
-  out.assign(stride_words, 0);
-  const int T = (int)s.T, half = T / 2, KP = (int)kp_of_taps(s.T);
-  for (int d = 0; d < KP; ++d) {
-    const int kq = d - (KP - half);
-    int a = 0, b = 0, c = 0, dd = 0;
-    if (kq >= 0 && kq < half) { a = s.cI[2 * kq]; b = s.cI[2 * kq + 1]; c = s.cQ[2 * kq + 1]; }
-    if (kq + 1 >= 0 && kq + 1 < half) dd = s.cQ[2 * (kq + 1)];
-    const int chunk = d / 4, t = d % 4;
-    int32_t *w = out.data() + (size_t)chunk * 24;
-    w[0 + t] = a;
-    w[4 + t] = b;
-    const double cd = (double)c, ddd = (double)dd;
-    memcpy(w + 8 + 2 * t, &cd, 8);
-    memcpy(w + 16 + 2 * t, &ddd, 8);
-  }
-}
-
-// Same sub-filters as plain ints (tensor-core study operand builder).
+// Derivation in DESIGN.md ("Polyphase form of the fs/4 mix + FIR"); tc_build_bmat turns them into the Toeplitz operands.
 void expand_set_int(uint32_t T, const int16_t *cI, const int16_t *cQ, std::vector<int> &A, std::vector<int> &B, std::vector<int> &C, std::vector<int> &D)
 {
   const int half = (int)T / 2, KP = (int)kp_of_taps(T);
@@ -77,17 +55,11 @@ struct msdr_chain {
   std::vector<uint8_t> h_mode, h_set; // h_set: 0xFF = FIR not initialised
   uint32_t n_uninit = 0;
   std::vector<FirSet> sets;
-  uint32_t set_stride_words = 0;
 
   uint8_t *d_mode = nullptr, *d_set = nullptr;
   int16_t *d_hist = nullptr;
   int32_t *d_bq = nullptr;
-  int32_t *d_sets = nullptr;
-  uint32_t *d_set_kp4 = nullptr;
-  int *d_ctrl = nullptr;
-  int *d_tile_flags = nullptr; // [groups][tiles] of the largest launch so far
-  size_t tile_flags_len = 0;
-  uint32_t epoch = 0;
+  int *d_ctrl = nullptr;       // [2] chain kernel v4: work counter, spans taken
 
   // staging for host-buffer updates
   int16_t *d_in = nullptr, *d_out = nullptr;
@@ -100,13 +72,13 @@ struct msdr_chain {
   struct TcPlan {
     uint64_t version = 0;
     uint32_t ch0 = 0, nch = 0, sms = 0, W = 0, K = 0, rings[4] = {0, 0, 0, 0}, n_rb = 0, n_waves = 0;
-    bool usable = false, want_dual = false, dual = false;
+    bool want_dual = false, want_v6 = false, dual = false;
     uint32_t ring_v5 = 0;  // msdr_chain_v5.cu: operand ring depth, 0 = the window does not fit that kernel
     uint32_t ring_v5l = 0; // msdr_chain_v5l.cu (half-tile hand-offs, for the 256-tap window)
     uint32_t slots_v6 = 0, n_gb = 0; // msdr_chain_v6.cu: sub-tile slots (0 = the window does not fit), group blocks of 32 same-table rows
     uint32_t *d_rowmap32 = nullptr;
     uint4 *d_rb32 = nullptr;
-    uint32_t *d_rowmap = nullptr, *d_grp = nullptr, *d_wave_rb0 = nullptr;
+    uint32_t *d_rowmap = nullptr, *d_wave_rb0 = nullptr;
     uint4 *d_rb = nullptr;
     uint8_t *d_bmat = nullptr;
   };
@@ -156,8 +128,6 @@ struct msdr_chain {
   // snapshots (msdr_chain_snapshot* / msdr_chain_restore*): host vectors their asynchronous uploads read from; `snap_ev` marks the
   // last such upload, and the next snapshot or restore waits for it before it writes them again
   std::vector<uint8_t> snap_host;
-  std::vector<int32_t> snap_ex;
-  std::vector<uint32_t> snap_kp4;
   std::vector<int16_t> snap_taps;
   fe::State snap_fe0{};
   cudaEvent_t snap_ev = nullptr;
@@ -207,19 +177,11 @@ int usage_resolve(msdr_chain *chain)
 
 int upload_set(msdr_chain *chain, uint32_t id)
 {
-  std::vector<int32_t> ex;
-  expand_set(chain->sets[id], ex, chain->set_stride_words);
-  const uint32_t kp4 = kp_of_taps(chain->sets[id].T) / 4;
-  CK(cudaMemcpyAsync(chain->d_sets + (size_t)id * chain->set_stride_words, ex.data(), ex.size() * sizeof(int32_t), cudaMemcpyHostToDevice,
-                     chain->stream));
-  CK(cudaMemcpyAsync(chain->d_set_kp4 + id, &kp4, sizeof(kp4), cudaMemcpyHostToDevice, chain->stream));
-  {
-    const FirSet &fs = chain->sets[id];
-    int16_t *dst = chain->d_set_taps + (size_t)id * 2 * MSDR_MAX_TAPS;
-    CK(cudaMemcpyAsync(dst, fs.cI.data(), fs.T * 2, cudaMemcpyHostToDevice, chain->stream));
-    CK(cudaMemcpyAsync(dst + MSDR_MAX_TAPS, fs.cQ.data(), fs.T * 2, cudaMemcpyHostToDevice, chain->stream));
-  }
-  CK(cudaStreamSynchronize(chain->stream)); // `ex` and `kp4` are stack/heap temporaries
+  const FirSet &fs = chain->sets[id];
+  int16_t *dst = chain->d_set_taps + (size_t)id * 2 * MSDR_MAX_TAPS;
+  CK(cudaMemcpyAsync(dst, fs.cI.data(), fs.T * 2, cudaMemcpyHostToDevice, chain->stream));
+  CK(cudaMemcpyAsync(dst + MSDR_MAX_TAPS, fs.cQ.data(), fs.T * 2, cudaMemcpyHostToDevice, chain->stream));
+  CK(cudaStreamSynchronize(chain->stream)); // the taps' vectors may be reassigned as soon as this returns
   chain->meta_version++;
   return MSDR_OK;
 }
@@ -321,7 +283,6 @@ int msdr_chain_create(msdr_chain **out, int device, uint32_t n_channels, uint32_
   chain->KPmax = kp_of_taps(max_taps);
   chain->H = hist_of_kp(chain->KPmax);
   chain->flags = flags;
-  chain->set_stride_words = chain->KPmax / 4 * 24; // kp4 chunks x 24 words
   chain->h_mode.assign(n_channels, (uint8_t)MSDR_MODE_AM);
   chain->h_set.assign(n_channels, 0xFF);
   chain->n_uninit = n_channels;
@@ -345,16 +306,12 @@ int msdr_chain_create(msdr_chain **out, int device, uint32_t n_channels, uint32_
   CKC(cudaMalloc(&chain->d_bq, (size_t)kBqWords * chain->Cpad * sizeof(int32_t)));
   CKC(cudaMalloc(&chain->d_pll, (size_t)3 * chain->Cpad * sizeof(float)));
   CKC(cudaMemsetAsync(chain->d_pll, 0, (size_t)3 * chain->Cpad * sizeof(float), chain->own_stream));
-  CKC(cudaMalloc(&chain->d_sets, (size_t)MSDR_MAX_FIR_SETS * chain->set_stride_words * sizeof(int32_t)));
-  CKC(cudaMalloc(&chain->d_set_kp4, MSDR_MAX_FIR_SETS * sizeof(uint32_t)));
   CKC(cudaMalloc(&chain->d_set_taps, (size_t)MSDR_MAX_FIR_SETS * 2 * MSDR_MAX_TAPS * sizeof(int16_t)));
-  CKC(cudaMalloc(&chain->d_ctrl, (size_t)(1 + chain->Cpad / kGroup + 1) * sizeof(int)));
+  CKC(cudaMalloc(&chain->d_ctrl, 2 * sizeof(int)));
   CKC(cudaMemsetAsync(chain->d_mode, MSDR_MODE_AM, n_channels, chain->stream));
   CKC(cudaMemsetAsync(chain->d_set, 0, n_channels, chain->stream));
   CKC(cudaMemsetAsync(chain->d_hist, 0, (size_t)n_channels * chain->H * sizeof(int16_t), chain->stream));
   CKC(cudaMemsetAsync(chain->d_bq, 0, (size_t)kBqWords * chain->Cpad * sizeof(int32_t), chain->stream));
-  CKC(cudaMemsetAsync(chain->d_sets, 0, (size_t)MSDR_MAX_FIR_SETS * chain->set_stride_words * sizeof(int32_t), chain->stream));
-  CKC(cudaMemsetAsync(chain->d_set_kp4, 0, MSDR_MAX_FIR_SETS * sizeof(uint32_t), chain->stream));
   CKC(cudaStreamSynchronize(chain->stream));
 #undef CKC
   *out = chain;
@@ -367,13 +324,13 @@ void msdr_chain_destroy(msdr_chain *chain)
   cudaSetDevice(chain->device);
   if (chain->stream) cudaStreamSynchronize(chain->stream);
   cudaFree(chain->d_mode); cudaFree(chain->d_set); cudaFree(chain->d_hist); cudaFree(chain->d_bq);
-  for (auto &pl : chain->plans) { cudaFree(pl.d_rowmap); cudaFree(pl.d_grp); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); }
+  for (auto &pl : chain->plans) { cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32); }
   cudaFree(chain->d_tile_cnt); cudaFree(chain->d_pll);
   cudaFree(chain->d_anr_d); cudaFree(chain->d_anr_w); cudaFree(chain->d_anr_lidx); cudaFree(chain->d_anr_ngamma); cudaFree(chain->d_anr_idx);
   cudaFree(chain->pll.d_kind); cudaFree(chain->pll.d_anr_mode);
   cudaFree(chain->pll.d_rows); cudaFree(chain->pll.d_chmap); cudaFree(chain->pll.d_raw); cudaFree(chain->pll.d_I); cudaFree(chain->pll.d_Q);
   cudaFree(chain->pll.d_If); cudaFree(chain->pll.d_Qf); cudaFree(chain->pll.d_taps); cudaFree(chain->pll.d_defs);
-  cudaFree(chain->d_sets); cudaFree(chain->d_set_kp4); cudaFree(chain->d_set_taps); cudaFree(chain->d_ctrl); cudaFree(chain->d_tile_flags);
+  cudaFree(chain->d_set_taps); cudaFree(chain->d_ctrl);
   cudaFree(chain->d_in); cudaFree(chain->d_out);
   cudaFree(chain->d_fe); cudaFree(chain->d_fe_if);
   if (chain->pin_in) cudaFreeHost(chain->pin_in);
@@ -603,22 +560,34 @@ namespace {
 
 void free_tc_plan(msdr_chain::TcPlan &pl)
 {
-  cudaFree(pl.d_rowmap); cudaFree(pl.d_grp); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32);
+  cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32);
   pl = msdr_chain::TcPlan{};
 }
 
 // Row plan of the tensor-core chain kernel for the channel range [ch0, ch0 + nch).  All 128 rows of a GEMM tile share the
 // B operand, i.e. one tap table, and a chain wave (W groups of 32 channels, one per CTA) must get its FIR input first; so
 // inside each wave the rows are sorted by table and cut into blocks of 128 (the last block of a table is padded).
-// Every block lists the channel groups it contributes to and with how many rows: the epilogue adds those counts to
-// tile_cnt[group][span], a chain starts a span when the count reaches the group's row count.
+// The epilogue finds each row's channel group in the row map and adds the group's rows to tile_cnt[group][unit]; a chain starts
+// a unit when the count reaches the group's row count.
 // want_dual: the caller would like waves of 2 x sms chains (two chain sets per SM); the plan is built with that width only if the
 // window leaves room for the second set of chain slots (rings[3]), which is known before any row is sorted — so the wave width
 // is chosen once and an unchanged configuration always hits the cache (256 taps beyond 148 groups used to rebuild twice per update).
-int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, bool want_dual, const msdr_chain::TcPlan **out)
+// want_v6: also the group-block plan of the time-folded kernel (msdr_chain_v6.cu), if the window fits that kernel.
+int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, bool want_dual, bool want_v6, const msdr_chain::TcPlan **out)
 {
   for (const auto &c : chain->plans)
-    if (c.version == chain->meta_version && c.ch0 == ch0 && c.nch == nch && c.sms == sms && c.want_dual == want_dual) { *out = &c; return MSDR_OK; }
+    if (c.version == chain->meta_version && c.ch0 == ch0 && c.nch == nch && c.sms == sms && c.want_dual == want_dual && c.want_v6 == want_v6) {
+      *out = &c;
+      return MSDR_OK;
+    }
+  uint32_t kp_max = 0;
+  for (uint32_t c = ch0; c < ch0 + nch; ++c) kp_max = std::max(kp_max, kp_of_taps(chain->sets[chain->h_set[c]].T));
+  const uint32_t K = tc_window_words_kp(kp_max);
+  int smem_max = 0;
+  CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, chain->device));
+  uint32_t rings[4];
+  if (!chain_v4_config(K, smem_max, rings)) // every window of up to MSDR_MAX_TAPS taps fits on a B200
+    return fail(chain, MSDR_ERR_UNSUPPORTED, "update: the FIR window of " + std::to_string(K) + " words does not fit the chain kernel's shared memory");
   CK(cudaStreamSynchronize(chain->stream)); // a launch in flight may still read the plan that is replaced
   size_t slot = chain->plans.size();
   for (size_t i = 0; i < chain->plans.size(); ++i)
@@ -631,24 +600,17 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
   free_tc_plan(pl);
   *out = &pl;
   chain->plan_builds++;
-  pl.version = chain->meta_version; pl.ch0 = ch0; pl.nch = nch; pl.sms = sms; pl.want_dual = want_dual;
-
-  uint32_t kp_max = 0;
-  for (uint32_t c = ch0; c < ch0 + nch; ++c) kp_max = std::max(kp_max, kp_of_taps(chain->sets[chain->h_set[c]].T));
-  const uint32_t K = tc_window_words_kp(kp_max);
-  int smem_max = 0;
-  CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, chain->device));
-  if (!chain_v4_config(K, smem_max, pl.rings)) { pl.usable = false; return MSDR_OK; }
+  pl.version = chain->meta_version; pl.ch0 = ch0; pl.nch = nch; pl.sms = sms; pl.want_dual = want_dual; pl.want_v6 = want_v6;
+  std::copy(rings, rings + 4, pl.rings);
   pl.K = K;
   pl.ring_v5 = chain_v5_config(K, smem_max);
   pl.ring_v5l = chain_v5l_config(K, smem_max);
-  // (the time-folded kernel takes one group block per SM at most: no point in its row plan for wide ranges unless a study variant forces it)
-  pl.slots_v6 = (nch <= 8192u || (chain->variant & 65536)) ? chain_v6_config(K, smem_max) : 0u;
+  pl.slots_v6 = want_v6 ? chain_v6_config(K, smem_max) : 0u;
   pl.dual = want_dual && pl.rings[3] != 0;
   const uint32_t W = pl.W = sms * (pl.dual ? 2u : 1u);
 
   const uint32_t NG = (nch + kGroup - 1) / kGroup, n_sets = (uint32_t)chain->sets.size(), M = tc_tile_rows();
-  std::vector<uint32_t> rowmap, grp, wave_rb0;
+  std::vector<uint32_t> rowmap, wave_rb0;
   std::vector<uint4> rbs;
   std::vector<std::vector<uint32_t>> bucket(n_sets);
   wave_rb0.push_back(0);
@@ -659,16 +621,8 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
     for (uint32_t sid = 0; sid < n_sets; ++sid) {
       const std::vector<uint32_t> &rows = bucket[sid];
       for (size_t i0 = 0; i0 < rows.size(); i0 += M) {
-        const size_t i1 = std::min(rows.size(), i0 + M);
-        const uint32_t grp_off = (uint32_t)grp.size();
-        for (size_t i = i0; i < i1; ++i) {
-          rowmap.push_back(rows[i]);
-          const uint32_t g = rows[i] / kGroup;
-          if (grp.size() > grp_off && (grp.back() & 0xFFFFFFu) == g) grp.back() += 1u << 24;
-          else grp.push_back(g | (1u << 24));
-        }
-        for (size_t i = i1; i < i0 + M; ++i) rowmap.push_back(0xFFFFFFFFu);
-        rbs.push_back(make_uint4(sid, grp_off, (uint32_t)grp.size() - grp_off, (uint32_t)wave_rb0.size() - 1));
+        for (size_t i = i0; i < i0 + M; ++i) rowmap.push_back(i < rows.size() ? rows[i] : 0xFFFFFFFFu);
+        rbs.push_back(make_uint4(sid, 0, 0, 0));
       }
     }
     wave_rb0.push_back((uint32_t)rbs.size());
@@ -730,10 +684,9 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
     expand_set_int(fs.T, fs.cI.data(), fs.cQ.data(), A, B, C, D);
     tc_build_bmat(A.data(), B.data(), C.data(), D.data(), kp_of_taps(fs.T), K, bm.data() + bsz * sid);
   }
-  CK(cudaMalloc(&pl.d_rowmap, rowmap.size() * 4)); CK(cudaMalloc(&pl.d_grp, std::max<size_t>(grp.size(), 1) * 4));
+  CK(cudaMalloc(&pl.d_rowmap, rowmap.size() * 4));
   CK(cudaMalloc(&pl.d_wave_rb0, wave_rb0.size() * 4)); CK(cudaMalloc(&pl.d_rb, rbs.size() * sizeof(uint4))); CK(cudaMalloc(&pl.d_bmat, bm.size()));
   CK(cudaMemcpyAsync(pl.d_rowmap, rowmap.data(), rowmap.size() * 4, cudaMemcpyHostToDevice, chain->stream));
-  CK(cudaMemcpyAsync(pl.d_grp, grp.data(), grp.size() * 4, cudaMemcpyHostToDevice, chain->stream));
   CK(cudaMemcpyAsync(pl.d_wave_rb0, wave_rb0.data(), wave_rb0.size() * 4, cudaMemcpyHostToDevice, chain->stream));
   CK(cudaMemcpyAsync(pl.d_rb, rbs.data(), rbs.size() * sizeof(uint4), cudaMemcpyHostToDevice, chain->stream));
   CK(cudaMemcpyAsync(pl.d_bmat, bm.data(), bm.size(), cudaMemcpyHostToDevice, chain->stream));
@@ -746,7 +699,6 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
   // the legacy stream, and the chain's stream is non-blocking - a kernel launched right after could read the plan before it had
   // arrived (seen as intermittent mismatches in the last, ragged channel chunk of msdr_chain_update).
   CK(cudaStreamSynchronize(chain->stream));
-  pl.usable = true;
   return MSDR_OK;
 }
 
@@ -876,6 +828,126 @@ int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, int16_t *d_out, size_t s
   return MSDR_OK;
 }
 
+// ---- the kernel choice -------------------------------------------------------------------------------------------------------
+// variant bits the choice reads (study and parity-test knobs, include/msdr.h); the kernels read their own stage-form and ablation bits
+constexpr int kV4Helper = 128;       // v4: the feed-forward helper-warp shape even beyond one channel group per SM
+constexpr int kV4Classic = 256;      // v4: the classic shape (neither helper nor post warps)
+constexpr int kV4OneSet = 512;       // v4: never two chain sets per SM
+constexpr int kV4Post = 2048;        // v4: the post-warp shape (whole stages in the chain warps)
+constexpr int kForceV5 = 4096;       // the row-block kernel for any channel count
+constexpr int kNoV5 = 8192;          // never the row-block kernel
+constexpr int kNoV6 = 16384;         // never the time-folded kernel
+constexpr int kV5lAnyWindow = 32768; // the row-block kernel's half-tile form for any window
+constexpr int kForceV6 = 65536;      // the time-folded kernel for any channel count
+constexpr int kV4Study = kV4Helper | kV4Classic | kV4OneSet | kV4Post; // any of these: v4, one chain set per SM
+
+enum Kernel { kV6, kV4, kV5, kV5l };
+struct Choice {
+  Kernel kernel = kV4;
+  const msdr_chain::TcPlan *plan = nullptr;
+  uint32_t shape = 0; // v4 (tc_ff): 0 post warps, 1 classic, 2 feed-forward helper warps, 3 two chain sets per SM
+};
+
+// The fused kernel for the range [ch0, ch0 + nch) of NG channel groups on `sms` SMs, and the row plan it runs from.
+int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t NG, int sms, Choice &ch)
+{
+  const int v = chain->variant;
+  // Many channels: the row-block kernel (msdr_chain_v5.cu), one CTA per 128 channels of one tap table walking through time.  It
+  // needs enough row blocks to fill the SMs (kV5MinChannels: below that the pinned chains of msdr_chain_v4.cu win).
+  // (more channel groups than one wave of two chain sets per SM holds - 9472 channels on 148 SMs - would make msdr_chain_v4.cu walk a
+  // second, mostly empty wave: 11 264 channels 172 Gsamples/s there against ~200 here)
+  const uint32_t kV5MinChannels = std::min<uint32_t>(12288u, 2u * (uint32_t)sms * (uint32_t)kGroup + 1u);
+  if (((v & kForceV5) || nch >= kV5MinChannels) && !(v & (kNoV5 | kV4Study))) {
+    // does the longest live table's window fit that kernel at all?  (known without sorting a single row: 256 taps do not)
+    int smem_max = 0;
+    CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, chain->device));
+    uint32_t kp_live = 0;
+    for (const FirSet &fs : chain->sets)
+      if (fs.users) kp_live = std::max(kp_live, kp_of_taps(fs.T));
+    const uint32_t K = tc_window_words_kp(kp_live);
+    if (chain_v5_config(K, smem_max) || chain_v5l_config(K, smem_max)) { // a plan with ONE wave: rows sorted by table over the range
+      const int st = build_tc_plan(chain, ch0, nch, NG, false, false, &ch.plan);
+      if (st != MSDR_OK) return st;
+      const msdr_chain::TcPlan &pl = *ch.plan;
+      if (pl.ring_v5 || pl.ring_v5l) { // else no row-block form fits this window: the kernels below
+        ch.kernel = !pl.ring_v5 || ((v & kV5lAnyWindow) && pl.ring_v5l) ? kV5l : kV5; // 256 taps: the half-tile form
+        return MSDR_OK;
+      }
+    }
+  }
+  // Few channels: the time-folded kernel (msdr_chain_v6.cu), one CTA per 32 same-table channels, nothing leaves the SM.  One group
+  // block per SM: a second round would double the launch, and beyond that the two chain sets per SM of msdr_chain_v4.cu (then the
+  // row-block kernel) are faster, so its plan is only asked for up to 8192 channels unless kForceV6 runs it anyway.
+  const bool want_v6 = !(v & (kNoV6 | kV4Study)) && (nch <= 8192u || (v & kForceV6));
+  // more channel groups than SMs: two chain sets per SM (waves of 2 x SMs groups)
+  const bool want_dual = NG > (uint32_t)sms && !(v & kV4Study);
+  const int st = build_tc_plan(chain, ch0, nch, (uint32_t)sms, want_dual, want_v6, &ch.plan);
+  if (st != MSDR_OK) return st;
+  const msdr_chain::TcPlan &pl = *ch.plan;
+  if (pl.slots_v6 && ((v & kForceV6) || pl.n_gb <= (uint32_t)std::max(1, sms - (int)chain->spare_sms))) {
+    ch.kernel = kV6;
+    return MSDR_OK;
+  }
+  // v4 shape: feed-forward helper warps where they fit, else post warps, else the plain classic shape; two chain sets per SM when
+  // the plan has them (false when the second set of chain slots does not fit next to the window: 256 taps)
+  ch.kernel = kV4;
+  ch.shape = pl.rings[2] ? 2u : pl.rings[0] ? 0u : 1u;
+  if ((v & kV4Post) && pl.rings[0]) ch.shape = 0u;
+  if ((v & kV4Classic) && pl.rings[1]) ch.shape = 1u;
+  if ((v & kV4Helper) && pl.rings[2]) ch.shape = 2u;
+  if (pl.dual) ch.shape = 3u;
+  return MSDR_OK;
+}
+
+// msdr_chain_last_kernel names "msdr::<ns>::chain_kernel (fused mix + ...; <form>)"; MSDR_PROF prints role r's counters i = 0..3,
+// which each kernel keeps at prof[cta * 64 + r * 4 + i]
+struct KernelNames {
+  const char *ns, *form;   // v4: the form is the shape's name
+  const char *prof, *items; // MSDR_PROF header "<prof> grid g[, n <items>], ..."
+  int n_roles;
+  const char *role[9];
+};
+const KernelNames kNames[4] = {
+    {"v6", "one CTA per 32-channel group block, tile rows folded over time", "[msdr prof v6]", "group blocks", 9,
+     {"convert", "mma", "epilogue", "chainA", "chainB", "load", "store", "ff1", "ff2"}},
+    {"v4", nullptr, "[msdr prof]", nullptr, 8, {"convert", "mma", "epilogue", "chainA", "chainB", "load", "store", "ff2/post"}},
+    {"v5", "one CTA per 128-channel row block", "[msdr prof v5]", "row blocks", 7, {"convert", "mma", "epilogue", "biquad1", "biquad2", "load", "store"}},
+    {"v5l", "one CTA per 128-channel row block, half-tile hand-offs for the long window", "[msdr prof v5]", "row blocks", 7,
+     {"convert", "mma", "epilogue", "biquad1", "biquad2", "load", "store"}},
+};
+const char *const kV4ShapeNames[4] = {"post-warp shape", "classic shape", "feed-forward helper-warp shape", "two chain sets per SM"};
+
+// MSDR_PROF (developer aid): the mean of every role's counters over the g CTAs on stderr; the time-folded kernel adds their maxima,
+// the time from kernel entry to the end of chain B and, with MSDR_PROF_CTAS, one line per CTA
+int prof_dump(msdr_chain *chain, Kernel k, long long *d_prof, uint32_t g, uint32_t items)
+{
+  const KernelNames &kn = kNames[k];
+  std::vector<long long> h((size_t)g * 64);
+  CK(cudaMemcpyAsync(h.data(), d_prof, h.size() * sizeof(long long), cudaMemcpyDeviceToHost, chain->stream));
+  CK(cudaStreamSynchronize(chain->stream));
+  cudaFree(d_prof);
+  auto at = [&](uint32_t b, int i) { return h[(size_t)b * 64 + i]; };
+  if (kn.items) fprintf(stderr, "%s grid %u, %u %s, mean cycles per CTA (counter 0..3):\n", kn.prof, g, items, kn.items);
+  else fprintf(stderr, "%s grid %u, mean cycles per CTA (counter 0..3):\n", kn.prof, g);
+  for (int r = 0; r < kn.n_roles; ++r) {
+    double m[4] = {0, 0, 0, 0}, mx[4] = {0, 0, 0, 0};
+    for (uint32_t b = 0; b < g; ++b)
+      for (int i = 0; i < 4; ++i) { m[i] += (double)at(b, r * 4 + i) / g; mx[i] = std::max(mx[i], (double)at(b, r * 4 + i)); }
+    fprintf(stderr, "  %-9s %10.0f %10.0f %10.0f %10.0f", kn.role[r], m[0], m[1], m[2], m[3]);
+    if (k == kV6) fprintf(stderr, "   max %10.0f %10.0f %10.0f %10.0f", mx[0], mx[1], mx[2], mx[3]);
+    fprintf(stderr, "\n");
+  }
+  if (k != kV6) return MSDR_OK;
+  double c = 0, n = 0, cm = 0, nm = 0;
+  for (uint32_t b = 0; b < g; ++b) { c += (double)at(b, 40) / g; n += (double)at(b, 41) / g; cm = std::max(cm, (double)at(b, 40)); nm = std::max(nm, (double)at(b, 41)); }
+  fprintf(stderr, "  kernel entry -> chain B done: %.0f cycles, %.0f ns (mean); max %.0f cycles, %.0f ns\n", c, n, cm, nm);
+  if (getenv("MSDR_PROF_CTAS")) // per-CTA totals of chain A (wait, work) and the epilogue
+    for (uint32_t b = 0; b < g; ++b)
+      fprintf(stderr, "  cta %3u sm %3lld start %8lld ns total %9lld cyc  chainA %9lld %9lld %9lld  ff1 %9lld %9lld yfull %9lld  epilogue %9lld %9lld %9lld %9lld\n", b,
+              at(b, 42), at(b, 43) - h[43], at(b, 40), at(b, 12), at(b, 13), at(b, 14), at(b, 28), at(b, 29), at(b, 31), at(b, 8), at(b, 9), at(b, 10), at(b, 11));
+  return MSDR_OK;
+}
+
 // d_adc != NULL: the rows are raw ADC codes for the chain's front end.  Where the int16 input would run the row-block kernels and no
 // channel of the range is on the side lane (which gathers IF samples from `d_in`), the front end runs inside their converters; in
 // every other case K4 conditions the range into a scratch buffer first and the int16 path follows.  Both are bit-exact.
@@ -893,33 +965,15 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d
   CK(cudaSetDevice(chain->device));
   chain->fe_composed = false;
 
-  ChainParams p{};
-  p.in = d_in; p.out = d_out; p.stride = stride;
-  p.C = nch; p.ch0 = ch0; p.Cpad = chain->Cpad; p.L = (uint32_t)L64; p.H = chain->H;
-  p.hist = chain->d_hist; p.bq = chain->d_bq; p.mode = chain->d_mode; p.setid = chain->d_set;
-  p.sets = chain->d_sets; p.set_kp4 = chain->d_set_kp4;
-  p.n_sets = (uint32_t)chain->sets.size(); p.set_stride_words = chain->set_stride_words;
-  p.ctrl = chain->d_ctrl;
-  p.am_q31 = (chain->flags & MSDR_FLAG_AM_Q31) ? 1u : 0u;
-  p.spare_sms = chain->spare_sms;
+  int sms = 0;
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, chain->device));
   const uint32_t NG = (nch + kGroup - 1) / kGroup;
-  const size_t n_flags = (size_t)NG * ((p.L + chain_tile_samples() - 1) / chain_tile_samples());
-  if (n_flags > chain->tile_flags_len || chain->epoch >= 0x7FFFFFF0u) { // (re)allocate zeroed flags; epochs restart
-    CK(cudaStreamSynchronize(chain->stream));
-    if (chain->d_tile_flags) cudaFree(chain->d_tile_flags);
-    chain->d_tile_flags = nullptr;
-    chain->tile_flags_len = 0;
-    const size_t len = std::max(n_flags, chain->tile_flags_len) + 1024;
-    CK(cudaMalloc(&chain->d_tile_flags, len * sizeof(int)));
-    CK(cudaMemsetAsync(chain->d_tile_flags, 0, len * sizeof(int), chain->stream));
-    chain->tile_flags_len = len;
-    chain->epoch = 0;
-  }
-  p.tile_flags = chain->d_tile_flags;
-  p.epoch = ++chain->epoch;
-  CK(cudaMemsetAsync(chain->d_ctrl, 0, (size_t)(1 + NG) * sizeof(int), chain->stream));
-  // ADC codes outside the fused path: K4 over the range into the scratch rows (same stride as `d_out`), then the int16 path reads them
-  auto compose = [&]() -> int {
+  Choice ch;
+  int st = choose_kernel(chain, ch0, nch, NG, sms, ch);
+  if (st != MSDR_OK) return st;
+  const msdr_chain::TcPlan &pl = *ch.plan;
+  if (d_adc && ((ch.kernel != kV5 && ch.kernel != kV5l) || side_lane_in_range(chain, ch0, nch))) {
+    // K4 over the range into the scratch rows (same stride as `d_out`), then the int16 path reads them
     const size_t need = (size_t)nch * stride;
     if (need > chain->fe_if_samples) {
       CK(cudaStreamSynchronize(chain->stream));
@@ -930,260 +984,84 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d
     }
     CK(launch_frontend(d_adc, chain->d_fe_if, stride, nch, n_blocks, chain->d_fe + ch0, chain->fe_agc_max, chain->fe_agc_on, 0, chain->stream));
     chain->launches++;
-    d_in = chain->d_fe_if; p.in = d_in;
+    d_in = chain->d_fe_if;
     d_adc = nullptr;
     chain->fe_composed = true;
-    return MSDR_OK;
-  };
-  bool use_tc = (chain->variant & 64) == 0; // variant bit 6: force the CUDA-core FIR kernel (msdr_chain_v3.cu)
-  if (d_adc && !use_tc) {
-    const int stc = compose();
-    if (stc != MSDR_OK) return stc;
   }
-  if (use_tc) { // tensor-core FIR producers (msdr_chain_v4.cu)
-    int sms = 0;
-    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, chain->device));
-    // more channel groups than SMs: two chain sets per SM (waves of 2 x SMs groups), unless a study variant asks for a
-    // specific shape (bits 7, 8) or forbids it (bit 9)
-    const bool want_dual = NG > (uint32_t)sms && !(chain->variant & (128 | 256 | 512 | 2048));
-    // Many channels: the row-block kernel (msdr_chain_v5.cu), one CTA per 128 channels of one tap table walking through time.  It
-    // needs enough row blocks to fill the SMs (kV5MinChannels: below that the pinned chains of msdr_chain_v4.cu win);
-    // variant bit 12 forces it for any channel count (parity tests), bit 13 forbids it.
-    // (more channel groups than one wave of two chain sets per SM holds - 9472 channels on 148 SMs - would make msdr_chain_v4.cu walk a
-    // second, mostly empty wave: 11 264 channels 172 Gsamples/s there against ~200 here)
-    const uint32_t kV5MinChannels = std::min<uint32_t>(12288u, 2u * (uint32_t)sms * (uint32_t)kGroup + 1u);
-    bool use_v5 = ((chain->variant & 4096) || nch >= kV5MinChannels) && !(chain->variant & (8192 | 128 | 256 | 512 | 2048));
-    if (use_v5) { // does the longest live table's window fit that kernel at all?  (known without sorting a single row: 256 taps do not)
-      int smem_max = 0;
-      CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, chain->device));
-      uint32_t kp_live = 0;
-      for (const FirSet &fs : chain->sets)
-        if (fs.users) kp_live = std::max(kp_live, kp_of_taps(fs.T));
-      if (!chain_v5_config(tc_window_words_kp(kp_live), smem_max) && !chain_v5l_config(tc_window_words_kp(kp_live), smem_max)) use_v5 = false;
-    }
-    const msdr_chain::TcPlan *plp = nullptr;
-    int st = MSDR_OK;
-    if (use_v5) { // a plan with ONE wave: rows sorted by table over the whole range (wave width = all groups)
-      st = build_tc_plan(chain, ch0, nch, NG, false, &plp);
-      if (st != MSDR_OK) return st;
-      if (!plp->usable || (!plp->ring_v5 && !plp->ring_v5l)) use_v5 = false; // no row-block form fits this window: the chain kernel below
-    }
-    if (use_v5) {
-      const msdr_chain::TcPlan &pl = *plp;
-      p.NG = NG;
-      p.n_items = pl.n_rb;
-      p.tc_rowmap = pl.d_rowmap; p.tc_rb = pl.d_rb; p.tc_grp = pl.d_grp; p.tc_wave_rb0 = pl.d_wave_rb0; p.tc_bmat = pl.d_bmat;
-      const bool long_window = !pl.ring_v5 || ((chain->variant & 32768) && pl.ring_v5l); // 256 taps: the half-tile form (bit 15: study, any window)
-      p.tc_K = pl.K; p.tc_ring = long_window ? pl.ring_v5l : pl.ring_v5;
-      if (d_adc && side_lane_in_range(chain, ch0, nch)) {
-        const int stc = compose();
-        if (stc != MSDR_OK) return stc;
-      }
-      if (d_adc) { // fused: the converters read codes and condition them (msdr_chain_v5_common.cuh: FeRow)
-        p.in = reinterpret_cast<const int16_t *>(d_adc);
-        p.fe = chain->d_fe; p.agc_max = chain->fe_agc_max; p.agc_on = chain->fe_agc_on ? 1u : 0u;
-      }
-      if (chain->timed) {
-        int stu = usage_resolve(chain);
-        if (stu != MSDR_OK) return stu;
-        CK(cudaEventRecord(chain->ev0, chain->stream));
-      }
-      {
-        int stl = syncam_lane_prepare(chain, ch0, nch, d_in, stride, p.L);
-        if (stl != MSDR_OK) return stl;
-      }
-      static const bool prof5 = getenv("MSDR_PROF") != nullptr;
-      long long *d_prof5 = nullptr;
-      if (prof5) {
-        CK(cudaMalloc(&d_prof5, (size_t)sms * 64 * sizeof(long long)));
-        CK(cudaMemsetAsync(d_prof5, 0, (size_t)sms * 64 * sizeof(long long), chain->stream));
-        p.prof = d_prof5;
-      }
-      if (long_window) {
-        CK(launch_chain_v5l(p, chain->stream, chain->variant, sms, &chain->last_info));
-        chain->last_kernel = "msdr::v5l::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; one CTA per 128-channel row block, half-tile hand-offs for the long window)";
-      } else {
-        CK(launch_chain_v5(p, chain->stream, chain->variant, sms, &chain->last_info));
-        chain->last_kernel = "msdr::v5::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; one CTA per 128-channel row block)";
-      }
-      if (p.fe) chain->last_kernel += "; front end fused into the converters";
-      {
-        int stl = syncam_lane_finish(chain, ch0, d_out, stride, p.L);
-        if (stl != MSDR_OK) return stl;
-      }
-      if (chain->timed) {
-        CK(cudaEventRecord(chain->ev1, chain->stream));
-        chain->usage_pending = true;
-        chain->usage_blocks = n_blocks;
-      }
-      chain->launches++;
-      if (d_prof5) {
-        const uint32_t g = (uint32_t)chain->last_info.grid;
-        std::vector<long long> h((size_t)g * 64);
-        CK(cudaMemcpyAsync(h.data(), d_prof5, h.size() * sizeof(long long), cudaMemcpyDeviceToHost, chain->stream));
-        CK(cudaStreamSynchronize(chain->stream));
-        cudaFree(d_prof5);
-        static const char *role[7] = {"convert", "mma", "epilogue", "biquad1", "biquad2", "load", "store"};
-        fprintf(stderr, "[msdr prof v5] grid %u, %u row blocks, mean cycles per CTA (counter 0..3):\n", g, pl.n_rb);
-        for (int r = 0; r < 7; ++r) {
-          double m[4] = {0, 0, 0, 0};
-          for (uint32_t b = 0; b < g; ++b)
-            for (int i = 0; i < 4; ++i) m[i] += (double)h[(size_t)b * 64 + r * 4 + i] / g;
-          fprintf(stderr, "  %-9s %10.0f %10.0f %10.0f %10.0f\n", role[r], m[0], m[1], m[2], m[3]);
-        }
-      }
-      return MSDR_OK;
-    }
-    if (d_adc) {
-      const int stc = compose();
-      if (stc != MSDR_OK) return stc;
-    }
-    st = build_tc_plan(chain, ch0, nch, (uint32_t)sms, want_dual, &plp);
-    if (st != MSDR_OK) return st;
-    const msdr_chain::TcPlan &pl = *plp;
-    // Few channels: the time-folded kernel (msdr_chain_v6.cu), one CTA per 32 same-table channels, nothing leaves the SM.  One group
-    // block per SM: a second round would double the launch, and beyond that the two chain sets per SM of msdr_chain_v4.cu (then the
-    // row-block kernel) are faster.  variant bit 16 forces it for any channel count (parity tests), bit 14 forbids it.
-    const bool use_v6 = pl.usable && pl.slots_v6 && !(chain->variant & (16384 | 128 | 256 | 512 | 2048)) &&
-                        ((chain->variant & 65536) || pl.n_gb <= (uint32_t)std::max(1, sms - (int)chain->spare_sms));
-    if (use_v6) {
-      p.NG = NG;
-      p.n_items = pl.n_gb;
-      p.tc_rowmap = pl.d_rowmap32; p.tc_rb = pl.d_rb32; p.tc_bmat = pl.d_bmat;
-      p.tc_K = pl.K; p.tc_ring = pl.slots_v6;
-      if (chain->timed) {
-        int stu = usage_resolve(chain);
-        if (stu != MSDR_OK) return stu;
-        CK(cudaEventRecord(chain->ev0, chain->stream));
-      }
-      {
-        int stl = syncam_lane_prepare(chain, ch0, nch, d_in, stride, p.L);
-        if (stl != MSDR_OK) return stl;
-      }
-      static const bool prof6 = getenv("MSDR_PROF") != nullptr;
-      long long *d_prof6 = nullptr;
-      if (prof6) {
-        CK(cudaMalloc(&d_prof6, (size_t)sms * 64 * sizeof(long long)));
-        CK(cudaMemsetAsync(d_prof6, 0, (size_t)sms * 64 * sizeof(long long), chain->stream));
-        p.prof = d_prof6;
-      }
-      const int sms_use = std::max(1, sms - (int)chain->spare_sms);
-      CK(launch_chain_v6(p, chain->stream, chain->variant, sms_use, &chain->last_info));
-      chain->last_kernel = "msdr::v6::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; one CTA per 32-channel group block, tile rows folded over time)";
-      {
-        int stl = syncam_lane_finish(chain, ch0, d_out, stride, p.L);
-        if (stl != MSDR_OK) return stl;
-      }
-      if (chain->timed) {
-        CK(cudaEventRecord(chain->ev1, chain->stream));
-        chain->usage_pending = true;
-        chain->usage_blocks = n_blocks;
-      }
-      chain->launches++;
-      if (d_prof6) {
-        const uint32_t g = (uint32_t)chain->last_info.grid;
-        std::vector<long long> h((size_t)g * 64);
-        CK(cudaMemcpyAsync(h.data(), d_prof6, h.size() * sizeof(long long), cudaMemcpyDeviceToHost, chain->stream));
-        CK(cudaStreamSynchronize(chain->stream));
-        cudaFree(d_prof6);
-        static const char *role[9] = {"convert", "mma", "epilogue", "chainA", "chainB", "load", "store", "ff1", "ff2"};
-        fprintf(stderr, "[msdr prof v6] grid %u, %u group blocks, mean cycles per CTA (counter 0..3):\n", g, pl.n_gb);
-        for (int r = 0; r < 9; ++r) {
-          double m[4] = {0, 0, 0, 0}, mx[4] = {0, 0, 0, 0};
-          for (uint32_t b = 0; b < g; ++b)
-            for (int i = 0; i < 4; ++i) { m[i] += (double)h[(size_t)b * 64 + r * 4 + i] / g; mx[i] = std::max(mx[i], (double)h[(size_t)b * 64 + r * 4 + i]); }
-          fprintf(stderr, "  %-9s %10.0f %10.0f %10.0f %10.0f   max %10.0f %10.0f %10.0f %10.0f\n", role[r], m[0], m[1], m[2], m[3], mx[0], mx[1], mx[2], mx[3]);
-        }
-        {
-          double c = 0, n = 0, cm = 0, nm = 0;
-          for (uint32_t b = 0; b < g; ++b) { c += (double)h[(size_t)b * 64 + 40] / g; n += (double)h[(size_t)b * 64 + 41] / g; cm = std::max(cm, (double)h[(size_t)b * 64 + 40]); nm = std::max(nm, (double)h[(size_t)b * 64 + 41]); }
-          fprintf(stderr, "  kernel entry -> chain B done: %.0f cycles, %.0f ns (mean); max %.0f cycles, %.0f ns\n", c, n, cm, nm);
-        }
-        if (getenv("MSDR_PROF_CTAS")) // per-CTA totals of chain A (wait, work) and the epilogue
-          for (uint32_t b = 0; b < g; ++b)
-            fprintf(stderr, "  cta %3u sm %3lld start %8lld ns total %9lld cyc  chainA %9lld %9lld %9lld  ff1 %9lld %9lld yfull %9lld  epilogue %9lld %9lld %9lld %9lld\n", b,
-                    h[(size_t)b * 64 + 42], h[(size_t)b * 64 + 43] - h[43], h[(size_t)b * 64 + 40], h[(size_t)b * 64 + 12], h[(size_t)b * 64 + 13], h[(size_t)b * 64 + 14],
-                    h[(size_t)b * 64 + 28], h[(size_t)b * 64 + 29], h[(size_t)b * 64 + 31], h[(size_t)b * 64 + 8], h[(size_t)b * 64 + 9], h[(size_t)b * 64 + 10], h[(size_t)b * 64 + 11]);
-      }
-      return MSDR_OK;
-    }
-    const bool dual = pl.dual; // false when the second set of chain slots does not fit next to this window (256 taps)
-    use_tc = pl.usable;
-    if (use_tc) {
-      p.NG = NG;
-      p.NT = (p.L + chain_v4_span_samples() - 1) / chain_v4_span_samples();
-      p.W = pl.W; // chains per wave
-      p.n_items = pl.n_rb * p.NT;
-      p.tc_rowmap = pl.d_rowmap; p.tc_rb = pl.d_rb; p.tc_grp = pl.d_grp; p.tc_wave_rb0 = pl.d_wave_rb0; p.tc_bmat = pl.d_bmat;
-      // kernel shape: feed-forward helper warps where they fit (shape 2), else post warps (0), else the plain classic shape (1);
-      // variant bits 11 / 8 / 7 ask for the post-warp, the classic and the helper-warp shape (study knobs, DESIGN.md 6)
-      uint32_t shape = pl.rings[2] ? 2u : pl.rings[0] ? 0u : 1u;
-      if ((chain->variant & 2048) && pl.rings[0]) shape = 0u;
-      if ((chain->variant & 256) && pl.rings[1]) shape = 1u;
-      if ((chain->variant & 128) && pl.rings[2]) shape = 2u;
-      if (dual) shape = 3u;
-      p.tc_K = pl.K; p.tc_ring = pl.rings[shape]; p.tc_ff = shape;
-      p.NU = p.L / chain_v4_unit_samples();
-      const size_t n_cnt = (size_t)NG * p.NU;
-      if (n_cnt > chain->tile_cnt_len) {
-        CK(cudaStreamSynchronize(chain->stream));
-        cudaFree(chain->d_tile_cnt);
-        chain->d_tile_cnt = nullptr; chain->tile_cnt_len = 0;
-        CK(cudaMalloc(&chain->d_tile_cnt, (n_cnt + 1024) * sizeof(int)));
-        chain->tile_cnt_len = n_cnt + 1024;
-      }
-      CK(cudaMemsetAsync(chain->d_tile_cnt, 0, n_cnt * sizeof(int), chain->stream));
-      p.tile_cnt = chain->d_tile_cnt;
-    }
+
+  ChainParams p{};
+  p.in = d_in; p.out = d_out; p.stride = stride;
+  p.C = nch; p.ch0 = ch0; p.Cpad = chain->Cpad; p.L = (uint32_t)L64; p.H = chain->H;
+  p.hist = chain->d_hist; p.bq = chain->d_bq; p.mode = chain->d_mode; p.setid = chain->d_set;
+  p.am_q31 = (chain->flags & MSDR_FLAG_AM_Q31) ? 1u : 0u;
+  p.spare_sms = chain->spare_sms;
+  p.NG = NG; p.tc_K = pl.K; p.tc_bmat = pl.d_bmat;
+  if (d_adc) { // fused: the converters read codes and condition them (msdr_chain_v5_common.cuh: FeRow)
+    p.in = reinterpret_cast<const int16_t *>(d_adc);
+    p.fe = chain->d_fe; p.agc_max = chain->fe_agc_max; p.agc_on = chain->fe_agc_on ? 1u : 0u;
   }
+  switch (ch.kernel) {
+  case kV5:
+  case kV5l:
+    p.n_items = pl.n_rb; p.tc_rowmap = pl.d_rowmap; p.tc_rb = pl.d_rb;
+    p.tc_ring = ch.kernel == kV5l ? pl.ring_v5l : pl.ring_v5;
+    break;
+  case kV6:
+    p.n_items = pl.n_gb; p.tc_rowmap = pl.d_rowmap32; p.tc_rb = pl.d_rb32;
+    p.tc_ring = pl.slots_v6;
+    break;
+  case kV4: {
+    p.NT = (p.L + chain_v4_span_samples() - 1) / chain_v4_span_samples();
+    p.W = pl.W; // chains per wave
+    p.n_items = pl.n_rb * p.NT;
+    p.tc_rowmap = pl.d_rowmap; p.tc_rb = pl.d_rb; p.tc_wave_rb0 = pl.d_wave_rb0;
+    p.tc_ring = pl.rings[ch.shape]; p.tc_ff = ch.shape;
+    p.NU = p.L / chain_v4_unit_samples();
+    const size_t n_cnt = (size_t)NG * p.NU;
+    if (n_cnt > chain->tile_cnt_len) {
+      CK(cudaStreamSynchronize(chain->stream));
+      cudaFree(chain->d_tile_cnt);
+      chain->d_tile_cnt = nullptr; chain->tile_cnt_len = 0;
+      CK(cudaMalloc(&chain->d_tile_cnt, (n_cnt + 1024) * sizeof(int)));
+      chain->tile_cnt_len = n_cnt + 1024;
+    }
+    CK(cudaMemsetAsync(chain->d_ctrl, 0, 2 * sizeof(int), chain->stream));
+    CK(cudaMemsetAsync(chain->d_tile_cnt, 0, n_cnt * sizeof(int), chain->stream));
+    p.ctrl = chain->d_ctrl; p.tile_cnt = chain->d_tile_cnt;
+    break;
+  }
+  }
+
   if (chain->timed) {
-    int stu = usage_resolve(chain); // the event pair is reused: fold the previous update in first
-    if (stu != MSDR_OK) return stu;
+    if ((st = usage_resolve(chain)) != MSDR_OK) return st; // the event pair is reused: fold the previous update in first
     CK(cudaEventRecord(chain->ev0, chain->stream));
   }
-  {
-    int stl = syncam_lane_prepare(chain, ch0, nch, d_in, stride, p.L);
-    if (stl != MSDR_OK) return stl;
-  }
-  static const bool prof_on = getenv("MSDR_PROF") != nullptr; // developer aid: per-role cycle totals of the v4 kernel on stderr
+  if ((st = syncam_lane_prepare(chain, ch0, nch, d_in, stride, p.L)) != MSDR_OK) return st;
+  static const bool prof_on = getenv("MSDR_PROF") != nullptr; // developer aid: per-role cycle counters on stderr
   long long *d_prof = nullptr;
-  if (use_tc && prof_on) {
-    CK(cudaMalloc(&d_prof, (size_t)p.W * 64 * sizeof(long long)));
-    CK(cudaMemsetAsync(d_prof, 0, (size_t)p.W * 64 * sizeof(long long), chain->stream));
+  if (prof_on) {
+    const size_t bytes = (size_t)(ch.kernel == kV4 ? p.W : (uint32_t)sms) * 64 * sizeof(long long);
+    CK(cudaMalloc(&d_prof, bytes));
+    CK(cudaMemsetAsync(d_prof, 0, bytes, chain->stream));
     p.prof = d_prof;
   }
-  if (use_tc) {
-    CK(launch_chain_v4(p, chain->stream, chain->variant, &chain->last_info));
-    static const char *shape_name[4] = {"post-warp shape", "classic shape", "feed-forward helper-warp shape", "two chain sets per SM"};
-    chain->last_kernel = std::string("msdr::v4::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; ") + shape_name[p.tc_ff & 3u] + ")";
-  } else {
-    CK(launch_chain(p, chain->stream, chain->variant, &chain->last_info));
-    chain->last_kernel = "msdr::v3::chain_kernel (fused chain, CUDA-core FIR)";
+  switch (ch.kernel) {
+  case kV6: CK(launch_chain_v6(p, chain->stream, chain->variant, std::max(1, sms - (int)chain->spare_sms), &chain->last_info)); break;
+  case kV4: CK(launch_chain_v4(p, chain->stream, chain->variant, &chain->last_info)); break;
+  case kV5: CK(launch_chain_v5(p, chain->stream, chain->variant, sms, &chain->last_info)); break;
+  case kV5l: CK(launch_chain_v5l(p, chain->stream, chain->variant, sms, &chain->last_info)); break;
   }
-  {
-    int stl = syncam_lane_finish(chain, ch0, d_out, stride, p.L);
-    if (stl != MSDR_OK) return stl;
-  }
+  chain->last_kernel = std::string("msdr::") + kNames[ch.kernel].ns + "::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; " +
+                       (ch.kernel == kV4 ? kV4ShapeNames[ch.shape] : kNames[ch.kernel].form) + ")";
+  if (p.fe) chain->last_kernel += "; front end fused into the converters";
+  if ((st = syncam_lane_finish(chain, ch0, d_out, stride, p.L)) != MSDR_OK) return st;
   if (chain->timed) {
     CK(cudaEventRecord(chain->ev1, chain->stream));
     chain->usage_pending = true;
     chain->usage_blocks = n_blocks;
   }
   chain->launches++;
-  if (d_prof) {
-    std::vector<long long> h((size_t)p.W * 64);
-    CK(cudaMemcpyAsync(h.data(), d_prof, h.size() * sizeof(long long), cudaMemcpyDeviceToHost, chain->stream));
-    CK(cudaStreamSynchronize(chain->stream));
-    cudaFree(d_prof);
-    static const char *role[8] = {"convert", "mma", "epilogue", "chainA", "chainB", "load", "store", "ff2/post"};
-    fprintf(stderr, "[msdr prof] grid %u, mean cycles per CTA (counter 0..3):\n", p.W);
-    for (int r = 0; r < 8; ++r) {
-      double m[4] = {0, 0, 0, 0};
-      for (uint32_t b = 0; b < p.W; ++b)
-        for (int i = 0; i < 4; ++i) m[i] += (double)h[(size_t)b * 64 + r * 4 + i] / p.W;
-      fprintf(stderr, "  %-9s %10.0f %10.0f %10.0f %10.0f\n", role[r], m[0], m[1], m[2], m[3]);
-    }
-  }
+  if (d_prof) return prof_dump(chain, ch.kernel, d_prof, ch.kernel == kV4 ? p.W : (uint32_t)chain->last_info.grid, p.n_items);
   return MSDR_OK;
 }
 
@@ -1705,8 +1583,6 @@ int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre
   for (uint32_t c = ch0; c < ch0 + n; ++c)
     if (chain->h_set[c] != kNoTable) { chain->sets[chain->h_set[c]].users--; chain->h_set[c] = kNoTable; chain->n_uninit++; }
   uint8_t map[MSDR_MAX_FIR_SETS];
-  chain->snap_ex.resize((size_t)MSDR_MAX_FIR_SETS * chain->set_stride_words);
-  chain->snap_kp4.resize(MSDR_MAX_FIR_SETS);
   chain->snap_taps.resize((size_t)MSDR_MAX_FIR_SETS * 2 * MSDR_MAX_TAPS);
   for (uint32_t k = 0; k < h.n_tables; ++k) {
     if (!used[k]) continue;
@@ -1722,16 +1598,9 @@ int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre
       fs.T = t.T;
       fs.cI.assign(t.cI, t.cI + t.T);
       fs.cQ.assign(t.cQ, t.cQ + t.T);
-      std::vector<int32_t> ex;
-      expand_set(fs, ex, chain->set_stride_words);
-      int32_t *sx = chain->snap_ex.data() + slot * chain->set_stride_words;
-      std::copy(ex.begin(), ex.end(), sx);
-      chain->snap_kp4[slot] = kp_of_taps(t.T) / 4;
       int16_t *tp = chain->snap_taps.data() + slot * 2 * MSDR_MAX_TAPS;
       std::copy(t.cI, t.cI + t.T, tp);
       std::copy(t.cQ, t.cQ + t.T, tp + MSDR_MAX_TAPS);
-      CK(cudaMemcpyAsync(chain->d_sets + slot * chain->set_stride_words, sx, ex.size() * 4, cudaMemcpyHostToDevice, chain->stream));
-      CK(cudaMemcpyAsync(chain->d_set_kp4 + slot, &chain->snap_kp4[slot], 4, cudaMemcpyHostToDevice, chain->stream));
       CK(cudaMemcpyAsync(chain->d_set_taps + slot * 2 * MSDR_MAX_TAPS, tp, 2 * MSDR_MAX_TAPS * 2, cudaMemcpyHostToDevice, chain->stream));
     }
     chain->sets[slot].users += used[k]; // counted at once: an identical later entry finds this slot

@@ -1,129 +1,10 @@
 // msdr_chain_common.cuh — device code shared by the fused receive-chain kernels:
-// polyphase fs/4-mix + FIR pair + demod for one channel row (FIR warps), biquad cascade helpers (biquad warps).
+// demodulation kind of a mode, biquad cascade helpers (biquad warps).
 #pragma once
 #include "msdr_device.cuh"
 #include "msdr_internal.h"
 
 namespace msdr {
-
-__host__ __device__ inline uint32_t align_up(uint32_t v, uint32_t a) { return (v + a - 1u) / a * a; }
-
-// words per 4-tap chunk of an expanded coefficient set: A[4], B[4] as int32, C[4], D[4] as double
-constexpr int kSetChunkWords = 24;
-
-// unpack 4 words (even sample | odd sample << 16): even samples as int32 for the IMAD pipe, odd ones as double for DFMA
-__device__ __forceinline__ void unpack4(const uint4 v, uint32_t *e, double *od)
-{
-  e[0] = (uint32_t)(int)(short)(v.x & 0xFFFFu); od[0] = (double)((int)v.x >> 16);
-  e[1] = (uint32_t)(int)(short)(v.y & 0xFFFFu); od[1] = (double)((int)v.y >> 16);
-  e[2] = (uint32_t)(int)(short)(v.z & 0xFFFFu); od[2] = (double)((int)v.z >> 16);
-  e[3] = (uint32_t)(int)(short)(v.w & 0xFFFFu); od[3] = (double)((int)v.w >> 16);
-}
-
-// 4 taps x R output pairs x 4 sub-filters = 16R multiply-accumulates on a rotating register window, split over TWO pipes:
-// the I branch (sub-filters A, B on the even samples) as 32-bit wrapping IMAD, the Q branch (C, D on the odd samples) as
-// DFMA.  Products are < 2^30 and at most 128 of them are summed, so the double accumulators hold the exact integer sum
-// (|sum| < 2^37 << 2^53) and its low 32 bits are the reference's wrapped accumulator.  IMAD and DFMA co-issue at 1.65x the
-// IMAD-only rate on B200 (tools/microbench/pipes.cu).
-// The window holds W = R + 4 consecutive words; logical position x lives in physical register (x + 4*ROT) % W, so
-// sliding the window by one chunk (4 words) is a change of ROT, not a register move.
-template <int R, int ROT>
-__device__ __forceinline__ void fir_chunk(uint32_t (&e)[R + 4], double (&od)[R + 4], uint32_t (&aA)[R], uint32_t (&aB)[R], double (&aC)[R],
-                                          double (&aD)[R], const int4 *__restrict__ cf)
-{
-  constexpr int W = R + 4;
-  const int4 cA = cf[0], cB = cf[1];
-  const double2 cC0 = reinterpret_cast<const double2 *>(cf)[2], cC1 = reinterpret_cast<const double2 *>(cf)[3];
-  const double2 cD0 = reinterpret_cast<const double2 *>(cf)[4], cD1 = reinterpret_cast<const double2 *>(cf)[5];
-  const uint32_t ca[4] = {(uint32_t)cA.x, (uint32_t)cA.y, (uint32_t)cA.z, (uint32_t)cA.w};
-  const uint32_t cb[4] = {(uint32_t)cB.x, (uint32_t)cB.y, (uint32_t)cB.z, (uint32_t)cB.w};
-  const double cc[4] = {cC0.x, cC0.y, cC1.x, cC1.y};
-  const double cd[4] = {cD0.x, cD0.y, cD1.x, cD1.y};
-#pragma unroll
-  for (int t = 0; t < 4; ++t) {
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const uint32_t ev = e[(1 + r + t + 4 * ROT) % W];
-      const double ov = od[(1 + r + t + 4 * ROT) % W];
-      aA[r] = ca[t] * ev + aA[r];
-      aC[r] = fma(cc[t], ov, aC[r]);
-      aB[r] = cb[t] * ev + aB[r];
-      aD[r] = fma(cd[t], ov, aD[r]);
-    }
-  }
-}
-
-// One channel row of one tile: FIR pair + demod for lane's 2R output samples.
-//   rowW  : sign-folded raw samples of the row as words (even sample | odd sample << 16); word Hw is tile sample 0
-//   cf    : expanded taps of the row's coefficient set: per 4-tap chunk c, 6 x 16 bytes = A, B (int32), C, D (double)
-//           A: I taps for odd outputs, B: I taps for even outputs, C: Q taps for odd outputs, D: Q taps for even
-//   With u = folded samples, ue[j] = u[2j], uo[j] = u[2j+1], output pair i = (n = 2i, 2i+1), KP = 4*kp4:
-//     accX[i] = sum_{d < KP} cX[d] * {ue|uo}[i - KP + 1 + d]      (exact mod 2^32, any order)
-template <int R>
-__device__ __forceinline__ void fir_demod_row(const uint32_t *__restrict__ rowW, const int4 *__restrict__ cf, const int kp4, const int Hw,
-                                              const int lane, const int len, const int kind, uint32_t *__restrict__ drow)
-{
-  static_assert(R == 8, "the rotation schedule below assumes a 12-word window (3 chunks per turn)");
-  constexpr int W = R + 4;
-  constexpr int CS = kSetChunkWords / 4; // int4 per chunk
-  const int i0 = lane * R;
-  if (2 * i0 >= len) return;
-  const uint4 *wp = reinterpret_cast<const uint4 *>(rowW + Hw + i0 - 4 * kp4);
-  uint32_t e[W];
-  double od[W];
-#pragma unroll
-  for (int g = 0; g < W / 4; ++g) unpack4(wp[g], e + 4 * g, od + 4 * g);
-  wp += W / 4;
-  uint32_t aA[R], aB[R];
-  double aC[R], aD[R];
-#pragma unroll
-  for (int r = 0; r < R; ++r) { aA[r] = aB[r] = 0u; aC[r] = aD[r] = 0.0; }
-
-  // chunk c consumes window rotation c % 3 and then refills the 4 slots it vacated with words for chunk c + 1;
-  // the refill after the very last chunk reads 4 words past the lane's window (still inside the row buffer) and is unused.
-  int c = 0;
-#pragma unroll 1
-  for (; c + 3 <= kp4; c += 3) {
-    fir_chunk<R, 0>(e, od, aA, aB, aC, aD, cf + CS * c);
-    unpack4(wp[0], e + 0, od + 0);
-    fir_chunk<R, 1>(e, od, aA, aB, aC, aD, cf + CS * (c + 1));
-    unpack4(wp[1], e + 4, od + 4);
-    fir_chunk<R, 2>(e, od, aA, aB, aC, aD, cf + CS * (c + 2));
-    unpack4(wp[2], e + 8, od + 8);
-    wp += 3;
-  }
-  if (c < kp4) {
-    fir_chunk<R, 0>(e, od, aA, aB, aC, aD, cf + CS * c);
-    if (c + 1 < kp4) {
-      unpack4(wp[0], e + 0, od + 0);
-      fir_chunk<R, 1>(e, od, aA, aB, aC, aD, cf + CS * (c + 1));
-    }
-  }
-
-  // arm_fir_fast_q15.c:234-238: acc >> 15, SSAT16; then the demodulation switch (Minimal-SDR.ino:589-628)
-  uint32_t outw[R];
-  if (kind < 2) { // SSB: out = (int16)(I -/+ Q), two samples per word
-    const int sgn = kind ? 1 : -1;
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const int Io = ssat16((int)aA[r] >> 15), Ie = ssat16((int)aB[r] >> 15);
-      // exact integer in a double -> its value mod 2^32: low word of (x + 1.5 * 2^52)
-      const int Qo = ssat16(__double2loint(aC[r] + kBqM) >> 15), Qe = ssat16(__double2loint(aD[r] + kBqM) >> 15);
-      outw[r] = ((uint32_t)(Ie + sgn * Qe) & 0xFFFFu) | ((uint32_t)(Io + sgn * Qo) << 16);
-    }
-  } else {
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const int Io = ssat16((int)aA[r] >> 15), Ie = ssat16((int)aB[r] >> 15);
-      const int Qo = ssat16(__double2loint(aC[r] + kBqM) >> 15), Qe = ssat16(__double2loint(aD[r] + kBqM) >> 15);
-      const int se = demod_envelope(kind, Ie, Qe), so = demod_envelope(kind, Io, Qo);
-      outw[r] = ((uint32_t)se & 0xFFFFu) | ((uint32_t)so << 16);
-    }
-  }
-  uint4 *dp = reinterpret_cast<uint4 *>(drow + i0);
-#pragma unroll
-  for (int g = 0; g < R / 4; ++g) dp[g] = make_uint4(outw[4 * g], outw[4 * g + 1], outw[4 * g + 2], outw[4 * g + 3]);
-}
 
 __device__ __forceinline__ int demod_kind_of(int mode, uint32_t am_q31)
 {
@@ -177,19 +58,6 @@ __device__ __forceinline__ uint32_t bq_word(BqStageHS (&st)[NS], uint32_t w)
   for (int k = 0; k < NS; ++k) xo = bq_step(st[k], xo);
   return __byte_perm((uint32_t)xe, (uint32_t)xo, 0x7632);
 }
-// same on the FP64 pipe (D-form values)
-template <int NS>
-__device__ __forceinline__ uint32_t bq_word(BqStageD (&st)[NS], uint32_t w)
-{
-  double xe = bq_d_from_int((int)(short)(w & 0xFFFFu)), xo = bq_d_from_int((int)w >> 16);
-  int ye = 0, yo = 0;
-#pragma unroll
-  for (int k = 0; k < NS; ++k) xe = bq_step(st[k], xe, ye);
-#pragma unroll
-  for (int k = 0; k < NS; ++k) xo = bq_step(st[k], xo, yo);
-  return __byte_perm((uint32_t)ye, (uint32_t)yo, 0x5410);
-}
-
 // hybrid stage (feed-forward on the FP64 pipe): inputs sign-extended with one PRMT each, outputs arrive as y << 16
 template <int NS>
 __device__ __forceinline__ uint32_t bq_word(BqStageH (&st)[NS], uint32_t w)
@@ -323,26 +191,6 @@ __device__ __forceinline__ void bq_store_stage(const BqStage &s, uint32_t flag, 
   b[6 * (size_t)Cpad] = (int32_t)bq_pack_hist(s.y1, s.y2);
   b[7 * (size_t)Cpad] = (int32_t)((uint32_t)s.res | flag); // filter_biquad.cpp:75-78
 }
-__device__ __forceinline__ void bq_load_stage(BqStageD &s, uint32_t &flag, const int32_t *__restrict__ bq, uint32_t Cpad, int obj, int stage, uint32_t ch)
-{
-  const int32_t *b = bq + (size_t)((obj * 4 + stage) * 8) * Cpad + ch;
-  bq_set_coefs(s, __ldcg(b + 0 * (size_t)Cpad), __ldcg(b + 1 * (size_t)Cpad), __ldcg(b + 2 * (size_t)Cpad), __ldcg(b + 3 * (size_t)Cpad),
-               __ldcg(b + 4 * (size_t)Cpad));
-  const uint32_t w5 = (uint32_t)__ldcg(b + 5 * (size_t)Cpad), w6 = (uint32_t)__ldcg(b + 6 * (size_t)Cpad);
-  s.x1 = bq_d_from_int((int)w5 >> 16); s.x2 = bq_d_from_int((int)(short)(w5 & 0xFFFFu));
-  s.y1 = bq_d_from_int((int)w6 >> 16); s.y2 = bq_d_from_int((int)(short)(w6 & 0xFFFFu));
-  const uint32_t w7 = (uint32_t)__ldcg(b + 7 * (size_t)Cpad);
-  s.res = (int)(w7 & 0x3FFFu);
-  flag = w7 & 0x80000000u;
-}
-__device__ __forceinline__ void bq_store_stage(const BqStageD &s, uint32_t flag, int32_t *__restrict__ bq, uint32_t Cpad, int obj, int stage, uint32_t ch)
-{
-  int32_t *b = bq + (size_t)((obj * 4 + stage) * 8) * Cpad + ch;
-  b[5 * (size_t)Cpad] = (int32_t)(((uint32_t)bq_int_from_d(s.x1) << 16) | ((uint32_t)bq_int_from_d(s.x2) & 0xFFFFu));
-  b[6 * (size_t)Cpad] = (int32_t)(((uint32_t)bq_int_from_d(s.y1) << 16) | ((uint32_t)bq_int_from_d(s.y2) & 0xFFFFu));
-  b[7 * (size_t)Cpad] = (int32_t)((uint32_t)s.res | flag);
-}
-
 __device__ __forceinline__ void bq_load_stage(BqStageH &s, uint32_t &flag, const int32_t *__restrict__ bq, uint32_t Cpad, int obj, int stage, uint32_t ch)
 {
   const int32_t *b = bq + (size_t)((obj * 4 + stage) * 8) * Cpad + ch;

@@ -6,7 +6,7 @@
 // Reference semantics: Minimal-SDR.ino:546-558 (mix), arm_fir_fast_q15.c:60-329 (FIR), Minimal-SDR.ino:589-628 (demod),
 // filter_biquad.cpp:33-82 (biquad).
 //
-// Same decoupling as msdr_chain_v3.cu — FIR work is produced by any SM, biquad chains are pinned to an SM for the whole
+// FIR work and biquad chains are decoupled — FIR work is produced by any SM, biquad chains are pinned to an SM for the whole
 // launch and only ever wait for their own input — but the FIR producers are a tensor-core pipeline, which takes the FIR off
 // the integer/FP64 issue slots the serial biquad recurrence needs.  One persistent CTA per SM, 16 warps, roles by warp id
 // (warp id % 4 = SM sub-partition).  Default shape (POST; the others are listed at `Roles` below):
@@ -259,7 +259,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
       const uint32_t tb = span * (SPAN / N), te = min(tb + SPAN / N, n_tiles);
       const uint32_t qbase = q;
       const uint32_t npairs = (te - tb) + KS - 1;
-      const uint4 rbi = __ldg(p.tc_rb + rb); // x: table id, y: first group entry, z: number of group entries
+      const uint4 rbi = __ldg(p.tc_rb + rb); // x: table id (the other words are 0)
       const uint32_t *rmap = p.tc_rowmap + (size_t)rb * M;
 
       if (is_conv) {

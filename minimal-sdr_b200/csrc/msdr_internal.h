@@ -29,26 +29,16 @@ struct ChainParams {
   int32_t *bq;            // [64][Cpad] biquad definition words, SoA
   const uint8_t *mode;    // [C] msdr_mode
   const uint8_t *setid;   // [C] FIR coefficient-set id
-  const int32_t *sets;    // [n_sets][set_stride_words] expanded polyphase taps
-  const uint32_t *set_kp4; // [n_sets] number of 4-tap chunks
-  uint32_t n_sets;
-  uint32_t set_stride_words;
   uint32_t NG;            // channel groups
-  uint32_t NT;            // tiles per channel in this launch
-  uint32_t TPS;           // tiles per segment
-  uint32_t S;             // segments per group
-  uint32_t n_items;       // NG * S
-  int *ctrl;              // [0] work counter, [1 + g] segments completed for group g (hand-off kernel)
-  int *tile_flags;        // [NG][NT] == epoch once the demodulated tile is in `out` (chain kernel v3)
-  uint32_t epoch;         // launch counter, never 0
-  uint32_t W;             // biquad chains per wave = grid (v3)
+  uint32_t NT;            // spans per channel in this launch (v4)
+  uint32_t n_items;       // work items: v4 row blocks x spans, v5 / v5l row blocks, v6 group blocks
+  int *ctrl;              // v4: [0] work counter, [1] spans the loaders have taken (flow control)
+  uint32_t W;             // v4: biquad chains per wave
   uint32_t ablate;        // study only: bit 0 skip the FIR arithmetic, bit 1 skip the biquad arithmetic (results are wrong)
-  uint32_t sets_in_smem;  // 0: the tap tables do not fit next to the tile buffers and are read from global memory
   uint32_t am_q31;
   // tensor-core FIR plan (chain kernel v4, msdr_chain_v4.cu)
   const uint32_t *tc_rowmap;   // [n_rb][128] launch-relative row, 0xFFFFFFFF = padding
-  const uint4 *tc_rb;          // [n_rb] {table id, first group entry, group entries, wave}
-  const uint32_t *tc_grp;      // group entries: group | rows << 24
+  const uint4 *tc_rb;          // [n_rb] .x = table id, the other words 0 (v6: [n_items] .x, .y = the tables of the two half blocks)
   const uint32_t *tc_wave_rb0; // [n_waves + 1] first row block of each wave
   const uint8_t *tc_bmat;      // [n_sets][4 * 64 * K] Toeplitz operands
   uint32_t tc_K, tc_ring, tc_sub, tc_ff; // tc_ff: kernel shape 0/1/2 (msdr_chain_v4.cu: chain_v4_config)
@@ -68,10 +58,7 @@ struct ChainLaunchInfo {
   int tile;
 };
 
-// Fused mix + FIR pair + demod + biquad cascade (K1). variant: 0 = default.
-cudaError_t launch_chain(const ChainParams &p, cudaStream_t stream, int variant, ChainLaunchInfo *info);
-cudaError_t launch_chain_v3(const ChainParams &p, cudaStream_t stream, int variant, ChainLaunchInfo *info);
-uint32_t chain_tile_samples();
+// Fused mix + FIR pair + demod + biquad cascade (K1, msdr_chain_v4.cu). variant: 0 = default.
 cudaError_t launch_chain_v4(const ChainParams &p, cudaStream_t stream, int variant, ChainLaunchInfo *info);
 uint32_t chain_v4_span_samples();
 uint32_t chain_v4_unit_samples();
@@ -84,8 +71,8 @@ cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, ui
 // p.fe != NULL selects the ADC-code instantiation (default biquad form only)
 cudaError_t launch_chain_v5(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
 uint32_t chain_v5_config(uint32_t K, int smem_max);
-// pinned 32-channel group blocks with the tile rows folded over time (msdr_chain_v6.cu): p.tc_rowmap = [n_items][32] rows of one table,
-// p.tc_rb[i].x = table id, p.tc_ring = sub-tile slots from chain_v6_config (0 = the window does not fit)
+// pinned 32-channel group blocks with the tile rows folded over time (msdr_chain_v6.cu): p.tc_rowmap = [n_items][32] rows,
+// p.tc_rb[i].x / .y = the tables of its two half blocks, p.tc_ring = sub-tile slots from chain_v6_config (0 = the window does not fit)
 cudaError_t launch_chain_v6(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
 uint32_t chain_v6_config(uint32_t K, int smem_max);
 uint32_t chain_v6_group_rows();

@@ -1,6 +1,6 @@
 // msdr_stage_kernels.cu — one kernel per reference primitive, on device buffers.
 // These back the stage-level C-ABI operators (msdr_op_*) used by the AudioStream façade and the per-stage
-// parity tests; the production path is the fused kernel in msdr_chain_kernel.cu.
+// parity tests; the production path is the fused chain kernels in msdr_chain_v4.cu, v5.cu, v5l.cu and v6.cu.
 #include "msdr_device.cuh"
 #include "msdr_internal.h"
 #include <algorithm>

@@ -328,8 +328,8 @@ def test_update_range_device(msdr, orc, K):
 
 @pytest.mark.parametrize("variant,name", [(0, "default (time-folded kernel, msdr_chain_v6.cu)"), (16384, "chain kernel (msdr_chain_v4.cu), feed-forward helper warps"),
                                             (2048, "tensor-core FIR + post warps"),
-                                            (256, "tensor-core FIR, inline epilogue"), (128, "helper warps, forced"), (64, "CUDA-core FIR (v3)"),
-                                            (65, "v3, FP64 biquad"), (4096, "row-block kernel (msdr_chain_v5.cu), forced"),
+                                            (256, "tensor-core FIR, inline epilogue"), (128, "helper warps, forced"),
+                                            (2, "time-folded kernel, DFMA feed-forward"), (4096, "row-block kernel (msdr_chain_v5.cu), forced"),
                                             (4097, "row-block kernel, IMAD.WIDE stages"), (4098, "row-block kernel, DFMA feed-forward"),
                                             (4100, "row-block kernel, chained DFMA feed-forward"), (4104, "row-block kernel, all five products one DFMA chain"),
                                             (4108, "row-block kernel, split 16 x 16-bit products")])
@@ -354,7 +354,7 @@ def test_every_kernel_shape_is_bit_exact(msdr, orc, K, variant, name):
     assert o.fir_init(7, 2, cI, cQ) == 0
     yg, yo = run_pair(g, o, x, splits=[3, 1, 17, 2, 18])
     assert_same(yg, yo, name)
-    want = "v6::" if variant == 0 else "v5::" if variant & 4096 else "v3::" if variant & 64 else "v4::"
+    want = "v6::" if variant in (0, 2) else "v5::" if variant & 4096 else "v4::"
     assert want in g.last_kernel(), (variant, g.last_kernel())
 
 

@@ -71,7 +71,7 @@ def test_two_waves_long_update_all_shapes_agree(msdr, orc, K):
     outs = {}
     # 0 = the chain kernel with two chain sets per SM (188 groups > 148 SMs), 65536 = the time-folded kernel forced (188 group blocks on
     # 148 SMs: 40 CTAs walk two blocks), 512 = one set, helper warps
-    for variant in (0, 65536, 512, 2048, 256, 128, 64):
+    for variant in (0, 65536, 512, 2048, 256, 128):
         g, modes = _setup(msdr, K, C)
         g.set_option("variant", variant)
         y = torch.empty_like(x)
@@ -80,7 +80,7 @@ def test_two_waves_long_update_all_shapes_agree(msdr, orc, K):
         torch.cuda.synchronize()
         outs[variant] = y
         g.close()
-    for variant in (65536, 512, 2048, 256, 128, 64):
+    for variant in (65536, 512, 2048, 256, 128):
         assert torch.equal(outs[0], outs[variant]), f"variant {variant} differs from the default shape"
     pick = [0, 31, 4735, 4736, 4737, 5000, 5999]
     o = orc.chain(len(pick))

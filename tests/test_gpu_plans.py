@@ -53,8 +53,6 @@ def family(kernel):
         return "v5"
     if "v4::" in kernel:
         return "v4 two sets" if "two chain sets per SM" in kernel else "v4 one set"
-    if "v3::" in kernel:
-        return "v3"
     raise AssertionError(f"unknown kernel: {kernel}")
 
 
@@ -168,6 +166,28 @@ def test_selection_threshold_every_channel(msdr, orc, K, sms, case):
     assert_same(yg, yo, f"{case}: {nch} channels, {n_gb} group blocks, {sms} SMs, spare {spare}")
 
 
+def test_forced_time_folded_kernel_after_a_cached_plan(msdr, orc, K, sms):
+    """A variant that asks for the time-folded kernel takes effect on a range whose plan is already cached.  9000 channels run the
+    chain kernel with two chain sets per SM at variant 0, and that plan has no group blocks (more than 8192 channels); after
+    set_option("variant", 65536) the next update of the same range runs the time-folded kernel.  Every channel against the oracle."""
+    nch = 9000
+    rng = np.random.default_rng(nch)
+    modes = msdr.synth.mixed_modes(nch)
+    am = np.array(K["FIR_AM_coeffs_bw2800_fs24000"], np.int16)
+    tables = [(am, am), _table(86, rng, wrap=True)]
+    table_of = np.zeros(nch, np.int64)
+    table_of[[1, 31, 32, 127, 128, 4000, nch - 1]] = 1
+    assert predict(nch, v6_group_blocks(table_of), sms) == "v4 two sets"
+    x = msdr.synth.batch(modes, 128 * 4)
+    _adversarial_rows(x, rng, low=[31, nch - 1], full=[32, 128])
+    g, o = _pair(msdr, orc, K, modes, table_of, tables)
+    g.set_option("variant", 0)
+    y0 = _run(g, o, x[:, :128 * 2], [2], "v4 two sets")
+    g.set_option("variant", 65536)
+    y1 = _run(g, o, x[:, 128 * 2:], [2], "v6")
+    assert_same(np.concatenate([y0[0], y1[0]], axis=1), np.concatenate([y0[1], y1[1]], axis=1), f"{nch} channels, variant 0 then 65536")
+
+
 # ---- 2. MSDR_MAX_FIR_SETS tables on every kernel ----------------------------------------------------------------------------
 
 def _full_layout(msdr, K, sms, layout):
@@ -187,7 +207,7 @@ def _full_layout(msdr, K, sms, layout):
 
 
 FULL_CASES = [("base", 0, "v6"), ("base", 16384, "v4 one set"), ("base", 512, "v4 one set"), ("base", 4096, "v5"),
-              ("base", 4096 | 32768, "v5l"), ("base", 64, "v3"), ("wide", 0, "v4 two sets"), ("wide", 512, "v4 one set"),
+              ("base", 4096 | 32768, "v5l"), ("wide", 0, "v4 two sets"), ("wide", 512, "v4 one set"),
               ("taps256", 0, "v4 one set"), ("taps256", 4096, "v5l")]
 
 

@@ -15,7 +15,7 @@ lib = ol.CheckerLib("ref") if ol.have_ref() else ol.CheckerLib("orc")
 chans = m.workloads.sample_channels(C, want=24)
 idx = torch.tensor(chans, device=dev)
 modes = w.modes(C)
-for variant in (0, 2048, 256, 64):
+for variant in (0, 2048, 256):
     for nb1 in (64, 128, 256, 384, 512, 1024):
         g = m.ReceiveChain(C, max_taps=w.max_taps)
         g.set_option("variant", variant)
