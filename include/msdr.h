@@ -126,6 +126,21 @@ int msdr_chain_update_device(msdr_chain *chain, const int16_t *d_in, int16_t *d_
 int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
                                    size_t stride);
 
+/* Channels channels[0..n) only, in list order: row i of d_in / d_out is channel channels[i].  Same buffer, alignment, stride and
+ * state rules as msdr_chain_update_range_device; results, outputs and state equal those of range updates of the same channels.
+ * `channels` is a host array in any order.  MSDR_ERR_ARGUMENT, before anything is enqueued, for a channel >= the chain's
+ * channel count, a channel listed twice, or channels == NULL with n > 0; n == 0 launches nothing.  int16 input only: the
+ * front-end state (msdr_chain_enable_frontend) is left alone.  Runs on the time-folded kernel while the list's channel
+ * groups fit one per SM, else on the row-block kernel, never on the chain kernel v4; scattered channels gather their state,
+ * so a list can run below a range of the same size (rates: DESIGN.md §6).  The row plan of each distinct list is cached
+ * like that of a range (INTEGRATION.md §3h). */
+int msdr_chain_update_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *d_in, int16_t *d_out,
+                                  uint32_t n_blocks, size_t stride);
+/* The same on host buffers of n rows, through the 3-slot copy / kernel / copy pipeline of msdr_chain_update (the list is cut
+ * into chunks of host_chunk_channels entries like the chain is there). */
+int msdr_chain_update_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *in, int16_t *out, uint32_t n_blocks,
+                           size_t stride);
+
 /* Device time of the last update in milliseconds (CUDA events), the analogue of the reference's
  * micros()-around-demodulation() load figure (Minimal-SDR.ino:533,774; :415-432). Synchronises. */
 int msdr_chain_last_update_ms(msdr_chain *chain, float *ms);

@@ -74,6 +74,8 @@ SYMBOLS = {
     "msdr_chain_update": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
     "msdr_chain_update_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
     "msdr_chain_update_range_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_update_list_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_update_list": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
     "msdr_chain_last_update_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "msdr_chain_launch_count": (C.c_uint64, [C.c_void_p]),
     "msdr_chain_plan_build_count": (C.c_uint64, [C.c_void_p]),

@@ -183,6 +183,27 @@ class ReceiveChain:
         return self._ck(self._L.msdr_chain_update_range_device(self.h, int(ch0), int(nch), C.c_void_p(int(d_in)), C.c_void_p(int(d_out)),
                                                                int(n_blocks), int(stride)))
 
+    def update_list(self, channels, x, out=None):
+        """Only the listed chain channels, in list order: row i of x (int16 [len(channels), n_blocks*128], HOST memory) is
+        channel channels[i]; returns the audio of those rows, same shape."""
+        ch = np.ascontiguousarray(channels, np.uint32).ravel()
+        x = np.asarray(x)
+        assert x.dtype == np.int16 and x.ndim == 2 and x.shape[0] == ch.size and x.shape[1] % capi.BLOCK == 0
+        assert x.strides[1] == 2 and x.strides[0] % 2 == 0
+        if out is None:
+            out = np.empty(x.shape, np.int16)
+        assert out.dtype == np.int16 and out.shape == x.shape and out.strides[1] == 2
+        assert out.strides[0] == x.strides[0], "in/out must share the row stride"
+        self._ck(self._L.msdr_chain_update_list(self.h, capi.ptr(ch), ch.size, capi.ptr(x), capi.ptr(out), x.shape[1] // capi.BLOCK,
+                                                x.strides[0] // 2))
+        return out
+
+    def update_list_device(self, channels, d_in, d_out, n_blocks, stride):
+        """Only the listed chain channels (host array, any order); device buffers of len(channels) rows, row i = channels[i]."""
+        ch = np.ascontiguousarray(channels, np.uint32).ravel()
+        return self._ck(self._L.msdr_chain_update_list_device(self.h, capi.ptr(ch), ch.size, C.c_void_p(int(d_in)), C.c_void_p(int(d_out)),
+                                                              int(n_blocks), int(stride)))
+
     # -- raw ADC codes in: the front end (frontend.Frontend) per channel in front of the chain -----------------------------------
     def enable_frontend(self, agc_start=0.25, agc_max=40.0, agc_on=True):
         """(Re)initialise every channel's front end like frontend.Frontend(...): DC-block state 0, AGC at agc_start."""

@@ -81,11 +81,16 @@ struct msdr_chain {
     uint32_t *d_rowmap = nullptr, *d_wave_rb0 = nullptr;
     uint4 *d_rb = nullptr;
     uint8_t *d_bmat = nullptr;
+    std::vector<uint32_t> list;  // a channel-list plan: row r is chain channel list[r] (ch0 = 0, nch = list size); empty for a range
+    uint32_t *d_list = nullptr;  // the same on the device (ChainParams::chlist)
   };
-  // one plan per updated channel range: msdr_chain_update cuts wide chains into channel chunks, each its own range
+  // one plan per updated channel range or channel list: msdr_chain_update cuts wide chains into channel chunks, each its own range
   static constexpr size_t kMaxPlans = 64;
   std::vector<TcPlan> plans;
   size_t plan_victim = 0;
+  // channel-list updates: list_seen[c] == list_stamp marks a channel already met in the list being checked
+  std::vector<uint32_t> list_seen;
+  uint32_t list_stamp = 0;
   int *d_tile_cnt = nullptr;
   size_t tile_cnt_len = 0;
 
@@ -108,6 +113,7 @@ struct msdr_chain {
     bool cached = false;
     uint64_t key_epoch = 0, key_version = 0;
     uint32_t key_ch0 = 0, key_nch = 0;
+    std::vector<uint32_t> key_list;    // the channel list of the last update; empty for a range
     std::vector<uint32_t> chmap;
     std::vector<uint8_t> kind, amode;
     std::vector<uint32_t> channels;    // every chain channel that needs the lane, ascending
@@ -560,7 +566,7 @@ namespace {
 
 void free_tc_plan(msdr_chain::TcPlan &pl)
 {
-  cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32);
+  cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32); cudaFree(pl.d_list);
   pl = msdr_chain::TcPlan{};
 }
 
@@ -573,15 +579,20 @@ void free_tc_plan(msdr_chain::TcPlan &pl)
 // window leaves room for the second set of chain slots (rings[3]), which is known before any row is sorted — so the wave width
 // is chosen once and an unchanged configuration always hits the cache (256 taps beyond 148 groups used to rebuild twice per update).
 // want_v6: also the group-block plan of the time-folded kernel (msdr_chain_v6.cu), if the window fits that kernel.
-int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, bool want_dual, bool want_v6, const msdr_chain::TcPlan **out)
+// list != NULL: the rows are the chain channels list[0 .. nch) (ch0 = 0) instead of the range; the plan keeps the list, and a lookup
+// compares its contents.
+int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, uint32_t sms, bool want_dual, bool want_v6,
+                  const msdr_chain::TcPlan **out)
 {
   for (const auto &c : chain->plans)
-    if (c.version == chain->meta_version && c.ch0 == ch0 && c.nch == nch && c.sms == sms && c.want_dual == want_dual && c.want_v6 == want_v6) {
+    if (c.version == chain->meta_version && c.ch0 == ch0 && c.nch == nch && c.sms == sms && c.want_dual == want_dual && c.want_v6 == want_v6 &&
+        c.list.empty() == !list && (!list || std::equal(c.list.begin(), c.list.end(), list))) {
       *out = &c;
       return MSDR_OK;
     }
+  auto chan = [&](uint32_t r) { return list ? list[r] : ch0 + r; }; // chain channel of row r
   uint32_t kp_max = 0;
-  for (uint32_t c = ch0; c < ch0 + nch; ++c) kp_max = std::max(kp_max, kp_of_taps(chain->sets[chain->h_set[c]].T));
+  for (uint32_t r = 0; r < nch; ++r) kp_max = std::max(kp_max, kp_of_taps(chain->sets[chain->h_set[chan(r)]].T));
   const uint32_t K = tc_window_words_kp(kp_max);
   int smem_max = 0;
   CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, chain->device));
@@ -617,7 +628,7 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
   for (uint32_t g0 = 0; g0 < NG; g0 += W) {
     const uint32_t g1 = std::min(NG, g0 + W);
     for (auto &b : bucket) b.clear();
-    for (uint32_t r = g0 * kGroup; r < std::min(nch, g1 * (uint32_t)kGroup); ++r) bucket[chain->h_set[ch0 + r]].push_back(r);
+    for (uint32_t r = g0 * kGroup; r < std::min(nch, g1 * (uint32_t)kGroup); ++r) bucket[chain->h_set[chan(r)]].push_back(r);
     for (uint32_t sid = 0; sid < n_sets; ++sid) {
       const std::vector<uint32_t> &rows = bucket[sid];
       for (size_t i0 = 0; i0 < rows.size(); i0 += M) {
@@ -640,13 +651,13 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
     struct Half { uint32_t sid; size_t i0; bool costly; };
     std::vector<Half> costly, cheap;
     for (auto &b : bucket) b.clear();
-    for (uint32_t r = 0; r < nch; ++r) bucket[chain->h_set[ch0 + r]].push_back(r);
+    for (uint32_t r = 0; r < nch; ++r) bucket[chain->h_set[chan(r)]].push_back(r);
     for (uint32_t sid = 0; sid < n_sets; ++sid) {
       const std::vector<uint32_t> &rows = bucket[sid];
       for (size_t i0 = 0; i0 < rows.size(); i0 += HR) {
         bool env = false;
         for (size_t i = i0; i < std::min(rows.size(), i0 + HR); ++i) {
-          const int md = chain->h_mode[ch0 + rows[i]];
+          const int md = chain->h_mode[chan(rows[i])];
           env |= !(md == MSDR_MODE_LSB || md == MSDR_MODE_USB);
         }
         (env ? costly : cheap).push_back(Half{sid, i0, env});
@@ -695,6 +706,11 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t sms, b
     CK(cudaMemcpyAsync(pl.d_rowmap32, rowmap32.data(), rowmap32.size() * 4, cudaMemcpyHostToDevice, chain->stream));
     CK(cudaMemcpyAsync(pl.d_rb32, rbs32.data(), rbs32.size() * sizeof(uint4), cudaMemcpyHostToDevice, chain->stream));
   }
+  if (list) {
+    pl.list.assign(list, list + nch);
+    CK(cudaMalloc(&pl.d_list, (size_t)nch * 4));
+    CK(cudaMemcpyAsync(pl.d_list, pl.list.data(), (size_t)nch * 4, cudaMemcpyHostToDevice, chain->stream));
+  }
   // On the chain's stream, NOT cudaMemcpy: a synchronous copy from pageable memory returns once the data is staged, its DMA runs in
   // the legacy stream, and the chain's stream is non-blocking - a kernel launched right after could read the plan before it had
   // arrived (seen as intermittent mismatches in the last, ragged channel chunk of msdr_chain_update).
@@ -736,26 +752,33 @@ bool side_lane_in_range(msdr_chain *chain, uint32_t ch0, uint32_t nch)
   return it != ch.end() && *it < ch0 + nch;
 }
 
-int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, size_t stride, uint32_t L)
+// list != NULL: the update's rows are the chain channels list[0 .. nch) (ch0 = 0)
+int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, const int16_t *d_in, size_t stride, uint32_t L)
 {
   msdr_chain::PllLane &ln = chain->pll;
   const bool pll_build = !(chain->flags & MSDR_FLAG_AM_Q31); // Teensy 3.2 arithmetic: SYNCAM is the q31 envelope (.ino:618-620)
-  // The lane's index vectors depend on the range, the modes / ANR switches (epoch) and the table bindings (meta_version) only: an update
-  // that repeats the last one's configuration re-uses them on the device, and nothing in this function waits for the stream.
-  const bool hit = ln.cached && ln.key_epoch == ln.epoch && ln.key_version == chain->meta_version && ln.key_ch0 == ch0 && ln.key_nch == nch;
+  // The lane's index vectors depend on the range or list, the modes / ANR switches (epoch) and the table bindings (meta_version) only: an
+  // update that repeats the last one's configuration re-uses them on the device, and nothing in this function waits for the stream.
+  const bool hit = ln.cached && ln.key_epoch == ln.epoch && ln.key_version == chain->meta_version && ln.key_ch0 == ch0 && ln.key_nch == nch &&
+                   ln.key_list.empty() == !list && (!list || std::equal(ln.key_list.begin(), ln.key_list.end(), list));
+  auto chan = [&](uint32_t r) { return list ? list[r] : ch0 + r; }; // chain channel of row r
   if (!hit) {
     ln.rows.clear();
     ln.any_pll = ln.any_anr = false;
-    side_lane_channels(chain);
-    for (auto it = std::lower_bound(ln.channels.begin(), ln.channels.end(), ch0); it != ln.channels.end() && *it < ch0 + nch; ++it) {
-      const uint32_t r = *it - ch0;
-      const bool is_pll = pll_build && chain->h_mode[ch0 + r] == MSDR_MODE_SYNCAM;
-      const bool is_anr = chain->n_anr && chain->h_anr[ch0 + r] != 0;
-      ln.rows.push_back(r);
+    auto take = [&](uint32_t r) {
+      const bool is_pll = pll_build && chain->h_mode[chan(r)] == MSDR_MODE_SYNCAM;
+      const bool is_anr = chain->n_anr && chain->h_anr[chan(r)] != 0;
+      if (!list || is_pll || is_anr) ln.rows.push_back(r);
       ln.any_pll |= is_pll; ln.any_anr |= is_anr;
-    }
-    std::stable_sort(ln.rows.begin(), ln.rows.end(), [&](uint32_t a, uint32_t b) { return chain->h_set[ch0 + a] < chain->h_set[ch0 + b]; });
+    };
+    const std::vector<uint32_t> &lane = side_lane_channels(chain);
+    if (!list)
+      for (auto it = std::lower_bound(lane.begin(), lane.end(), ch0); it != lane.end() && *it < ch0 + nch; ++it) take(*it - ch0);
+    else if (!lane.empty())
+      for (uint32_t r = 0; r < nch; ++r) take(r);
+    std::stable_sort(ln.rows.begin(), ln.rows.end(), [&](uint32_t a, uint32_t b) { return chain->h_set[chan(a)] < chain->h_set[chan(b)]; });
     ln.cached = true; ln.key_epoch = ln.epoch; ln.key_version = chain->meta_version; ln.key_ch0 = ch0; ln.key_nch = nch;
+    if (list) ln.key_list.assign(list, list + nch); else ln.key_list.clear();
   }
   if (ln.rows.empty()) return MSDR_OK;
   const uint32_t n = (uint32_t)ln.rows.size();
@@ -777,7 +800,7 @@ int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int
   if (upload) {
     ln.chmap.resize(n); ln.kind.resize(n); ln.amode.resize(n);
     for (uint32_t i = 0; i < n; ++i) {
-      const uint32_t ch = ch0 + ln.rows[i];
+      const uint32_t ch = chan(ln.rows[i]);
       ln.chmap[i] = ch;
       const int md = chain->h_mode[ch];
       // demodulation kind of the row (Minimal-SDR.ino:589-628); 255 = the PLL demodulator takes the row
@@ -790,13 +813,14 @@ int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int
     CK(cudaMemcpyAsync(ln.d_kind, ln.kind.data(), n, cudaMemcpyHostToDevice, chain->stream));
     CK(cudaMemcpyAsync(ln.d_anr_mode, ln.amode.data(), n, cudaMemcpyHostToDevice, chain->stream));
   }
-  CK(launch_gather_rows(ln.d_rows, n, ch0, chain->d_hist, chain->H, d_in, stride, ln.d_raw, L, chain->stream));
-  CK(launch_bq_words(0, ln.d_rows, n, ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
+  const uint32_t *d_chmap = list ? ln.d_chmap : nullptr;
+  CK(launch_gather_rows(ln.d_rows, d_chmap, n, ch0, chain->d_hist, chain->H, d_in, stride, ln.d_raw, L, chain->stream));
+  CK(launch_bq_words(0, ln.d_rows, d_chmap, n, ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
   chain->launches += 2;
   return MSDR_OK;
 }
 
-int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, int16_t *d_out, size_t stride, uint32_t L)
+int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, bool list, int16_t *d_out, size_t stride, uint32_t L)
 {
   msdr_chain::PllLane &ln = chain->pll;
   if (ln.rows.empty()) return MSDR_OK;
@@ -804,9 +828,9 @@ int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, int16_t *d_out, size_t s
   const size_t Lp = (size_t)H + L;
   CK(launch_mix_fs4(ln.d_raw, ln.d_I, ln.d_Q, n, (uint32_t)Lp, Lp, chain->stream));
   for (uint32_t i0 = 0; i0 < n;) { // one FIR launch pair per run of channels sharing a tap table
-    const uint8_t sid = chain->h_set[ch0 + ln.rows[i0]];
+    const uint8_t sid = chain->h_set[ln.chmap[i0]];
     uint32_t i1 = i0;
-    while (i1 < n && chain->h_set[ch0 + ln.rows[i1]] == sid) ++i1;
+    while (i1 < n && chain->h_set[ln.chmap[i1]] == sid) ++i1;
     const FirSet &fs = chain->sets[sid];
     const int16_t *taps = chain->d_set_taps + (size_t)sid * 2 * MSDR_MAX_TAPS; // resident since upload_set: no copy, no wait per table
     CK(launch_fir_fast_q15(fs.T, taps, nullptr, nullptr, ln.d_I + i0 * Lp, ln.d_If + i0 * Lp, i1 - i0, (uint32_t)Lp, Lp, chain->stream));
@@ -823,7 +847,7 @@ int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, int16_t *d_out, size_t s
   CK(launch_biquad(ln.d_defs, audio, n, L, Lp, chain->stream));
   CK(launch_biquad(ln.d_defs + (size_t)n * 32, audio, n, L, Lp, chain->stream));
   CK(launch_scatter_rows(ln.d_rows, n, audio, Lp, d_out, stride, L, chain->stream));
-  CK(launch_bq_words(1, ln.d_rows, n, ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
+  CK(launch_bq_words(1, ln.d_rows, list ? ln.d_chmap : nullptr, n, ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
   chain->launches += 6;
   return MSDR_OK;
 }
@@ -848,10 +872,25 @@ struct Choice {
   uint32_t shape = 0; // v4 (tc_ff): 0 post warps, 1 classic, 2 feed-forward helper warps, 3 two chain sets per SM
 };
 
-// The fused kernel for the range [ch0, ch0 + nch) of NG channel groups on `sms` SMs, and the row plan it runs from.
-int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t NG, int sms, Choice &ch)
+// The fused kernel for the range [ch0, ch0 + nch) (or the channel list[0 .. nch)) of NG channel groups on `sms` SMs, and the row plan
+// it runs from.
+int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, uint32_t NG, int sms, Choice &ch)
 {
   const int v = chain->variant;
+  if (list) {
+    // A channel list has no chain kernel v4 form (its chain warps own contiguous 32-channel groups): the time-folded kernel when its
+    // group blocks fit one per SM, else the row-block kernels whatever the channel count.  The plan has one wave (sms = NG), and the
+    // v6 group blocks are only asked for when the list's channel groups alone fit.
+    const int v6_sms = std::max(1, sms - (int)chain->spare_sms);
+    const bool want_v6 = !(v & (kNoV6 | kForceV5)) && ((v & kForceV6) || NG <= (uint32_t)v6_sms);
+    const int st = build_tc_plan(chain, 0, nch, list, NG, false, want_v6, &ch.plan);
+    if (st != MSDR_OK) return st;
+    const msdr_chain::TcPlan &pl = *ch.plan;
+    if (pl.slots_v6 && ((v & kForceV6) || pl.n_gb <= (uint32_t)v6_sms)) ch.kernel = kV6;
+    else if (pl.ring_v5 || pl.ring_v5l) ch.kernel = !pl.ring_v5 || ((v & kV5lAnyWindow) && pl.ring_v5l) ? kV5l : kV5;
+    else return fail(chain, MSDR_ERR_UNSUPPORTED, "update_list: the FIR window of " + std::to_string(pl.K) + " words fits no kernel with a channel-list form");
+    return MSDR_OK;
+  }
   // Many channels: the row-block kernel (msdr_chain_v5.cu), one CTA per 128 channels of one tap table walking through time.  It
   // needs enough row blocks to fill the SMs (kV5MinChannels: below that the pinned chains of msdr_chain_v4.cu win).
   // (more channel groups than one wave of two chain sets per SM holds - 9472 channels on 148 SMs - would make msdr_chain_v4.cu walk a
@@ -866,7 +905,7 @@ int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t NG, in
       if (fs.users) kp_live = std::max(kp_live, kp_of_taps(fs.T));
     const uint32_t K = tc_window_words_kp(kp_live);
     if (chain_v5_config(K, smem_max) || chain_v5l_config(K, smem_max)) { // a plan with ONE wave: rows sorted by table over the range
-      const int st = build_tc_plan(chain, ch0, nch, NG, false, false, &ch.plan);
+      const int st = build_tc_plan(chain, ch0, nch, nullptr, NG, false, false, &ch.plan);
       if (st != MSDR_OK) return st;
       const msdr_chain::TcPlan &pl = *ch.plan;
       if (pl.ring_v5 || pl.ring_v5l) { // else no row-block form fits this window: the kernels below
@@ -881,7 +920,7 @@ int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t NG, in
   const bool want_v6 = !(v & (kNoV6 | kV4Study)) && (nch <= 8192u || (v & kForceV6));
   // more channel groups than SMs: two chain sets per SM (waves of 2 x SMs groups)
   const bool want_dual = NG > (uint32_t)sms && !(v & kV4Study);
-  const int st = build_tc_plan(chain, ch0, nch, (uint32_t)sms, want_dual, want_v6, &ch.plan);
+  const int st = build_tc_plan(chain, ch0, nch, nullptr, (uint32_t)sms, want_dual, want_v6, &ch.plan);
   if (st != MSDR_OK) return st;
   const msdr_chain::TcPlan &pl = *ch.plan;
   if (pl.slots_v6 && ((v & kForceV6) || pl.n_gb <= (uint32_t)std::max(1, sms - (int)chain->spare_sms))) {
@@ -948,15 +987,35 @@ int prof_dump(msdr_chain *chain, Kernel k, long long *d_prof, uint32_t g, uint32
   return MSDR_OK;
 }
 
+// Refuses a channel list with a channel outside the chain or listed twice (two rows would race on one channel's state).
+int check_list(msdr_chain *chain, const uint32_t *list, uint32_t n)
+{
+  if (chain->list_seen.size() != chain->C) { chain->list_seen.assign(chain->C, 0u); chain->list_stamp = 0; }
+  if (++chain->list_stamp == 0) { std::fill(chain->list_seen.begin(), chain->list_seen.end(), 0u); chain->list_stamp = 1; }
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t c = list[i];
+    if (c >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: channel " + std::to_string(c) + " is not in the chain");
+    if (chain->list_seen[c] == chain->list_stamp) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: channel " + std::to_string(c) + " is listed twice");
+    chain->list_seen[c] = chain->list_stamp;
+  }
+  return MSDR_OK;
+}
+
 // d_adc != NULL: the rows are raw ADC codes for the chain's front end.  Where the int16 input would run the row-block kernels and no
 // channel of the range is on the side lane (which gathers IF samples from `d_in`), the front end runs inside their converters; in
 // every other case K4 conditions the range into a scratch buffer first and the int16 path follows.  Both are bit-exact.
-int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks, size_t stride,
-                 const uint16_t *d_adc)
+// list != NULL (int16 input only, ch0 = 0): row r of d_in / d_out is chain channel list[r] instead of ch0 + r.
+int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
+                 size_t stride, const uint16_t *d_adc)
 {
   if (n_blocks == 0 || nch == 0) return MSDR_OK;
   const uint64_t L64 = (uint64_t)n_blocks * MSDR_BLOCK_SAMPLES;
-  if (!range_ok(chain, ch0, nch)) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad channel range");
+  if (list) {
+    const int st = check_list(chain, list, nch);
+    if (st != MSDR_OK) return st;
+  } else if (!range_ok(chain, ch0, nch)) {
+    return fail(chain, MSDR_ERR_ARGUMENT, "update: bad channel range");
+  }
   const void *src_rows = d_adc ? static_cast<const void *>(d_adc) : static_cast<const void *>(d_in);
   if (!src_rows || !d_out || L64 > stride || L64 > 0x7FFFFF00ull) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
   if (((uintptr_t)src_rows & 15u) || ((uintptr_t)d_out & 15u) || (stride & 7u))
@@ -969,7 +1028,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d
   CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, chain->device));
   const uint32_t NG = (nch + kGroup - 1) / kGroup;
   Choice ch;
-  int st = choose_kernel(chain, ch0, nch, NG, sms, ch);
+  int st = choose_kernel(chain, ch0, nch, list, NG, sms, ch);
   if (st != MSDR_OK) return st;
   const msdr_chain::TcPlan &pl = *ch.plan;
   if (d_adc && ((ch.kernel != kV5 && ch.kernel != kV5l) || side_lane_in_range(chain, ch0, nch))) {
@@ -996,6 +1055,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d
   p.am_q31 = (chain->flags & MSDR_FLAG_AM_Q31) ? 1u : 0u;
   p.spare_sms = chain->spare_sms;
   p.NG = NG; p.tc_K = pl.K; p.tc_bmat = pl.d_bmat;
+  p.chlist = pl.d_list; // NULL for a range
   if (d_adc) { // fused: the converters read codes and condition them (msdr_chain_v5_common.cuh: FeRow)
     p.in = reinterpret_cast<const int16_t *>(d_adc);
     p.fe = chain->d_fe; p.agc_max = chain->fe_agc_max; p.agc_on = chain->fe_agc_on ? 1u : 0u;
@@ -1036,7 +1096,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d
     if ((st = usage_resolve(chain)) != MSDR_OK) return st; // the event pair is reused: fold the previous update in first
     CK(cudaEventRecord(chain->ev0, chain->stream));
   }
-  if ((st = syncam_lane_prepare(chain, ch0, nch, d_in, stride, p.L)) != MSDR_OK) return st;
+  if ((st = syncam_lane_prepare(chain, ch0, nch, list, d_in, stride, p.L)) != MSDR_OK) return st;
   static const bool prof_on = getenv("MSDR_PROF") != nullptr; // developer aid: per-role cycle counters on stderr
   long long *d_prof = nullptr;
   if (prof_on) {
@@ -1054,7 +1114,8 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *d
   chain->last_kernel = std::string("msdr::") + kNames[ch.kernel].ns + "::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; " +
                        (ch.kernel == kV4 ? kV4ShapeNames[ch.shape] : kNames[ch.kernel].form) + ")";
   if (p.fe) chain->last_kernel += "; front end fused into the converters";
-  if ((st = syncam_lane_finish(chain, ch0, d_out, stride, p.L)) != MSDR_OK) return st;
+  if (list) chain->last_kernel += "; channel list";
+  if ((st = syncam_lane_finish(chain, ch0, list != nullptr, d_out, stride, p.L)) != MSDR_OK) return st;
   if (chain->timed) {
     CK(cudaEventRecord(chain->ev1, chain->stream));
     chain->usage_pending = true;
@@ -1071,7 +1132,15 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
                                    size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
-  return update_range(chain, ch0, nch, d_in, d_out, n_blocks, stride, nullptr);
+  return update_range(chain, ch0, nch, nullptr, d_in, d_out, n_blocks, stride, nullptr);
+}
+
+int msdr_chain_update_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
+                                  size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: NULL channel list");
+  return update_range(chain, 0, n, channels, d_in, d_out, n_blocks, stride, nullptr);
 }
 
 int msdr_chain_update_device(msdr_chain *chain, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks, size_t stride)
@@ -1085,8 +1154,11 @@ namespace {
 // Host buffers: channels are cut into chunks that flow through a 3-slot device ring — H2D copy (stream copy_in),
 // fused kernel (chain stream), D2H copy (stream copy_out) — so PCIe traffic in both directions overlaps the kernels.
 // adc: `in` holds uint16 ADC codes (2 bytes a sample like int16 IF samples) for the chain's front end.
-int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride, bool adc)
+// list != NULL: the rows of `in` / `out` are the n chain channels list[0 .. n), cut into chunks of the list instead of the chain.
+int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride, bool adc, const uint32_t *list = nullptr,
+                  uint32_t n = 0)
 {
+  const uint32_t rows = list ? n : chain->C;
   const size_t L = (size_t)n_blocks * MSDR_BLOCK_SAMPLES;
   if (!in || !out || L > stride) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
   if (chain->n_uninit) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update: some channels have no FIR bound (call msdr_fir_init_q15)");
@@ -1103,8 +1175,8 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
     const size_t want = ((size_t)128 << 20) / ((size_t)deep * MSDR_BLOCK_SAMPLES * 2);
     Cc = (uint32_t)std::min<size_t>(1u << 19, std::max<size_t>(8192, (want + 4095) / 4096 * 4096));
   }
-  Cc = std::max<uint32_t>(kGroup, std::min(Cc, (chain->C + kGroup - 1) / kGroup * kGroup) / kGroup * kGroup);
-  if (nbk == 0) nbk = (uint32_t)std::max<size_t>(64, ((size_t)64 << 20) / ((size_t)std::min(Cc, chain->C) * MSDR_BLOCK_SAMPLES * 2));
+  Cc = std::max<uint32_t>(kGroup, std::min(Cc, (rows + kGroup - 1) / kGroup * kGroup) / kGroup * kGroup);
+  if (nbk == 0) nbk = (uint32_t)std::max<size_t>(64, ((size_t)64 << 20) / ((size_t)std::min(Cc, rows) * MSDR_BLOCK_SAMPLES * 2));
   nbk = std::min(nbk, n_blocks);
   const size_t Lc = (size_t)nbk * MSDR_BLOCK_SAMPLES; // device row pitch of a chunk
   const size_t slot_samples = (size_t)Cc * Lc;
@@ -1117,8 +1189,8 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
   cudaEvent_t *ev_h2d = chain->pipe_ev.data(), *ev_k = ev_h2d + kSlots, *ev_d2h = ev_k + kSlots;
   // everything queued so far on the chain stream (setters, earlier updates) precedes this update's first kernel by stream order
   uint32_t k = 0;
-  for (uint32_t c0 = 0; c0 < chain->C; c0 += Cc) {
-    const uint32_t nc = std::min(Cc, chain->C - c0);
+  for (uint32_t c0 = 0; c0 < rows; c0 += Cc) {
+    const uint32_t nc = std::min(Cc, rows - c0);
     for (uint32_t b0 = 0; b0 < n_blocks; b0 += nbk, ++k) { // time order within a channel range: state carries
       const uint32_t nb = std::min(nbk, n_blocks - b0);
       const size_t w = (size_t)nb * MSDR_BLOCK_SAMPLES * 2; // bytes per row in this chunk
@@ -1132,8 +1204,9 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
       CK(cudaMemcpy2DAsync(din, Lc * 2, in + hoff, stride * 2, w, nc, cudaMemcpyHostToDevice, chain->copy_in));
       CK(cudaEventRecord(ev_h2d[slot], chain->copy_in));
       CK(cudaStreamWaitEvent(chain->stream, ev_h2d[slot], 0));
-      st = adc ? msdr_chain_update_adc_range_device(chain, c0, nc, reinterpret_cast<const uint16_t *>(din), dout, nb, Lc)
-               : msdr_chain_update_range_device(chain, c0, nc, din, dout, nb, Lc);
+      st = list ? msdr_chain_update_list_device(chain, list + c0, nc, din, dout, nb, Lc)
+           : adc ? msdr_chain_update_adc_range_device(chain, c0, nc, reinterpret_cast<const uint16_t *>(din), dout, nb, Lc)
+                 : msdr_chain_update_range_device(chain, c0, nc, din, dout, nb, Lc);
       if (st != MSDR_OK) return st;
       CK(cudaEventRecord(ev_k[slot], chain->stream));
       CK(cudaStreamWaitEvent(chain->copy_out, ev_k[slot], 0));
@@ -1153,6 +1226,16 @@ int msdr_chain_update(msdr_chain *chain, const int16_t *in, int16_t *out, uint32
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (n_blocks == 0) return MSDR_OK;
   return host_pipeline(chain, in, out, n_blocks, stride, false);
+}
+
+int msdr_chain_update_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: NULL channel list");
+  if (n == 0 || n_blocks == 0) return MSDR_OK;
+  const int st = check_list(chain, channels, n); // the whole list before the first chunk is queued
+  if (st != MSDR_OK) return st;
+  return host_pipeline(chain, in, out, n_blocks, stride, false, channels, n);
 }
 
 // ---- ADC-code input: the front end of msdr_frontend.cu per chain channel, in front of the chain ------------------------------------
@@ -1195,7 +1278,7 @@ int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
-  const int st = update_range(chain, ch0, nch, nullptr, d_out, n_blocks, stride, d_adc);
+  const int st = update_range(chain, ch0, nch, nullptr, nullptr, d_out, n_blocks, stride, d_adc);
   if (st == MSDR_OK && chain->fe_composed) chain->last_kernel = "msdr::fe::frontend_kernel (front end), then " + chain->last_kernel;
   return st;
 }

@@ -74,7 +74,8 @@ size_t smem_bytes(uint32_t K, uint32_t ring)
 // here two biquad warps, two epilogue warps and a converter share a sub-partition and the integer multiplier is the scarce pipe
 // (IMAD.HI occupies it for 5 cycles), so the default moves three of the five products off it.
 // kAdc: `p.in` holds raw ADC codes; the converters run the front end over them (FeRow, msdr_chain_v5_common.cuh)
-template <class BQ, bool kAdc>
+// kList: launch row r is chain channel p.chlist[r] (chan_of); int16 input only
+template <class BQ, bool kAdc, bool kList = false>
 __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -126,7 +127,19 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
       uint32_t rows[M / 4];
 #pragma unroll
       for (int i = 0; i < M / 4; ++i) rows[i] = __ldg(rmap + r0 + 4 * i);
+      // a list: the same registers hold the rows' chain channels (their history rows) for the stages in front of sample 0, then
+      // the launch rows again (a second set of offsets beside them spilled)
+      if constexpr (kList) {
+#pragma unroll
+        for (int i = 0; i < M / 4; ++i) rows[i] = rows[i] != kPad ? chan_of<true>(p, rows[i]) : kPad;
+      }
       for (int j = -(int)(KS - 1); j < (int)NT; ++j, ++pseq) {
+        if constexpr (kList) {
+          if (j == 0) {
+#pragma unroll
+            for (int i = 0; i < M / 4; ++i) rows[i] = __ldg(p.tc_rowmap + (size_t)rb * M + r0 + 4 * i);
+          }
+        }
         const uint32_t stage = pseq % RS;
         prof.start();
         mbar_wait(&pc->raw_free[stage], ((pseq / RS) & 1u) ^ 1u, kNsLoad);
@@ -146,7 +159,8 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 #pragma unroll
           for (int i = 0; i < M / 4; ++i) {
             const bool valid = rows[i] != kPad && s >= -Hs;
-            const int16_t *src = valid ? p.hist + ((size_t)p.ch0 + rows[i]) * p.H + (Hs + s) : p.in; // never dereferenced when the size is 0
+            const size_t hc = kList ? (size_t)rows[i] : (size_t)p.ch0 + rows[i];
+            const int16_t *src = valid ? p.hist + hc * p.H + (Hs + s) : p.in; // never dereferenced when the size is 0
             asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst0 + (uint32_t)i * 4u * RAWP), "l"(src), "r"(valid ? 16 : 0) : "memory");
           }
         }
@@ -208,7 +222,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + r);
         if (row != kPad) {
           const uint32_t hq = p.H >> 3; // uint4 per history row (<= 33)
-          uint4 *hrow = reinterpret_cast<uint4 *>(p.hist + ((size_t)p.ch0 + row) * p.H);
+          uint4 *hrow = reinterpret_cast<uint4 *>(p.hist + hist_ch<kList>(p, row) * p.H);
           const uint4 *irow = reinterpret_cast<const uint4 *>(p.in + (size_t)row * p.stride);
           if (p.L >= p.H) {
             const uint4 *src = irow + ((p.L - p.H) >> 3);
@@ -269,7 +283,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
     uint32_t tseq = 0;
     for (uint32_t rb = blockIdx.x; rb < n_rb; rb += gridDim.x) {
       const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + trow);
-      const int kind = row != kPad ? demod_kind_of((int)p.mode[p.ch0 + row], p.am_q31) : 0;
+      const int kind = row != kPad ? demod_kind_of((int)p.mode[chan_of<kList>(p, row)], p.am_q31) : 0;
       // Eight columns per pass, the passes not unrolled: unrolled, the epilogue streamed ~7-26 KB of straight-line code per tile and warp
       // through the instruction caches it shares with the biquad warps (ncu: instruction-cache hit rate 86 %, no_instruction 8 % of the
       // warp samples; msdr_chain_v6.cu gained 16 % from the same change).  The per-branch tensor-memory hand-off stays: the I pass parks
@@ -351,7 +365,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
     for (uint32_t rb = blockIdx.x; rb < n_rb; rb += gridDim.x) {
       const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + trow);
       const bool active = row != kPad;
-      const uint32_t ch = p.ch0 + (active ? row : 0u);
+      const uint32_t ch = kList ? (active ? chan_of<true>(p, row) : 0u) : p.ch0 + (active ? row : 0u);
       // cascade structure of this lane's object: stages run while bit31 of word 7 says another follows (filter_biquad.cpp:75,79)
       int nst = 1;
       BQ st[1];
@@ -462,7 +476,7 @@ cudaError_t launch_chain_v5(const ChainParams &p_in, cudaStream_t stream, int va
   const size_t smem = smem_bytes(p.tc_K, p.tc_ring);
   // default: the products as IMAD.HI (with the looped epilogue 352 against 339 Gsamples/s at C5 for the IMAD.WIDE form, which was 1.5 %
   // ahead before); study knobs: variant bit 0 = IMAD.WIDE for the four products off the recurrence, bit 1 = feed-forward products as DFMA
-  auto kern = p.fe ? chain_kernel<BqStage, true>
+  auto kern = p.fe ? chain_kernel<BqStage, true> : p.chlist ? chain_kernel<BqStage, false, true>
                    : (variant & 12) == 12 ? chain_kernel<BqStageS, false> : (variant & 1) ? chain_kernel<BqStageW, false> : (variant & 2) ? chain_kernel<BqStageH, false>
                    : (variant & 4) ? chain_kernel<BqStageC, false> : (variant & 8) ? chain_kernel<BqStageE, false> : chain_kernel<BqStage, false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -12,6 +12,21 @@ namespace v5 {
 using namespace tc;
 
 constexpr uint32_t kPad = 0xFFFFFFFFu;
+
+// chain channel of launch row `row` (never kPad): its entry of the channel list, or ch0 + row for a range; hist_ch as the 64-bit index
+// of the history row (the range form keeps the index arithmetic the kernels had before lists)
+template <bool kList>
+__device__ __forceinline__ uint32_t chan_of(const ChainParams &p, uint32_t row)
+{
+  if constexpr (kList) return __ldg(p.chlist + row);
+  else return p.ch0 + row;
+}
+template <bool kList>
+__device__ __forceinline__ size_t hist_ch(const ChainParams &p, uint32_t row)
+{
+  if constexpr (kList) return __ldg(p.chlist + row);
+  else return (size_t)p.ch0 + row;
+}
 // sleep between mbarrier probes per role (nanoseconds; msdr_device.cuh::mbar_wait).  The tensor-memory hand-off between the MMA warp
 // and the epilogue is the kernel's tightest loop and probes often; everything that sits behind a ring of slots can afford to find
 // out late that its barrier has flipped, and its probes otherwise delay the dependent instruction chains of the biquad warps.

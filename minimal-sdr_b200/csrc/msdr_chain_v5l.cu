@@ -51,7 +51,8 @@ size_t smem_bytes(uint32_t K, uint32_t ring)
 }
 
 // kAdc: `p.in` holds raw ADC codes; the converters run the front end over them (FeRow, msdr_chain_v5_common.cuh)
-template <class BQ, bool kAdc>
+// kList: launch row r is chain channel p.chlist[r] (chan_of); int16 input only
+template <class BQ, bool kAdc, bool kList = false>
 __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -103,7 +104,19 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
       uint32_t rows[M / 8];
 #pragma unroll
       for (int i = 0; i < M / 8; ++i) rows[i] = __ldg(rmap + r0 + 8 * i);
+      // a list: the same registers hold the rows' chain channels (their history rows) for the stages in front of sample 0, then
+      // the launch rows again (a second set of offsets beside them spilled)
+      if constexpr (kList) {
+#pragma unroll
+        for (int i = 0; i < M / 8; ++i) rows[i] = rows[i] != kPad ? chan_of<true>(p, rows[i]) : kPad;
+      }
       for (int hh = -2 * (int)(KS - 1); hh < 2 * (int)NT; ++hh, ++hseq) {
+        if constexpr (kList) {
+          if (hh == 0) {
+#pragma unroll
+            for (int i = 0; i < M / 8; ++i) rows[i] = __ldg(p.tc_rowmap + (size_t)rb * M + r0 + 8 * i);
+          }
+        }
         const uint32_t stage = hseq % RSH;
         prof.start();
         mbar_wait(&pc->raw_free[stage], ((hseq / RSH) & 1u) ^ 1u, kNsLoad);
@@ -123,7 +136,8 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 #pragma unroll
           for (int i = 0; i < M / 8; ++i) {
             const bool valid = rows[i] != kPad && s >= -Hs;
-            const int16_t *src = valid ? p.hist + ((size_t)p.ch0 + rows[i]) * p.H + (Hs + s) : p.in; // never dereferenced when the size is 0
+            const size_t hc = kList ? (size_t)rows[i] : (size_t)p.ch0 + rows[i];
+            const int16_t *src = valid ? p.hist + hc * p.H + (Hs + s) : p.in; // never dereferenced when the size is 0
             asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst0 + (uint32_t)i * 8u * HP), "l"(src), "r"(valid ? 16 : 0) : "memory");
           }
         }
@@ -187,7 +201,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + r);
         if (row != kPad) {
           const uint32_t hq = p.H >> 3; // uint4 per history row (<= 33)
-          uint4 *hrow = reinterpret_cast<uint4 *>(p.hist + ((size_t)p.ch0 + row) * p.H);
+          uint4 *hrow = reinterpret_cast<uint4 *>(p.hist + hist_ch<kList>(p, row) * p.H);
           const uint4 *irow = reinterpret_cast<const uint4 *>(p.in + (size_t)row * p.stride);
           if (p.L >= p.H) {
             const uint4 *src = irow + ((p.L - p.H) >> 3);
@@ -246,7 +260,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
     uint32_t tseq = 0;
     for (uint32_t rb = blockIdx.x; rb < n_rb; rb += gridDim.x) {
       const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + trow);
-      const int kind = row != kPad ? demod_kind_of((int)p.mode[p.ch0 + row], p.am_q31) : 0;
+      const int kind = row != kPad ? demod_kind_of((int)p.mode[chan_of<kList>(p, row)], p.am_q31) : 0;
       for (uint32_t t = 0; t < NT; ++t, ++tseq) {
         const uint32_t useq = 2u * tseq + (uint32_t)half, slot = useq % NH; // this warp's half-slot of the tile
         uint32_t iq[32];
@@ -314,7 +328,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
     for (uint32_t rb = blockIdx.x; rb < n_rb; rb += gridDim.x) {
       const uint32_t row = __ldg(p.tc_rowmap + (size_t)rb * M + trow);
       const bool active = row != kPad;
-      const uint32_t ch = p.ch0 + (active ? row : 0u);
+      const uint32_t ch = kList ? (active ? chan_of<true>(p, row) : 0u) : p.ch0 + (active ? row : 0u);
       // cascade structure of this lane's object: stages run while bit31 of word 7 says another follows (filter_biquad.cpp:75,79)
       int nst = 1;
       BQ st[1];
@@ -422,7 +436,7 @@ cudaError_t launch_chain_v5l(const ChainParams &p_in, cudaStream_t stream, int v
   p.ablate = ((uint32_t)variant >> 4) & 3u;
   const size_t smem = smem_bytes(p.tc_K, p.tc_ring);
   // variant bit 0: all five products as IMAD.HI (cross-check)
-  auto kern = p.fe ? chain_kernel<BqStageW, true> : (variant & 1) ? chain_kernel<BqStage, false> : chain_kernel<BqStageW, false>;
+  auto kern = p.fe ? chain_kernel<BqStageW, true> : p.chlist ? chain_kernel<BqStageW, false, true> : (variant & 1) ? chain_kernel<BqStage, false> : chain_kernel<BqStageW, false>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   const uint32_t grid = p.n_items < (uint32_t)sms ? p.n_items : (uint32_t)sms;

@@ -193,7 +193,8 @@ __device__ __forceinline__ void bq_store_ff(const BqFFI &f, int32_t *__restrict_
   bq[(size_t)(obj * 4 * 8 + 5) * Cpad + ch] = (int32_t)(((uint32_t)f.x1 & 0xFFFF0000u) | ((uint32_t)f.x2 >> 16));
 }
 
-template <class FFT>
+// kList: launch row r is chain channel p.chlist[r] (chan_of); int16 input only
+template <class FFT, bool kList = false>
 __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -297,6 +298,9 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         if (lane == 0) mbar_arrive(&pc->b_full);
       }
       const uint32_t row2[2] = {__ldg(p.tc_rowmap + (size_t)gb * G + rr), __ldg(p.tc_rowmap + (size_t)gb * G + HR + rr)};
+      uint32_t hch2[kList ? 2 : 1]; // a list's history rows
+      if constexpr (kList)
+        for (int h = 0; h < 2; ++h) hch2[h] = row2[h] != kPad ? v5::chan_of<true>(p, row2[h]) : 0u;
       for (uint32_t s = 0; s < nspan; ++s, ++sseq) {
 #pragma unroll
         for (int h = 0; h < 2; ++h, ++tseq) {
@@ -324,7 +328,8 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                   const int smp = ((int)x - (int)KH) * 32 + 8 * j;
-                  v[j] = (row != kPad && smp >= -Hs) ? __ldg(reinterpret_cast<const uint4 *>(p.hist + ((size_t)p.ch0 + row) * p.H + (Hs + smp))) : make_uint4(0, 0, 0, 0);
+                  const size_t hc = kList ? (size_t)hch2[kList ? h : 0] : (size_t)p.ch0 + row;
+                  v[j] = (row != kPad && smp >= -Hs) ? __ldg(reinterpret_cast<const uint4 *>(p.hist + hc * p.H + (Hs + smp))) : make_uint4(0, 0, 0, 0);
                 }
                 convert_unit(abuf, a_plane, x, rr, v);
               }
@@ -349,7 +354,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
         const uint32_t row = __ldg(p.tc_rowmap + (size_t)gb * G + t);
         if (row != kPad) {
           const uint32_t hq = p.H >> 3; // uint4 per history row (<= 33)
-          uint4 *hrow = reinterpret_cast<uint4 *>(p.hist + ((size_t)p.ch0 + row) * p.H);
+          uint4 *hrow = reinterpret_cast<uint4 *>(p.hist + v5::hist_ch<kList>(p, row) * p.H);
           const uint4 *irow = reinterpret_cast<const uint4 *>(p.in + (size_t)row * p.stride);
           if (p.L >= p.H) {
             const uint4 *src = irow + ((p.L - p.H) >> 3);
@@ -425,7 +430,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
         const uint32_t row = __ldg(p.tc_rowmap + (size_t)gb * G + h * HR + rr);
-        kind2[h] = row != kPad ? demod_kind_of((int)p.mode[p.ch0 + row], p.am_q31) : 0;
+        kind2[h] = row != kPad ? demod_kind_of((int)p.mode[v5::chan_of<kList>(p, row)], p.am_q31) : 0;
       }
       // The loops below are deliberately NOT unrolled over tiles and column groups: the kernel's roles together stream far more
       // straight-line code than the instruction caches hold, and SMs with a longer path to the next cache level fell 7 % behind
@@ -514,7 +519,7 @@ __global__ void __launch_bounds__(kThreads, 1) chain_kernel(const ChainParams p)
     for (uint32_t gb = blockIdx.x; gb < n_gb; gb += gridDim.x) {
       const uint32_t row = __ldg(p.tc_rowmap + (size_t)gb * G + lane);
       const bool active = row != kPad;
-      const uint32_t ch = p.ch0 + (active ? row : 0u);
+      const uint32_t ch = kList ? (active ? v5::chan_of<true>(p, row) : 0u) : p.ch0 + (active ? row : 0u);
       // is every lane's object a single stage?  (generic cascades run whole stages in the chain warps, state in global)
       int nst = 1;
       if (active) {
@@ -749,7 +754,7 @@ cudaError_t launch_chain_v6(const ChainParams &p_in, cudaStream_t stream, int va
   p.ablate = ((uint32_t)variant >> 4) & 3u;
   if (const char *ev = getenv("MSDR_ABLATE")) p.ablate |= (uint32_t)atoi(ev) & ~3u; // study only: 4 = no demodulation, 8 = no TMEM drain (results are wrong)
   const size_t smem = smem_bytes(p.tc_K, p.tc_ring);
-  auto kern = (variant & 2) ? chain_kernel<BqFF> : chain_kernel<BqFFI>; // study knob: bit 1 = feed-forward products as DFMA instead of IMAD.HI
+  auto kern = p.chlist ? chain_kernel<BqFFI, true> : (variant & 2) ? chain_kernel<BqFF> : chain_kernel<BqFFI>; // study knob: bit 1 = feed-forward products as DFMA instead of IMAD.HI
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   const uint32_t grid = p.n_items < (uint32_t)sms ? p.n_items : (uint32_t)sms;

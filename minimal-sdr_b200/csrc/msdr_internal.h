@@ -50,6 +50,8 @@ struct ChainParams {
   fe::State *fe;               // [chain channels] front-end state, indexed like hist
   float agc_max;
   uint32_t agc_on;
+  // channel list (v5, v5l, v6 int16 only): non-NULL = launch row r is chain channel chlist[r] instead of ch0 + r
+  const uint32_t *chlist;
 };
 
 struct ChainLaunchInfo {
@@ -68,7 +70,7 @@ bool chain_v4_config(uint32_t K, int smem_max, uint32_t rings[4]);
 cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, uint32_t C, uint32_t n_blocks, fe::State *state, float agc_max,
                             int agc_on, int sms, cudaStream_t s);
 // row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config (0 = does not fit);
-// p.fe != NULL selects the ADC-code instantiation (default biquad form only)
+// p.fe != NULL selects the ADC-code instantiation (default biquad form only), p.chlist != NULL the channel-list one (the same)
 cudaError_t launch_chain_v5(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
 uint32_t chain_v5_config(uint32_t K, int smem_max);
 // pinned 32-channel group blocks with the tile rows folded over time (msdr_chain_v6.cu): p.tc_rowmap = [n_items][32] rows,
@@ -85,11 +87,12 @@ cudaError_t launch_mix_fs4(const int16_t *in, int16_t *I, int16_t *Q, uint32_t r
 cudaError_t launch_fir_fast_q15(uint32_t T, const int16_t *coef, const int16_t *hist_in, int16_t *hist_out, const int16_t *in, int16_t *out,
                                 uint32_t rows, uint32_t n, size_t stride, cudaStream_t s);
 cudaError_t launch_demod(int kind, const int16_t *I, const int16_t *Q, int16_t *out, uint32_t rows, uint32_t n, size_t stride, cudaStream_t s);
-cudaError_t launch_gather_rows(const uint32_t *rows, uint32_t n, uint32_t ch0, const int16_t *hist, uint32_t H, const int16_t *in, size_t stride, int16_t *raw,
-                               uint32_t L, cudaStream_t s);
+// side-lane glue (msdr_stage_kernels.cu): chmap != NULL gives the chain channel of each scratch row, else it is ch0 + rows[i]
+cudaError_t launch_gather_rows(const uint32_t *rows, const uint32_t *chmap, uint32_t n, uint32_t ch0, const int16_t *hist, uint32_t H, const int16_t *in, size_t stride,
+                               int16_t *raw, uint32_t L, cudaStream_t s);
 cudaError_t launch_scatter_rows(const uint32_t *rows, uint32_t n, const int16_t *audio, size_t astride, int16_t *out, size_t stride, uint32_t L, cudaStream_t s);
 cudaError_t launch_zero_hist_rows(int16_t *hist, uint32_t H, const uint32_t *channels, uint32_t n, cudaStream_t s);
-cudaError_t launch_bq_words(int dir, const uint32_t *rows, uint32_t n, uint32_t ch0, int32_t *bq, uint32_t Cpad, int32_t *defs, cudaStream_t s);
+cudaError_t launch_bq_words(int dir, const uint32_t *rows, const uint32_t *chmap, uint32_t n, uint32_t ch0, int32_t *bq, uint32_t Cpad, int32_t *defs, cudaStream_t s);
 cudaError_t launch_demod_rows(const uint8_t *kinds, const int16_t *I, const int16_t *Q, size_t stride, int16_t *out, size_t ostride, uint32_t rows, uint32_t n,
                               cudaStream_t s);
 cudaError_t launch_anr(int16_t *data, size_t stride, uint32_t rows, uint32_t n_blocks, const uint8_t *row_mode, const uint32_t *chmap, float *d, float *w,

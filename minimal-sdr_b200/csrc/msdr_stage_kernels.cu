@@ -302,14 +302,15 @@ cudaError_t launch_sqrt_check(unsigned long long *d_mismatch, cudaStream_t s)
 
 
 // ---- glue for channels the fused kernel does not demodulate itself (mode SYNCAM with the f32 PLL): rows and biquad words are
-// copied out to dense scratch arrays, run through the stage kernels, and copied back (msdr_capi.cu)
-__global__ void gather_rows_kernel(const uint32_t *__restrict__ rows, uint32_t ch0, const int16_t *__restrict__ hist, uint32_t H,
+// copied out to dense scratch arrays, run through the stage kernels, and copied back (msdr_capi.cu).  The chain channel of scratch row i
+// is chmap[i] when a channel map is given (a channel-list update), else ch0 + rows[i].
+__global__ void gather_rows_kernel(const uint32_t *__restrict__ rows, const uint32_t *__restrict__ chmap, uint32_t ch0, const int16_t *__restrict__ hist, uint32_t H,
                                    const int16_t *__restrict__ in, size_t stride, int16_t *__restrict__ raw, uint32_t L)
 {
   const uint32_t s = blockIdx.y, row = rows[s];
-  const size_t Lp = (size_t)H + L;
+  const size_t Lp = (size_t)H + L, ch = chmap ? (size_t)chmap[s] : (size_t)ch0 + row;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < Lp; i += (size_t)gridDim.x * blockDim.x)
-    raw[s * Lp + i] = i < H ? hist[((size_t)ch0 + row) * H + i] : in[(size_t)row * stride + (i - H)];
+    raw[s * Lp + i] = i < H ? hist[ch * H + i] : in[(size_t)row * stride + (i - H)];
 }
 __global__ void scatter_rows_kernel(const uint32_t *__restrict__ rows, const int16_t *__restrict__ audio, size_t astride, int16_t *__restrict__ out,
                                     size_t stride, uint32_t L)
@@ -319,12 +320,13 @@ __global__ void scatter_rows_kernel(const uint32_t *__restrict__ rows, const int
     out[(size_t)row * stride + i] = audio[s * astride + i];
 }
 // d_bq is [2 objects * 4 stages * 8 words][Cpad]; defs is [object][n][32]
-__global__ void bq_words_kernel(int dir, const uint32_t *__restrict__ rows, uint32_t ch0, int32_t *__restrict__ bq, uint32_t Cpad, int32_t *__restrict__ defs, uint32_t n)
+__global__ void bq_words_kernel(int dir, const uint32_t *__restrict__ rows, const uint32_t *__restrict__ chmap, uint32_t ch0, int32_t *__restrict__ bq, uint32_t Cpad,
+                                int32_t *__restrict__ defs, uint32_t n)
 {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n * 64u) return;
   const uint32_t s = i / 64u, w = i % 64u; // w = object * 32 + word
-  int32_t *g = bq + (size_t)w * Cpad + ch0 + rows[s];
+  int32_t *g = bq + (size_t)w * Cpad + (chmap ? chmap[s] : ch0 + rows[s]);
   int32_t *d = defs + ((size_t)(w / 32u) * n + s) * 32u + (w % 32u);
   if (dir == 0) *d = *g; else *g = *d;
 }
@@ -346,12 +348,13 @@ cudaError_t launch_demod_rows(const uint8_t *kinds, const int16_t *I, const int1
     demod_rows_kernel<<<dim3(8, std::min(rows - r0, 32768u)), 256, 0, s>>>(kinds + r0, I + (size_t)r0 * stride, Q + (size_t)r0 * stride, stride, out + (size_t)r0 * ostride, ostride, n);
   return cudaGetLastError();
 }
-cudaError_t launch_gather_rows(const uint32_t *rows, uint32_t n, uint32_t ch0, const int16_t *hist, uint32_t H, const int16_t *in, size_t stride, int16_t *raw,
-                               uint32_t L, cudaStream_t s)
+cudaError_t launch_gather_rows(const uint32_t *rows, const uint32_t *chmap, uint32_t n, uint32_t ch0, const int16_t *hist, uint32_t H, const int16_t *in, size_t stride,
+                               int16_t *raw, uint32_t L, cudaStream_t s)
 {
   if (n == 0) return cudaSuccess;
   for (uint32_t r0 = 0; r0 < n; r0 += 32768u) // gridDim.y limit
-    gather_rows_kernel<<<dim3(8, std::min(n - r0, 32768u)), 256, 0, s>>>(rows + r0, ch0, hist, H, in, stride, raw + (size_t)r0 * ((size_t)H + L), L);
+    gather_rows_kernel<<<dim3(8, std::min(n - r0, 32768u)), 256, 0, s>>>(rows + r0, chmap ? chmap + r0 : nullptr, ch0, hist, H, in, stride,
+                                                                         raw + (size_t)r0 * ((size_t)H + L), L);
   return cudaGetLastError();
 }
 cudaError_t launch_scatter_rows(const uint32_t *rows, uint32_t n, const int16_t *audio, size_t astride, int16_t *out, size_t stride, uint32_t L, cudaStream_t s)
@@ -375,10 +378,10 @@ cudaError_t launch_zero_hist_rows(int16_t *hist, uint32_t H, const uint32_t *cha
   zero_hist_rows_kernel<<<(unsigned)std::min<size_t>((total + 255) / 256, 148 * 16), 256, 0, s>>>(hist, H, channels, n);
   return cudaGetLastError();
 }
-cudaError_t launch_bq_words(int dir, const uint32_t *rows, uint32_t n, uint32_t ch0, int32_t *bq, uint32_t Cpad, int32_t *defs, cudaStream_t s)
+cudaError_t launch_bq_words(int dir, const uint32_t *rows, const uint32_t *chmap, uint32_t n, uint32_t ch0, int32_t *bq, uint32_t Cpad, int32_t *defs, cudaStream_t s)
 {
   if (n == 0) return cudaSuccess;
-  bq_words_kernel<<<(n * 64u + 255u) / 256u, 256, 0, s>>>(dir, rows, ch0, bq, Cpad, defs, n);
+  bq_words_kernel<<<(n * 64u + 255u) / 256u, 256, 0, s>>>(dir, rows, chmap, ch0, bq, Cpad, defs, n);
   return cudaGetLastError();
 }
 
