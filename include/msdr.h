@@ -129,11 +129,11 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
 /* Channels channels[0..n) only, in list order: row i of d_in / d_out is channel channels[i].  Same buffer, alignment, stride and
  * state rules as msdr_chain_update_range_device; results, outputs and state equal those of range updates of the same channels.
  * `channels` is a host array in any order.  MSDR_ERR_ARGUMENT, before anything is enqueued, for a channel >= the chain's
- * channel count, a channel listed twice, or channels == NULL with n > 0; n == 0 launches nothing.  int16 input only: the
- * front-end state (msdr_chain_enable_frontend) is left alone.  Runs on the time-folded kernel while the list's channel
- * groups fit one per SM, else on the row-block kernel, never on the chain kernel v4; scattered channels gather their state,
- * so a list can run below a range of the same size (rates: DESIGN.md §6).  The row plan of each distinct list is cached
- * like that of a range (INTEGRATION.md §3h). */
+ * channel count, a channel listed twice, or channels == NULL with n > 0; n == 0 launches nothing.  int16 input: the
+ * front-end state (msdr_chain_enable_frontend) is left alone (ADC codes: msdr_chain_update_adc_list_device).  Runs on the
+ * time-folded kernel while the list's channel groups fit one per SM, else on the row-block kernel, never on the chain kernel
+ * v4; scattered channels gather their state, so a list can run below a range of the same size (rates: DESIGN.md §6).  The
+ * row plan of each distinct list is cached like that of a range (INTEGRATION.md §3h). */
 int msdr_chain_update_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *d_in, int16_t *d_out,
                                   uint32_t n_blocks, size_t stride);
 /* The same on host buffers of n rows, through the 3-slot copy / kernel / copy pipeline of msdr_chain_update (the list is cut
@@ -299,11 +299,29 @@ int32_t msdr_amp_gain_multiplier(float gain);
    hpf 0, agc_idx 25, agc_val = agc_start, multiplier = gain(agc_start). */
 int msdr_chain_enable_frontend(msdr_chain *chain, float agc_start, float agc_max, int agc_on);
 int msdr_chain_frontend_preset(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint16_t first_reading); /* input_adc.cpp:59-63 */
+/* The same for the channels channels[0..n) (host array, any order): MSDR_ERR_ARGUMENT for a channel >= the chain's channel count
+ * or channels == NULL with n > 0, MSDR_ERR_NOT_INITIALISED before msdr_chain_enable_frontend; a refused call changes nothing.
+ * One synchronising call for the whole list; its cost grows with n, not with the span of the listed channels. */
+int msdr_chain_frontend_preset_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, uint16_t first_reading);
 /* MSDR_ERR_NOT_INITIALISED before msdr_chain_enable_frontend */
 int msdr_chain_update_adc(msdr_chain *chain, const uint16_t *adc, int16_t *out, uint32_t n_blocks, size_t stride);  /* host buffers */
 int msdr_chain_update_adc_device(msdr_chain *chain, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks, size_t stride);
 int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint16_t *d_adc, int16_t *d_out,
                                        uint32_t n_blocks, size_t stride);
+/* Channel lists of ADC codes: row i of d_adc / d_out is chain channel channels[i] (host array, any order), asynchronous on the
+ * chain's stream.  Output, chain state and front-end state equal those of msdr_chain_update_adc_range_device calls over the same
+ * channels, however a stream is cut into calls; unlisted channels, their front end included, are not touched.  Refusals, before
+ * anything is enqueued and changing nothing: MSDR_ERR_NOT_INITIALISED before msdr_chain_enable_frontend or while a channel has
+ * no FIR bound; MSDR_ERR_ARGUMENT for a channel >= the chain's channel count, a channel listed twice, channels == NULL with
+ * n > 0, or buffers, alignment and stride that msdr_chain_update_adc_range_device refuses.  n == 0 launches nothing.  The
+ * front-end kernel conditions the listed rows with each listed channel's front-end state, then the kernel and the cached row
+ * plan of msdr_chain_update_list_device for the same list run on them (msdr_chain_last_kernel: "msdr::fe::frontend_kernel
+ * (front end), then ...; channel list"). */
+int msdr_chain_update_adc_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const uint16_t *d_adc, int16_t *d_out,
+                                      uint32_t n_blocks, size_t stride);
+/* The same on host buffers of n rows, through the copy pipeline of msdr_chain_update_list. */
+int msdr_chain_update_adc_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, const uint16_t *adc, int16_t *out,
+                               uint32_t n_blocks, size_t stride);
 /* agc_idx outside [0, 25] is MSDR_ERR_ARGUMENT */
 int msdr_chain_get_frontend_state(msdr_chain *chain, uint32_t ch, msdr_frontend_state *out);
 int msdr_chain_set_frontend_state(msdr_chain *chain, uint32_t ch, const msdr_frontend_state *in);

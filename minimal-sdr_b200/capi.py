@@ -111,6 +111,9 @@ SYMBOLS = {
     "msdr_chain_update_adc": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
     "msdr_chain_update_adc_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
     "msdr_chain_update_adc_range_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_update_adc_list_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_update_adc_list": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32, C.c_size_t]),
+    "msdr_chain_frontend_preset_list": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint16]),
     "msdr_chain_get_frontend_state": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(FrontendState)]),
     "msdr_chain_set_frontend_state": (C.c_int, [C.c_void_p, C.c_uint32, C.POINTER(FrontendState)]),
     "msdr_amp_gain_multiplier": (C.c_int32, [C.c_float]),

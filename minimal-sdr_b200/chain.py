@@ -214,6 +214,11 @@ class ReceiveChain:
         ch0, nch = self._rng(ch0, nch)
         return self._ck(self._L.msdr_chain_frontend_preset(self.h, ch0, nch, int(first_reading)))
 
+    def frontend_preset_list(self, first_reading, channels):
+        """frontend_preset for the listed chain channels (any order) in one call."""
+        ch = np.ascontiguousarray(channels, np.uint32).ravel()
+        return self._ck(self._L.msdr_chain_frontend_preset_list(self.h, capi.ptr(ch), ch.size, int(first_reading)))
+
     def update_adc(self, adc, out=None):
         """adc: uint16 raw codes [n_channels, n_blocks*128] in HOST memory -> audio, as frontend.Frontend.update then update()."""
         adc = np.asarray(adc)
@@ -234,6 +239,27 @@ class ReceiveChain:
         """Only channels [ch0, ch0+nch); the buffers hold nch rows."""
         return self._ck(self._L.msdr_chain_update_adc_range_device(self.h, int(ch0), int(nch), C.c_void_p(int(d_adc)), C.c_void_p(int(d_out)),
                                                                    int(n_blocks), int(stride)))
+
+    def update_adc_list(self, channels, adc, out=None):
+        """Only the listed chain channels, in list order: row i of adc (uint16 raw codes [len(channels), n_blocks*128], HOST memory)
+        is channel channels[i]; returns the audio of those rows, same shape."""
+        ch = np.ascontiguousarray(channels, np.uint32).ravel()
+        adc = np.asarray(adc)
+        assert adc.dtype == np.uint16 and adc.ndim == 2 and adc.shape[0] == ch.size and adc.shape[1] % capi.BLOCK == 0
+        assert adc.strides[1] == 2 and adc.strides[0] % 2 == 0
+        if out is None:
+            out = np.empty(adc.shape, np.int16)
+        assert out.dtype == np.int16 and out.shape == adc.shape and out.strides[1] == 2
+        assert out.strides[0] == adc.strides[0], "in/out must share the row stride"
+        self._ck(self._L.msdr_chain_update_adc_list(self.h, capi.ptr(ch), ch.size, capi.ptr(adc), capi.ptr(out), adc.shape[1] // capi.BLOCK,
+                                                    adc.strides[0] // 2))
+        return out
+
+    def update_adc_list_device(self, channels, d_adc, d_out, n_blocks, stride):
+        """Only the listed chain channels (host array, any order); device buffers of len(channels) rows, row i = channels[i]."""
+        ch = np.ascontiguousarray(channels, np.uint32).ravel()
+        return self._ck(self._L.msdr_chain_update_adc_list_device(self.h, capi.ptr(ch), ch.size, C.c_void_p(int(d_adc)), C.c_void_p(int(d_out)),
+                                                                  int(n_blocks), int(stride)))
 
     def get_frontend_state(self, ch):
         st = capi.FrontendState()

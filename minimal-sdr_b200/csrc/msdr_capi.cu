@@ -129,7 +129,6 @@ struct msdr_chain {
   int fe_agc_on = 1;
   int16_t *d_fe_if = nullptr;        // [rows][stride] of the largest composed update so far
   size_t fe_if_samples = 0;
-  bool fe_composed = false;          // the last ADC update ran K4, then the int16 path
 
   // snapshots (msdr_chain_snapshot* / msdr_chain_restore*): host vectors their asynchronous uploads read from; `snap_ev` marks the
   // last such upload, and the next snapshot or restore waits for it before it writes them again
@@ -1004,7 +1003,9 @@ int check_list(msdr_chain *chain, const uint32_t *list, uint32_t n)
 // d_adc != NULL: the rows are raw ADC codes for the chain's front end.  Where the int16 input would run the row-block kernels and no
 // channel of the range is on the side lane (which gathers IF samples from `d_in`), the front end runs inside their converters; in
 // every other case K4 conditions the range into a scratch buffer first and the int16 path follows.  Both are bit-exact.
-// list != NULL (int16 input only, ch0 = 0): row r of d_in / d_out is chain channel list[r] instead of ch0 + r.
+// list != NULL (ch0 = 0): row r of d_in / d_adc / d_out is chain channel list[r] instead of ch0 + r.  ADC codes of a list always take
+// K4, which reads each row's front-end state through the plan's device copy of the list: a front end fused into the row-block list
+// kernels measured 0.96x of this composition (DESIGN.md §6).
 int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
                  size_t stride, const uint16_t *d_adc)
 {
@@ -1022,7 +1023,6 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
     return fail(chain, MSDR_ERR_ARGUMENT, "update_device: buffers must be 16-byte aligned and stride a multiple of 8 samples");
   if (chain->n_uninit) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update: some channels have no FIR bound (call msdr_fir_init_q15)");
   CK(cudaSetDevice(chain->device));
-  chain->fe_composed = false;
 
   int sms = 0;
   CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, chain->device));
@@ -1031,8 +1031,9 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
   int st = choose_kernel(chain, ch0, nch, list, NG, sms, ch);
   if (st != MSDR_OK) return st;
   const msdr_chain::TcPlan &pl = *ch.plan;
-  if (d_adc && ((ch.kernel != kV5 && ch.kernel != kV5l) || side_lane_in_range(chain, ch0, nch))) {
-    // K4 over the range into the scratch rows (same stride as `d_out`), then the int16 path reads them
+  const bool fe_composed = d_adc && (list || (ch.kernel != kV5 && ch.kernel != kV5l) || side_lane_in_range(chain, ch0, nch));
+  if (fe_composed) {
+    // K4 over the range or list into the scratch rows (same stride as `d_out`), then the int16 path reads them
     const size_t need = (size_t)nch * stride;
     if (need > chain->fe_if_samples) {
       CK(cudaStreamSynchronize(chain->stream));
@@ -1041,11 +1042,10 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
       CK(cudaMalloc(&chain->d_fe_if, need * sizeof(int16_t)));
       chain->fe_if_samples = need;
     }
-    CK(launch_frontend(d_adc, chain->d_fe_if, stride, nch, n_blocks, chain->d_fe + ch0, chain->fe_agc_max, chain->fe_agc_on, 0, chain->stream));
+    CK(launch_frontend(d_adc, chain->d_fe_if, stride, nch, n_blocks, chain->d_fe + ch0, chain->fe_agc_max, chain->fe_agc_on, 0, chain->stream, pl.d_list));
     chain->launches++;
     d_in = chain->d_fe_if;
     d_adc = nullptr;
-    chain->fe_composed = true;
   }
 
   ChainParams p{};
@@ -1115,6 +1115,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
                        (ch.kernel == kV4 ? kV4ShapeNames[ch.shape] : kNames[ch.kernel].form) + ")";
   if (p.fe) chain->last_kernel += "; front end fused into the converters";
   if (list) chain->last_kernel += "; channel list";
+  if (fe_composed) chain->last_kernel = "msdr::fe::frontend_kernel (front end), then " + chain->last_kernel;
   if ((st = syncam_lane_finish(chain, ch0, list != nullptr, d_out, stride, p.L)) != MSDR_OK) return st;
   if (chain->timed) {
     CK(cudaEventRecord(chain->ev1, chain->stream));
@@ -1204,8 +1205,10 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
       CK(cudaMemcpy2DAsync(din, Lc * 2, in + hoff, stride * 2, w, nc, cudaMemcpyHostToDevice, chain->copy_in));
       CK(cudaEventRecord(ev_h2d[slot], chain->copy_in));
       CK(cudaStreamWaitEvent(chain->stream, ev_h2d[slot], 0));
-      st = list ? msdr_chain_update_list_device(chain, list + c0, nc, din, dout, nb, Lc)
-           : adc ? msdr_chain_update_adc_range_device(chain, c0, nc, reinterpret_cast<const uint16_t *>(din), dout, nb, Lc)
+      const uint16_t *dadc = reinterpret_cast<const uint16_t *>(din);
+      st = list ? (adc ? msdr_chain_update_adc_list_device(chain, list + c0, nc, dadc, dout, nb, Lc)
+                       : msdr_chain_update_list_device(chain, list + c0, nc, din, dout, nb, Lc))
+           : adc ? msdr_chain_update_adc_range_device(chain, c0, nc, dadc, dout, nb, Lc)
                  : msdr_chain_update_range_device(chain, c0, nc, din, dout, nb, Lc);
       if (st != MSDR_OK) return st;
       CK(cudaEventRecord(ev_k[slot], chain->stream));
@@ -1273,14 +1276,33 @@ int msdr_chain_frontend_preset(msdr_chain *chain, uint32_t ch0, uint32_t nch, ui
   return MSDR_OK;
 }
 
+int msdr_chain_frontend_preset_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, uint16_t first_reading)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (!channels && n) return fail(chain, MSDR_ERR_ARGUMENT, "frontend_preset_list: NULL channel list");
+  for (uint32_t i = 0; i < n; ++i)
+    if (channels[i] >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, "frontend_preset_list: channel out of range");
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "frontend_preset_list: call msdr_chain_enable_frontend first");
+  if (n == 0) return MSDR_OK;
+  CK(cudaSetDevice(chain->device));
+  uint32_t *d_list = nullptr;
+  CK(cudaMalloc(&d_list, (size_t)n * 4));
+  // pageable source: staged before the call returns; the stream order puts the preset after every update already queued
+  cudaError_t e = cudaMemcpyAsync(d_list, channels, (size_t)n * 4, cudaMemcpyHostToDevice, chain->stream);
+  if (e == cudaSuccess) e = launch_frontend_preset(chain->d_fe, d_list, n, first_reading, chain->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(chain->stream);
+  cudaFree(d_list);
+  if (e != cudaSuccess) return cuda_fail(chain, e, "frontend_preset_list");
+  chain->launches++;
+  return MSDR_OK;
+}
+
 int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks,
                                        size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
-  const int st = update_range(chain, ch0, nch, nullptr, nullptr, d_out, n_blocks, stride, d_adc);
-  if (st == MSDR_OK && chain->fe_composed) chain->last_kernel = "msdr::fe::frontend_kernel (front end), then " + chain->last_kernel;
-  return st;
+  return update_range(chain, ch0, nch, nullptr, nullptr, d_out, n_blocks, stride, d_adc);
 }
 
 int msdr_chain_update_adc_device(msdr_chain *chain, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks, size_t stride)
@@ -1295,6 +1317,27 @@ int msdr_chain_update_adc(msdr_chain *chain, const uint16_t *adc, int16_t *out, 
   if (n_blocks == 0) return MSDR_OK;
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
   return host_pipeline(chain, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true);
+}
+
+int msdr_chain_update_adc_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const uint16_t *d_adc, int16_t *d_out,
+                                      uint32_t n_blocks, size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_adc_list: NULL channel list");
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc_list: call msdr_chain_enable_frontend first");
+  return update_range(chain, 0, n, channels, nullptr, d_out, n_blocks, stride, d_adc);
+}
+
+int msdr_chain_update_adc_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, const uint16_t *adc, int16_t *out, uint32_t n_blocks,
+                               size_t stride)
+{
+  if (!chain) return MSDR_ERR_ARGUMENT;
+  if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_adc_list: NULL channel list");
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc_list: call msdr_chain_enable_frontend first");
+  if (n == 0 || n_blocks == 0) return MSDR_OK;
+  const int st = check_list(chain, channels, n); // the whole list before the first chunk is queued
+  if (st != MSDR_OK) return st;
+  return host_pipeline(chain, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true, channels, n);
 }
 
 int msdr_chain_get_frontend_state(msdr_chain *chain, uint32_t ch, msdr_frontend_state *out)

@@ -28,16 +28,17 @@ struct Params {
   int16_t *out;        // [C][stride]
   size_t stride;
   uint32_t C, n_blocks;
-  State *state;        // [C]
+  State *state;        // [C], or indexed through map
   float agc_max;
   int agc_on;
+  const uint32_t *map; // kMap: row r's state is state[map[r]] (a chain's channel list); its codes and output stay row r
 };
 
 // Shared memory decides how many of these one-warp CTAs an SM holds: the blocks travel in pieces of kPart samples through a
 // ring of kNBuf buffers (64 samples, three deep: 13.8 KB per CTA, 16 CTAs per SM).
 // The warps of a CTA are independent (only __syncwarp): blockDim.x / 32 > 1 packs several channel groups onto one SM, which confines
 // the kernel to a few SMs so that a chain kernel that leaves SMs free can run beside it (msdr_frontend_set_option "sms").
-template <int kPart, int kNBuf>
+template <int kPart, int kNBuf, bool kMap>
 __global__ void frontend_kernel(const Params p)
 {
   constexpr int kPartPitchW = kPart / 2 + 4;     // 4 mod 32, conflict-free row-wise 128-bit access
@@ -50,8 +51,9 @@ __global__ void frontend_kernel(const Params p)
   if (g * kGroup >= p.C) return; // a warp past the last channel group (whole warps only: nothing below is block-wide)
   const bool active = row < p.C;
   const int nrows = min(kGroup, (int)(p.C - g * kGroup));
+  const uint32_t srow = kMap ? (active ? __ldg(p.map + row) : 0u) : row;
   State s;
-  if (active) s = p.state[row];
+  if (active) s = p.state[srow];
 
   // coalesced mapping for the copies: 4 rows of 128 bytes per warp instruction
   const int r0 = lane / CPR, c = lane % CPR;
@@ -104,25 +106,41 @@ __global__ void frontend_kernel(const Params p)
     __syncwarp(); // this buffer is the target of the copy issued at the top of the next iteration
   }
   s.hpf_x1 = x1; s.hpf_y1 = y1;
-  if (active) p.state[row] = s;
+  if (active) p.state[srow] = s;
+}
+
+// AudioInputAnalog::init (input_adc.cpp:59-63) for the states state[channels[i]], i < n: x1 = first reading << 14, y1 = 0
+__global__ void preset_kernel(State *state, const uint32_t *channels, uint32_t n, int32_t x1)
+{
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  State &s = state[channels[i]];
+  s.hpf_x1 = x1;
+  s.hpf_y1 = 0;
 }
 
 } // namespace fe
 
+cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t n, uint16_t first_reading, cudaStream_t s)
+{
+  fe::preset_kernel<<<(n + 255) / 256, 256, 0, s>>>(state, channels, n, (int32_t)((uint32_t)first_reading << 14));
+  return cudaGetLastError();
+}
+
 // piece length / ring depth measured at 65 536 and 262 144 channels (profiles/r01_frontend.txt): <64, 3> 1018 / 1189 Gsamples/s,
 // <128, 2> 914 / 1225, <64, 2> 1043 / 1153, <32, 4> 1040 / 1125, <32, 3> 1031 / 1027, <64, 4> 884 / 1195
 cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, uint32_t C, uint32_t n_blocks, fe::State *state, float agc_max,
-                            int agc_on, int sms, cudaStream_t s)
+                            int agc_on, int sms, cudaStream_t s, const uint32_t *map)
 {
   fe::Params p{};
   p.adc = adc; p.out = out; p.stride = stride; p.C = C; p.n_blocks = n_blocks; p.state = state;
-  p.agc_max = agc_max; p.agc_on = agc_on;
+  p.agc_max = agc_max; p.agc_on = agc_on; p.map = map;
   constexpr int kPart = 64, kNBuf = 3;
   const uint32_t groups = (C + kGroup - 1) / kGroup;
   const size_t warp_smem = (size_t)kNBuf * kGroup * (kPart / 2 + 4) * 4; // 13.8 KB per channel group
   uint32_t wpc = 1;
   if (sms > 0) wpc = std::min<uint32_t>(16, std::max<uint32_t>(1, (groups + (uint32_t)sms - 1) / (uint32_t)sms));
-  auto kern = fe::frontend_kernel<kPart, kNBuf>;
+  auto kern = map ? fe::frontend_kernel<kPart, kNBuf, true> : fe::frontend_kernel<kPart, kNBuf, false>;
   if (wpc * warp_smem > 48 * 1024) {
     const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(wpc * warp_smem));
     if (e != cudaSuccess) return e;

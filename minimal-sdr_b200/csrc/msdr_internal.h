@@ -65,10 +65,13 @@ cudaError_t launch_chain_v4(const ChainParams &p, cudaStream_t stream, int varia
 uint32_t chain_v4_span_samples();
 uint32_t chain_v4_unit_samples();
 bool chain_v4_config(uint32_t K, int smem_max, uint32_t rings[4]);
-// K4 (msdr_frontend.cu) over C rows: raw codes -> conditioned int16 IF samples; state = the first row's front-end state.
+// K4 (msdr_frontend.cu) over C rows: raw codes -> conditioned int16 IF samples; state = the first row's front-end state, or with
+// map != NULL the state array that row r indexes at map[r] (the rows' codes and outputs stay row r).
 // sms > 0 packs the channel groups into about that many CTAs.
+// launch_frontend_preset: hpf_x1 = first_reading << 14, hpf_y1 = 0 in state[channels[i]] for the n device-resident channels.
+cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t n, uint16_t first_reading, cudaStream_t s);
 cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, uint32_t C, uint32_t n_blocks, fe::State *state, float agc_max,
-                            int agc_on, int sms, cudaStream_t s);
+                            int agc_on, int sms, cudaStream_t s, const uint32_t *map = nullptr);
 // row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config (0 = does not fit);
 // p.fe != NULL selects the ADC-code instantiation (default biquad form only), p.chlist != NULL the channel-list one (the same)
 cudaError_t launch_chain_v5(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
