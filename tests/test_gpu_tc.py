@@ -45,9 +45,10 @@ def test_tc_reference_tables(msdr, orc, K, q31):
         assert_same(_tc(msdr, cI, cQ, kinds, x), _oracle(orc, cI, cQ, kinds, x, q31), f"tc mode {mode} q31 {q31}")
 
 
-@pytest.mark.parametrize("T", [4, 38, 86, 102, 256])
+@pytest.mark.parametrize("T", [4, 38, 62, 64, 86, 102, 128, 190, 192, 254, 256])
 def test_tc_wrap_and_saturation(msdr, orc, T):
-    """Random full-range taps (accumulator wraps, outputs saturate) on the adversarial inputs, every tap count class."""
+    """Random full-range taps (accumulator wraps, outputs saturate) on the adversarial inputs, every tap count class, both edges of
+    every FIR window (64, 96, 128, 160 and 192 words)."""
     rng = np.random.default_rng(T)
     ins = adversarial_inputs(128 * 4, rng)
     names = sorted(ins)
