@@ -201,7 +201,7 @@ int msdr_anr_create(msdr_anr **out, int device, uint32_t n_channels)
   if (e == cudaSuccess) e = cudaMemset(anr->d_w, 0, msdr::anr::kTaps * cp * 4);
   if (e == cudaSuccess) e = cudaMemset(anr->d_in_idx, 0, cp * 4);
   if (e == cudaSuccess) {
-    std::vector<float> l(cp, 120.0f), n(cp, 0.001f); // .ino:715,718
+    std::vector<float> l(cp, msdr::kAnrLidx0), n(cp, msdr::kAnrNgamma0);
     e = cudaMemcpy(anr->d_lidx, l.data(), cp * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMemcpy(anr->d_ngamma, n.data(), cp * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaDeviceSynchronize(); // legacy-stream copies / memsets vs this object's non-blocking stream

@@ -23,6 +23,32 @@ struct FirSet {
   uint32_t users = 0;
 };
 
+// The channels one call touches: the range [ch0, ch0 + n) or, `listed`, the chain channels list[0 .. n) (ch0 = 0).  Row r of the
+// call's buffers is chain channel chan(r).
+struct Rows {
+  uint32_t ch0 = 0, n = 0;
+  const uint32_t *list = nullptr;
+  bool listed = false;
+  uint32_t chan(uint32_t r) const { return listed ? list[r] : ch0 + r; }
+  Rows sub(uint32_t r0, uint32_t nr) const { return listed ? Rows{0, nr, list + r0, true} : Rows{ch0 + r0, nr, nullptr, false}; }
+};
+
+// A stored selection, the key of the caches built for one (the row plans, the side lane): a list is compared by its contents.
+struct RowsKey {
+  uint32_t ch0 = 0, n = 0;
+  bool listed = false;
+  std::vector<uint32_t> list;
+  bool matches(const Rows &r) const
+  {
+    return ch0 == r.ch0 && n == r.n && listed == r.listed && (!listed || std::equal(list.begin(), list.end(), r.list));
+  }
+  void assign(const Rows &r)
+  {
+    ch0 = r.ch0; n = r.n; listed = r.listed;
+    if (listed) list.assign(r.list, r.list + r.n); else list.clear();
+  }
+};
+
 // Split one (cI, cQ) table into the four polyphase sub-filters of the fs/4 mix + FIR pair; KP = roundup4(T/2 + 1).
 // With k' = d - (KP - T/2):  A[d] = cI[2k'], B[d] = cI[2k'+1], C[d] = cQ[2k'+1], D[d] = cQ[2(k'+1)], zero outside.
 // Derivation in DESIGN.md ("Polyphase form of the fs/4 mix + FIR"); tc_build_bmat turns them into the Toeplitz operands.
@@ -63,15 +89,17 @@ struct msdr_chain {
 
   // staging for host-buffer updates
   int16_t *d_in = nullptr, *d_out = nullptr;
-  size_t stage_samples = 0; // per buffer
-  int16_t *pin_in = nullptr, *pin_out = nullptr;
-  size_t pin_samples = 0;
+  size_t in_samples = 0, out_samples = 0;
+  // the device copy of the channel list of a setter call
+  uint32_t *d_sel = nullptr;
+  size_t sel_len = 0;
 
   // tensor-core FIR plan (chain kernel v4): rows sorted by tap table inside each wave of chains, see build_tc_plan()
   uint64_t meta_version = 1;  // bumped whenever a channel's table binding or a table's contents change
   struct TcPlan {
     uint64_t version = 0;
-    uint32_t ch0 = 0, nch = 0, sms = 0, W = 0, K = 0, rings[4] = {0, 0, 0, 0}, n_rb = 0, n_waves = 0;
+    RowsKey sel;
+    uint32_t sms = 0, W = 0, K = 0, rings[4] = {0, 0, 0, 0}, n_rb = 0, n_waves = 0;
     bool want_dual = false, want_v6 = false, dual = false;
     uint32_t ring_v5 = 0;  // msdr_chain_v5.cu: operand ring depth, 0 = the window does not fit that kernel
     uint32_t ring_v5l = 0; // msdr_chain_v5l.cu (half-tile hand-offs, for the 256-tap window)
@@ -81,14 +109,13 @@ struct msdr_chain {
     uint32_t *d_rowmap = nullptr, *d_wave_rb0 = nullptr;
     uint4 *d_rb = nullptr;
     uint8_t *d_bmat = nullptr;
-    std::vector<uint32_t> list;  // a channel-list plan: row r is chain channel list[r] (ch0 = 0, nch = list size); empty for a range
-    uint32_t *d_list = nullptr;  // the same on the device (ChainParams::chlist)
+    uint32_t *d_list = nullptr;  // a channel-list plan: sel.list on the device (ChainParams::chlist)
   };
   // one plan per updated channel range or channel list: msdr_chain_update cuts wide chains into channel chunks, each its own range
   static constexpr size_t kMaxPlans = 64;
   std::vector<TcPlan> plans;
   size_t plan_victim = 0;
-  // channel-list updates: list_seen[c] == list_stamp marks a channel already met in the list being checked
+  // channel lists: list_seen[c] == list_stamp marks a channel already met in the list being walked
   std::vector<uint32_t> list_seen;
   uint32_t list_stamp = 0;
   int *d_tile_cnt = nullptr;
@@ -109,15 +136,14 @@ struct msdr_chain {
     bool any_pll = false, any_anr = false;
     bool dirty = true;                 // modes / ANR switches changed: rebuild `channels`
     uint64_t epoch = 0;                // counts those changes
-    // the index vectors of the last update's range stay valid (host copies persist: their uploads are asynchronous)
+    // the index vectors of the last update's selection stay valid (host copies persist: their uploads are asynchronous)
     bool cached = false;
     uint64_t key_epoch = 0, key_version = 0;
-    uint32_t key_ch0 = 0, key_nch = 0;
-    std::vector<uint32_t> key_list;    // the channel list of the last update; empty for a range
+    RowsKey key;
     std::vector<uint32_t> chmap;
     std::vector<uint8_t> kind, amode;
     std::vector<uint32_t> channels;    // every chain channel that needs the lane, ascending
-    int16_t *d_raw = nullptr, *d_I = nullptr, *d_Q = nullptr, *d_If = nullptr, *d_Qf = nullptr, *d_taps = nullptr;
+    int16_t *d_raw = nullptr, *d_I = nullptr, *d_Q = nullptr, *d_If = nullptr, *d_Qf = nullptr;
     int32_t *d_defs = nullptr;
     size_t cap_rows = 0, cap_samples = 0;
   } pll;
@@ -130,13 +156,13 @@ struct msdr_chain {
   int16_t *d_fe_if = nullptr;        // [rows][stride] of the largest composed update so far
   size_t fe_if_samples = 0;
 
-  // snapshots (msdr_chain_snapshot* / msdr_chain_restore*): host vectors their asynchronous uploads read from; `snap_ev` marks the
-  // last such upload, and the next snapshot or restore waits for it before it writes them again
-  std::vector<uint8_t> snap_host;
-  std::vector<int16_t> snap_taps;
-  fe::State snap_fe0{};
-  cudaEvent_t snap_ev = nullptr;
-  bool snap_pending = false;
+  // host data that asynchronous uploads read from (snapshots, restores, mode and table ids, the initial front-end state); `stage_ev`
+  // marks the last such upload, and the next call that writes them waits for it first (staging_wait)
+  std::vector<uint8_t> snap_host, span_host;
+  std::vector<uint32_t> snap_rows; // a restore's channels grouped by table (kept: 4 bytes a channel, allocated once)
+  fe::State fe0{};
+  cudaEvent_t stage_ev = nullptr;
+  bool stage_pending = false;
 
   int variant = 0;
   uint32_t host_chunk_channels = 0, host_chunk_blocks = 0; // 0 = auto
@@ -180,81 +206,291 @@ int usage_resolve(msdr_chain *chain)
   return MSDR_OK;
 }
 
-int upload_set(msdr_chain *chain, uint32_t id)
+// ---- channel selections -----------------------------------------------------------------------------------------------------
+// a fresh mark for list_seen: no channel carries it yet
+uint32_t new_stamp(msdr_chain *chain)
+{
+  if (chain->list_seen.size() != chain->C) { chain->list_seen.assign(chain->C, 0u); chain->list_stamp = 0; }
+  if (++chain->list_stamp == 0) { std::fill(chain->list_seen.begin(), chain->list_seen.end(), 0u); chain->list_stamp = 1; }
+  return chain->list_stamp;
+}
+
+// A range must lie inside the chain; a list must not be NULL when n > 0 and must name chain channels only, and with `distinct` each
+// of them once (an update: two rows would race on one channel's state).
+int check_rows(msdr_chain *chain, const Rows &rows, bool distinct, const char *what)
+{
+  if (!rows.listed)
+    return range_ok(chain, rows.ch0, rows.n) ? MSDR_OK : fail(chain, MSDR_ERR_ARGUMENT, std::string(what) + ": bad channel range");
+  if (rows.n && !rows.list) return fail(chain, MSDR_ERR_ARGUMENT, std::string(what) + ": NULL channel list");
+  const uint32_t stamp = distinct ? new_stamp(chain) : 0u;
+  for (uint32_t r = 0; r < rows.n; ++r) {
+    const uint32_t c = rows.list[r];
+    if (c >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, std::string(what) + ": channel " + std::to_string(c) + " is not in the chain");
+    if (!distinct) continue;
+    if (chain->list_seen[c] == stamp) return fail(chain, MSDR_ERR_ARGUMENT, std::string(what) + ": channel " + std::to_string(c) + " is listed twice");
+    chain->list_seen[c] = stamp;
+  }
+  return MSDR_OK;
+}
+
+// f(c) for every channel of the selection, each once (a list may name a channel twice)
+template <class F> void each_channel(msdr_chain *chain, const Rows &rows, F f)
+{
+  if (!rows.listed) {
+    for (uint32_t c = rows.ch0; c < rows.ch0 + rows.n; ++c) f(c);
+    return;
+  }
+  const uint32_t stamp = new_stamp(chain);
+  for (uint32_t r = 0; r < rows.n; ++r)
+    if (chain->list_seen[rows.list[r]] != stamp) { chain->list_seen[rows.list[r]] = stamp; f(rows.list[r]); }
+}
+
+// p holds at least `need` elements (`need + spare` when it has to grow).  It only grows; the stream may still read the old buffer.
+template <class T> int grow(msdr_chain *chain, T *&p, size_t &len, size_t need, size_t spare = 0)
+{
+  if (need <= len) return MSDR_OK;
+  CK(cudaStreamSynchronize(chain->stream));
+  cudaFree(p);
+  p = nullptr;
+  len = 0;
+  CK(cudaMalloc(&p, (need + spare) * sizeof(T)));
+  len = need + spare;
+  return MSDR_OK;
+}
+
+// the selection's list in the chain's device list buffer; the copy reads the caller's list, so the call waits for the stream before
+// it returns
+int upload_list(msdr_chain *chain, const Rows &rows, const uint32_t **d_list)
+{
+  const int st = grow(chain, chain->d_sel, chain->sel_len, rows.n);
+  if (st != MSDR_OK) return st;
+  CK(cudaMemcpyAsync(chain->d_sel, rows.list, (size_t)rows.n * 4, cudaMemcpyHostToDevice, chain->stream));
+  *d_list = chain->d_sel;
+  return MSDR_OK;
+}
+
+// before the staged host data is written again, the uploads that read it must have run
+int staging_wait(msdr_chain *chain)
+{
+  if (!chain->stage_ev) CK(cudaEventCreateWithFlags(&chain->stage_ev, cudaEventDisableTiming));
+  if (chain->stage_pending) CK(cudaEventSynchronize(chain->stage_ev));
+  chain->stage_pending = false;
+  return MSDR_OK;
+}
+
+int staging_uploaded(msdr_chain *chain)
+{
+  CK(cudaEventRecord(chain->stage_ev, chain->stream));
+  chain->stage_pending = true;
+  return MSDR_OK;
+}
+
+// h[c] -> d[c] for the selection's channels: one copy of the span they cover, staged, so that nothing waits for it
+int upload_span(msdr_chain *chain, uint8_t *d, const std::vector<uint8_t> &h, const Rows &rows)
+{
+  uint32_t lo = rows.ch0, hi = rows.ch0 + rows.n - 1;
+  if (rows.listed) {
+    lo = 0xFFFFFFFFu; hi = 0;
+    for (uint32_t r = 0; r < rows.n; ++r) { lo = std::min(lo, rows.list[r]); hi = std::max(hi, rows.list[r]); }
+  }
+  const int st = staging_wait(chain);
+  if (st != MSDR_OK) return st;
+  chain->span_host.assign(h.begin() + lo, h.begin() + hi + 1);
+  CK(cudaMemcpyAsync(d + lo, chain->span_host.data(), hi - lo + 1, cudaMemcpyHostToDevice, chain->stream));
+  return staging_uploaded(chain);
+}
+
+// ---- the FIR table registry.  A binding is the state in h_set, sets[].users, n_uninit, d_set, d_set_taps and meta_version, and
+// only the functions below change it.  A slot is live while it has users.
+
+// The live table (T, cI, cQ) of `sets`, else the first slot without users (a new one below MSDR_MAX_FIR_SETS) set to it with no users
+// yet and *fresh set; -1 when every slot is live.  snap_restore runs it on a copy of the sets to see whether its tables fit.
+int find_or_add_table(std::vector<FirSet> &sets, uint32_t T, const int16_t *cI, const int16_t *cQ, bool *fresh)
+{
+  size_t slot = sets.size();
+  for (size_t i = 0; i < sets.size(); ++i) {
+    const FirSet &s = sets[i];
+    if (s.users && s.T == T && !memcmp(s.cI.data(), cI, T * 2) && !memcmp(s.cQ.data(), cQ, T * 2)) { *fresh = false; return (int)i; }
+    if (!s.users && slot == sets.size()) slot = i;
+  }
+  if (slot == sets.size()) {
+    if (slot >= MSDR_MAX_FIR_SETS) return -1;
+    sets.emplace_back();
+  }
+  FirSet &s = sets[slot];
+  s.T = T;
+  s.cI.assign(cI, cI + T);
+  s.cQ.assign(cQ, cQ + T);
+  s.users = 0;
+  *fresh = true;
+  return (int)slot;
+}
+
+// table `id`'s taps into d_set_taps, where the side lane's FIR launches read them; waits for the stream, as the host vectors may be
+// reassigned once this returns
+int upload_table(msdr_chain *chain, uint32_t id)
 {
   const FirSet &fs = chain->sets[id];
   int16_t *dst = chain->d_set_taps + (size_t)id * 2 * MSDR_MAX_TAPS;
   CK(cudaMemcpyAsync(dst, fs.cI.data(), fs.T * 2, cudaMemcpyHostToDevice, chain->stream));
   CK(cudaMemcpyAsync(dst + MSDR_MAX_TAPS, fs.cQ.data(), fs.T * 2, cudaMemcpyHostToDevice, chain->stream));
-  CK(cudaStreamSynchronize(chain->stream)); // the taps' vectors may be reassigned as soon as this returns
-  chain->meta_version++;
-  return MSDR_OK;
-}
-
-// find or create a coefficient set; returns id or negative status
-int intern_set(msdr_chain *chain, uint32_t T, const int16_t *cI, const int16_t *cQ)
-{
-  for (size_t i = 0; i < chain->sets.size(); ++i) {
-    const FirSet &s = chain->sets[i];
-    if (s.T == T && s.users > 0 && !memcmp(s.cI.data(), cI, T * 2) && !memcmp(s.cQ.data(), cQ, T * 2)) return (int)i;
-  }
-  size_t slot = chain->sets.size();
-  for (size_t i = 0; i < chain->sets.size(); ++i)
-    if (chain->sets[i].users == 0) { slot = i; break; }
-  if (slot == chain->sets.size()) {
-    if (slot >= MSDR_MAX_FIR_SETS) return fail(chain, MSDR_ERR_NOMEM, "more than MSDR_MAX_FIR_SETS distinct FIR tables in one chain");
-    chain->sets.emplace_back();
-  }
-  FirSet &s = chain->sets[slot];
-  s.T = T;
-  s.cI.assign(cI, cI + T);
-  s.cQ.assign(cQ, cQ + T);
-  s.users = 0;
-  int st = upload_set(chain, (uint32_t)slot);
-  if (st != MSDR_OK) return st;
-  return (int)slot;
-}
-
-int assign_set(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint32_t id)
-{
-  for (uint32_t c = ch0; c < ch0 + nch; ++c) {
-    const uint8_t old = chain->h_set[c];
-    if (old == 0xFF) chain->n_uninit--; else chain->sets[old].users--;
-    chain->h_set[c] = (uint8_t)id;
-  }
-  chain->sets[id].users += nch;
-  chain->meta_version++;
-  CK(cudaMemcpyAsync(chain->d_set + ch0, chain->h_set.data() + ch0, nch, cudaMemcpyHostToDevice, chain->stream));
   CK(cudaStreamSynchronize(chain->stream));
+  chain->meta_version++;
   return MSDR_OK;
+}
+
+// the id of table (T, cI, cQ), uploaded when it is new; a negative status when MSDR_MAX_FIR_SETS other tables are live
+int intern_table(msdr_chain *chain, uint32_t T, const int16_t *cI, const int16_t *cQ)
+{
+  bool fresh = false;
+  const int id = find_or_add_table(chain->sets, T, cI, cQ, &fresh);
+  if (id < 0) return fail(chain, MSDR_ERR_NOMEM, "more than MSDR_MAX_FIR_SETS distinct FIR tables in one chain");
+  const int st = fresh ? upload_table(chain, (uint32_t)id) : MSDR_OK;
+  return st != MSDR_OK ? st : id;
+}
+
+// every channel of the selection bound to table `id` (a channel listed twice is one user); upload_bindings brings d_set up to date
+void bind_rows(msdr_chain *chain, const Rows &rows, uint32_t id)
+{
+  uint32_t left[MSDR_MAX_FIR_SETS] = {0}, added = 0; // channels that leave each table, channels bound to `id` by this call
+  for (uint32_t r = 0; r < rows.n; ++r) {
+    uint8_t &s = chain->h_set[rows.chan(r)];
+    if (s == id) continue;
+    if (s != 0xFF) left[s]++;
+    s = (uint8_t)id;
+    added++;
+  }
+  chain->n_uninit -= added;
+  for (uint32_t sid = 0; sid < chain->sets.size(); ++sid) { chain->sets[sid].users -= left[sid]; chain->n_uninit += left[sid]; }
+  chain->sets[id].users += added;
+  chain->meta_version++;
+}
+
+int upload_bindings(msdr_chain *chain, const Rows &rows) { return upload_span(chain, chain->d_set, chain->h_set, rows); }
+
+// every channel of the selection unbound; d_set keeps their old ids, which no kernel reads while a channel is unbound
+void unbind_rows(msdr_chain *chain, const Rows &rows)
+{
+  uint32_t left[MSDR_MAX_FIR_SETS] = {0};
+  each_channel(chain, rows, [&](uint32_t c) {
+    uint8_t &s = chain->h_set[c];
+    if (s != 0xFF) { left[s]++; s = 0xFF; }
+  });
+  for (uint32_t sid = 0; sid < chain->sets.size(); ++sid) { chain->sets[sid].users -= left[sid]; chain->n_uninit += left[sid]; }
+  chain->meta_version++;
 }
 
 // Before channels are bound to a new table, a table used by none but them gives its slot back (its channels stay unbound until the
 // caller binds them): re-tuning a full chain (MSDR_MAX_FIR_SETS live tables) then does not fail for want of the slot it frees itself.
 // A table that keeps another user keeps its slot, and nothing changes when no table is freed, so a refused table leaves the chain as
-// it was.  Used by both FIR setters.  `each(f)` calls f(channel) for every channel to be re-bound, each channel once.
-template <class Each> void release_sole_sets(msdr_chain *chain, Each each)
+// it was.
+void release_sole_sets(msdr_chain *chain, const Rows &rows)
 {
   uint32_t n[MSDR_MAX_FIR_SETS] = {0};
-  each([&](uint32_t c) { if (chain->h_set[c] != 0xFF) n[chain->h_set[c]]++; });
+  each_channel(chain, rows, [&](uint32_t c) { if (chain->h_set[c] != 0xFF) n[chain->h_set[c]]++; });
   auto sole = [&](uint32_t sid) { return n[sid] && n[sid] == chain->sets[sid].users; };
-  each([&](uint32_t c) {
+  each_channel(chain, rows, [&](uint32_t c) {
     if (chain->h_set[c] != 0xFF && sole(chain->h_set[c])) { chain->h_set[c] = 0xFF; chain->n_uninit++; }
   });
   for (uint32_t sid = 0; sid < chain->sets.size(); ++sid)
     if (sole(sid)) chain->sets[sid].users = 0;
 }
 
-int ensure_stage(msdr_chain *chain, size_t samples)
+// ---- uploads from the chain's own host data, and the initial states ---------------------------------------------------------
+// `count` copies of the element at host address `elem` (which outlives the copies) from d on: one upload, then doubling copies
+int replicate(msdr_chain *chain, void *d, size_t elem_bytes, size_t count, const void *elem)
 {
-  if (chain->stage_samples >= samples) return MSDR_OK;
-  if (chain->d_in) cudaFree(chain->d_in);
-  if (chain->d_out) cudaFree(chain->d_out);
-  chain->d_in = chain->d_out = nullptr;
-  chain->stage_samples = 0;
-  CK(cudaMalloc(&chain->d_in, samples * sizeof(int16_t)));
-  CK(cudaMalloc(&chain->d_out, samples * sizeof(int16_t)));
-  chain->stage_samples = samples;
+  if (!count) return MSDR_OK;
+  uint8_t *p = static_cast<uint8_t *>(d);
+  CK(cudaMemcpyAsync(p, elem, elem_bytes, cudaMemcpyHostToDevice, chain->stream));
+  for (size_t done = 1; done < count; done *= 2)
+    CK(cudaMemcpyAsync(p + done * elem_bytes, p, std::min(done, count - done) * elem_bytes, cudaMemcpyDeviceToDevice, chain->stream));
+  return MSDR_OK;
+}
+
+// initial LMS state for channels [ch0, ch0+n)
+int anr_initial(msdr_chain *chain, uint32_t ch0, uint32_t n)
+{
+  const size_t cp = (size_t)chain->Cpad * 4, w = (size_t)n * 4;
+  CK(cudaMemset2DAsync(chain->d_anr_d + ch0, cp, 0, w, 512, chain->stream));
+  CK(cudaMemset2DAsync(chain->d_anr_w + ch0, cp, 0, w, 64, chain->stream));
+  CK(cudaMemsetAsync(chain->d_anr_idx + ch0, 0, w, chain->stream));
+  int st = replicate(chain, chain->d_anr_lidx + ch0, 4, n, &kAnrLidx0);
+  if (st == MSDR_OK) st = replicate(chain, chain->d_anr_ngamma + ch0, 4, n, &kAnrNgamma0);
+  return st;
+}
+
+// the LMS state (512-entry delay line + 64 weights per channel) on first use, every channel at the initial state
+int anr_alloc(msdr_chain *chain)
+{
+  if (chain->d_anr_d) return MSDR_OK;
+  const size_t cp = (size_t)chain->Cpad * 4;
+  CK(cudaMalloc(&chain->d_anr_d, 512 * cp)); CK(cudaMalloc(&chain->d_anr_w, 64 * cp));
+  CK(cudaMalloc(&chain->d_anr_lidx, cp)); CK(cudaMalloc(&chain->d_anr_ngamma, cp)); CK(cudaMalloc(&chain->d_anr_idx, cp));
+  return anr_initial(chain, 0, chain->Cpad);
+}
+
+void free_tc_plan(msdr_chain::TcPlan &pl)
+{
+  cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32); cudaFree(pl.d_list);
+  pl = msdr_chain::TcPlan{};
+}
+
+// ---- the setters that take a range or a list ----------------------------------------------------------------------------------
+int set_mode(msdr_chain *chain, const Rows &rows, int mode)
+{
+  int st = check_rows(chain, rows, false, "set_mode");
+  if (st != MSDR_OK) return st;
+  if (mode < 0 || mode > 4) return fail(chain, MSDR_ERR_ARGUMENT, "set_mode: bad mode");
+  if (rows.n == 0) return MSDR_OK;
+  CK(cudaSetDevice(chain->device));
+  for (uint32_t r = 0; r < rows.n; ++r) chain->h_mode[rows.chan(r)] = (uint8_t)mode;
+  chain->pll.dirty = true; chain->pll.epoch++;
+  if (rows.listed) return upload_span(chain, chain->d_mode, chain->h_mode, rows);
+  CK(cudaMemsetAsync(chain->d_mode + rows.ch0, mode, rows.n, chain->stream));
+  return MSDR_OK;
+}
+
+// arm_fir_init_q15 on the selection: bind the table, zero the delay lines (init_FIR's memset, .ino:902-903)
+int fir_init(msdr_chain *chain, const Rows &rows, uint16_t numTaps, const int16_t *cI, const int16_t *cQ)
+{
+  if (numTaps & 1u) return fail(chain, MSDR_ERR_ARGUMENT, "arm_fir_init_q15: numTaps must be even (arm_fir_init_q15.c:93-96)");
+  if (!cI || !cQ) return fail(chain, MSDR_ERR_ARGUMENT, "fir_init: NULL coefficients");
+  int st = check_rows(chain, rows, false, "fir_init");
+  if (st != MSDR_OK) return st;
+  if (numTaps < 4 || numTaps > chain->max_taps) return fail(chain, MSDR_ERR_LENGTH, "fir_init: numTaps outside [4, max_taps of this chain]");
+  if (rows.n == 0) return MSDR_OK;
+  CK(cudaSetDevice(chain->device));
+  release_sole_sets(chain, rows);
+  const int id = intern_table(chain, numTaps, cI, cQ);
+  if (id < 0) return id;
+  bind_rows(chain, rows, (uint32_t)id);
+  if ((st = upload_bindings(chain, rows)) != MSDR_OK) return st;
+  if (!rows.listed) {
+    CK(cudaMemsetAsync(chain->d_hist + (size_t)rows.ch0 * chain->H, 0, (size_t)rows.n * chain->H * sizeof(int16_t), chain->stream));
+    return MSDR_OK;
+  }
+  const uint32_t *d_list = nullptr;
+  if ((st = upload_list(chain, rows, &d_list)) != MSDR_OK) return st;
+  CK(launch_zero_hist_rows(chain->d_hist, chain->H, d_list, rows.n, chain->stream));
+  chain->launches++;
+  CK(cudaStreamSynchronize(chain->stream));
+  return MSDR_OK;
+}
+
+// AudioInputAnalog::init (input_adc.cpp:59-63) on the selection: x1 = first reading << 14, y1 = 0
+int frontend_preset(msdr_chain *chain, const Rows &rows, uint16_t first_reading)
+{
+  int st = check_rows(chain, rows, false, "frontend_preset");
+  if (st != MSDR_OK) return st;
+  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "frontend_preset: call msdr_chain_enable_frontend first");
+  if (rows.n == 0) return MSDR_OK;
+  CK(cudaSetDevice(chain->device));
+  const uint32_t *d_list = nullptr;
+  if (rows.listed && (st = upload_list(chain, rows, &d_list)) != MSDR_OK) return st;
+  CK(launch_frontend_preset(chain->d_fe, d_list, rows.ch0, rows.n, first_reading, chain->stream));
+  chain->launches++;
+  if (rows.listed) CK(cudaStreamSynchronize(chain->stream));
   return MSDR_OK;
 }
 
@@ -329,21 +565,19 @@ void msdr_chain_destroy(msdr_chain *chain)
   cudaSetDevice(chain->device);
   if (chain->stream) cudaStreamSynchronize(chain->stream);
   cudaFree(chain->d_mode); cudaFree(chain->d_set); cudaFree(chain->d_hist); cudaFree(chain->d_bq);
-  for (auto &pl : chain->plans) { cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32); }
+  for (auto &pl : chain->plans) free_tc_plan(pl);
   cudaFree(chain->d_tile_cnt); cudaFree(chain->d_pll);
   cudaFree(chain->d_anr_d); cudaFree(chain->d_anr_w); cudaFree(chain->d_anr_lidx); cudaFree(chain->d_anr_ngamma); cudaFree(chain->d_anr_idx);
   cudaFree(chain->pll.d_kind); cudaFree(chain->pll.d_anr_mode);
   cudaFree(chain->pll.d_rows); cudaFree(chain->pll.d_chmap); cudaFree(chain->pll.d_raw); cudaFree(chain->pll.d_I); cudaFree(chain->pll.d_Q);
-  cudaFree(chain->pll.d_If); cudaFree(chain->pll.d_Qf); cudaFree(chain->pll.d_taps); cudaFree(chain->pll.d_defs);
+  cudaFree(chain->pll.d_If); cudaFree(chain->pll.d_Qf); cudaFree(chain->pll.d_defs);
   cudaFree(chain->d_set_taps); cudaFree(chain->d_ctrl);
-  cudaFree(chain->d_in); cudaFree(chain->d_out);
+  cudaFree(chain->d_in); cudaFree(chain->d_out); cudaFree(chain->d_sel);
   cudaFree(chain->d_fe); cudaFree(chain->d_fe_if);
-  if (chain->pin_in) cudaFreeHost(chain->pin_in);
-  if (chain->pin_out) cudaFreeHost(chain->pin_out);
   for (cudaEvent_t ev : chain->pipe_ev) cudaEventDestroy(ev);
   if (chain->ev0) cudaEventDestroy(chain->ev0);
   if (chain->ev1) cudaEventDestroy(chain->ev1);
-  if (chain->snap_ev) cudaEventDestroy(chain->snap_ev);
+  if (chain->stage_ev) cudaEventDestroy(chain->stage_ev);
   if (chain->own_stream) cudaStreamDestroy(chain->own_stream);
   if (chain->copy_in) cudaStreamDestroy(chain->copy_in);
   if (chain->copy_out) cudaStreamDestroy(chain->copy_out);
@@ -381,14 +615,7 @@ int msdr_chain_fir_taps(const msdr_chain *chain, uint32_t ch)
 
 int msdr_chain_set_mode(msdr_chain *chain, uint32_t ch0, uint32_t nch, int mode)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if (!range_ok(chain, ch0, nch) || mode < 0 || mode > 4) return fail(chain, MSDR_ERR_ARGUMENT, "set_mode: bad channel range or mode");
-  if (nch == 0) return MSDR_OK;
-  CK(cudaSetDevice(chain->device));
-  std::fill(chain->h_mode.begin() + ch0, chain->h_mode.begin() + ch0 + nch, (uint8_t)mode);
-  chain->pll.dirty = true; chain->pll.epoch++;
-  CK(cudaMemsetAsync(chain->d_mode + ch0, mode, nch, chain->stream));
-  return MSDR_OK;
+  return chain ? set_mode(chain, Rows{ch0, nch}, mode) : MSDR_ERR_ARGUMENT;
 }
 
 int msdr_chain_set_anr(msdr_chain *chain, uint32_t ch0, uint32_t nch, int anr_on)
@@ -398,16 +625,9 @@ int msdr_chain_set_anr(msdr_chain *chain, uint32_t ch0, uint32_t nch, int anr_on
   if (nch == 0) return MSDR_OK;
   CK(cudaSetDevice(chain->device));
   if (chain->h_anr.empty()) chain->h_anr.assign(chain->C, 0);
-  if (anr_on && !chain->d_anr_d) { // LMS state: 512-entry delay line + 64 weights per channel, allocated on first use
-    const size_t cp = chain->Cpad;
-    CK(cudaStreamSynchronize(chain->stream));
-    CK(cudaMalloc(&chain->d_anr_d, 512 * cp * 4)); CK(cudaMalloc(&chain->d_anr_w, 64 * cp * 4));
-    CK(cudaMalloc(&chain->d_anr_lidx, cp * 4)); CK(cudaMalloc(&chain->d_anr_ngamma, cp * 4)); CK(cudaMalloc(&chain->d_anr_idx, cp * 4));
-    CK(cudaMemset(chain->d_anr_d, 0, 512 * cp * 4)); CK(cudaMemset(chain->d_anr_w, 0, 64 * cp * 4)); CK(cudaMemset(chain->d_anr_idx, 0, cp * 4));
-    std::vector<float> l(cp, 120.0f), g(cp, 0.001f); // Minimal-SDR.ino:715,718
-    CK(cudaMemcpy(chain->d_anr_lidx, l.data(), cp * 4, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(chain->d_anr_ngamma, g.data(), cp * 4, cudaMemcpyHostToDevice));
-    CK(cudaDeviceSynchronize()); // legacy-stream copies / memsets vs the chain's non-blocking stream
+  if (anr_on) {
+    const int st = anr_alloc(chain);
+    if (st != MSDR_OK) return st;
   }
   for (uint32_t c = ch0; c < ch0 + nch; ++c) {
     chain->n_anr += (anr_on != 0) - (chain->h_anr[c] != 0);
@@ -437,96 +657,32 @@ int msdr_chain_set_anr_state(msdr_chain *chain, uint32_t ch, const msdr_anr_stat
   if (!chain || !in || ch >= chain->C || in->in_idx < 0 || in->in_idx >= 512) return MSDR_ERR_ARGUMENT;
   if (!chain->d_anr_d) return fail(chain, MSDR_ERR_NOT_INITIALISED, "set_anr_state: switch ANR on (msdr_chain_set_anr) first");
   CK(cudaSetDevice(chain->device));
-  CK(cudaStreamSynchronize(chain->stream));
   const size_t pitch = (size_t)chain->Cpad * 4;
-  CK(cudaMemcpy2D(chain->d_anr_d + ch, pitch, in->d, 4, 4, 512, cudaMemcpyHostToDevice));
-  CK(cudaMemcpy2D(chain->d_anr_w + ch, pitch, in->w, 4, 4, 64, cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(chain->d_anr_lidx + ch, &in->lidx, 4, cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(chain->d_anr_ngamma + ch, &in->ngamma, 4, cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(chain->d_anr_idx + ch, &in->in_idx, 4, cudaMemcpyHostToDevice));
-  CK(cudaDeviceSynchronize()); // legacy-stream copies vs the chain's non-blocking stream
+  cudaStream_t s = chain->stream;
+  CK(cudaMemcpy2DAsync(chain->d_anr_d + ch, pitch, in->d, 4, 4, 512, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpy2DAsync(chain->d_anr_w + ch, pitch, in->w, 4, 4, 64, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(chain->d_anr_lidx + ch, &in->lidx, 4, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(chain->d_anr_ngamma + ch, &in->ngamma, 4, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(chain->d_anr_idx + ch, &in->in_idx, 4, cudaMemcpyHostToDevice, s));
+  CK(cudaStreamSynchronize(s)); // the caller may free `in` on return
   return MSDR_OK;
 }
 
 int msdr_fir_init_q15(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint16_t numTaps, const int16_t *cI, const int16_t *cQ)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if (numTaps & 1u) return fail(chain, MSDR_ERR_ARGUMENT, "arm_fir_init_q15: numTaps must be even (arm_fir_init_q15.c:93-96)");
-  if (!cI || !cQ || !range_ok(chain, ch0, nch)) return fail(chain, MSDR_ERR_ARGUMENT, "fir_init: bad arguments");
-  if (numTaps < 4 || numTaps > chain->max_taps) return fail(chain, MSDR_ERR_LENGTH, "fir_init: numTaps outside [4, max_taps of this chain]");
-  if (nch == 0) return MSDR_OK;
-  CK(cudaSetDevice(chain->device));
-  release_sole_sets(chain, [&](auto &&f) { for (uint32_t c = ch0; c < ch0 + nch; ++c) f(c); });
-  const int id = intern_set(chain, numTaps, cI, cQ);
-  if (id < 0) return id;
-  int st = assign_set(chain, ch0, nch, (uint32_t)id);
-  if (st != MSDR_OK) return st;
-  CK(cudaMemsetAsync(chain->d_hist + (size_t)ch0 * chain->H, 0, (size_t)nch * chain->H * sizeof(int16_t), chain->stream)); // init_FIR memset, .ino:902-903
-  return MSDR_OK;
+  return chain ? fir_init(chain, Rows{ch0, nch}, numTaps, cI, cQ) : MSDR_ERR_ARGUMENT;
 }
 
 // ---- the same two setters for a LIST of channels: a batch of receivers whose modes interleave (mode = f(channel mod 4) in the
 // benchmark layouts) is configured with one call per mode instead of one per channel
 int msdr_chain_set_mode_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, int mode)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if ((!channels && n) || mode < 0 || mode > 4) return fail(chain, MSDR_ERR_ARGUMENT, "set_mode_list: bad arguments");
-  if (n == 0) return MSDR_OK;
-  uint32_t lo = 0xFFFFFFFFu, hi = 0;
-  for (uint32_t i = 0; i < n; ++i) {
-    if (channels[i] >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, "set_mode_list: channel out of range");
-    lo = std::min(lo, channels[i]); hi = std::max(hi, channels[i]);
-  }
-  CK(cudaSetDevice(chain->device));
-  for (uint32_t i = 0; i < n; ++i) chain->h_mode[channels[i]] = (uint8_t)mode;
-  chain->pll.dirty = true; chain->pll.epoch++;
-  CK(cudaMemcpyAsync(chain->d_mode + lo, chain->h_mode.data() + lo, hi - lo + 1, cudaMemcpyHostToDevice, chain->stream));
-  CK(cudaStreamSynchronize(chain->stream));
-  return MSDR_OK;
+  return chain ? set_mode(chain, Rows{0, n, channels, true}, mode) : MSDR_ERR_ARGUMENT;
 }
 
 int msdr_fir_init_q15_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, uint16_t numTaps, const int16_t *cI, const int16_t *cQ)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if (numTaps & 1u) return fail(chain, MSDR_ERR_ARGUMENT, "arm_fir_init_q15: numTaps must be even (arm_fir_init_q15.c:93-96)");
-  if (!cI || !cQ || (!channels && n)) return fail(chain, MSDR_ERR_ARGUMENT, "fir_init_list: bad arguments");
-  if (numTaps < 4 || numTaps > chain->max_taps) return fail(chain, MSDR_ERR_LENGTH, "fir_init: numTaps outside [4, max_taps of this chain]");
-  if (n == 0) return MSDR_OK;
-  uint32_t lo = 0xFFFFFFFFu, hi = 0;
-  for (uint32_t i = 0; i < n; ++i) {
-    if (channels[i] >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, "fir_init_list: channel out of range");
-    lo = std::min(lo, channels[i]); hi = std::max(hi, channels[i]);
-  }
-  CK(cudaSetDevice(chain->device));
-  {
-    std::vector<uint32_t> uniq(channels, channels + n); // a channel listed twice is one user
-    std::sort(uniq.begin(), uniq.end());
-    uniq.erase(std::unique(uniq.begin(), uniq.end()), uniq.end());
-    release_sole_sets(chain, [&](auto &&f) { for (uint32_t c : uniq) f(c); });
-  }
-  const int id = intern_set(chain, numTaps, cI, cQ);
-  if (id < 0) return id;
-  uint32_t added = 0;
-  for (uint32_t i = 0; i < n; ++i) {
-    const uint32_t c = channels[i];
-    const uint8_t old = chain->h_set[c];
-    if (old == (uint8_t)id) continue; // listed twice, or already bound to this table
-    if (old == 0xFF) chain->n_uninit--; else chain->sets[old].users--;
-    chain->h_set[c] = (uint8_t)id;
-    ++added;
-  }
-  chain->sets[id].users += added;
-  chain->meta_version++;
-  uint32_t *d_list = nullptr;
-  CK(cudaMemcpyAsync(chain->d_set + lo, chain->h_set.data() + lo, hi - lo + 1, cudaMemcpyHostToDevice, chain->stream));
-  CK(cudaMalloc(&d_list, (size_t)n * 4));
-  cudaError_t e = cudaMemcpyAsync(d_list, channels, (size_t)n * 4, cudaMemcpyHostToDevice, chain->stream);
-  if (e == cudaSuccess) e = launch_zero_hist_rows(chain->d_hist, chain->H, d_list, n, chain->stream); // init_FIR memset, .ino:902-903
-  if (e == cudaSuccess) e = cudaStreamSynchronize(chain->stream);
-  cudaFree(d_list);
-  if (e != cudaSuccess) return cuda_fail(chain, e, "fir_init_list");
-  chain->launches++;
-  return MSDR_OK;
+  return chain ? fir_init(chain, Rows{0, n, channels, true}, numTaps, cI, cQ) : MSDR_ERR_ARGUMENT;
 }
 
 int msdr_fir_set_coefficients(msdr_chain *chain, uint32_t ch0, uint32_t nch, const int16_t *cI, const int16_t *cQ)
@@ -542,11 +698,12 @@ int msdr_fir_set_coefficients(msdr_chain *chain, uint32_t ch0, uint32_t nch, con
   if (chain->sets[cur].users == nch) { // every user is in the range: rewrite in place, like the sketch's single table
     chain->sets[cur].cI.assign(cI, cI + T);
     chain->sets[cur].cQ.assign(cQ, cQ + T);
-    return upload_set(chain, cur);
+    return upload_table(chain, cur);
   }
-  const int id = intern_set(chain, T, cI, cQ);
+  const int id = intern_table(chain, T, cI, cQ);
   if (id < 0) return id;
-  return assign_set(chain, ch0, nch, (uint32_t)id); // delay lines untouched
+  bind_rows(chain, Rows{ch0, nch}, (uint32_t)id);
+  return upload_bindings(chain, Rows{ch0, nch}); // delay lines untouched
 }
 
 int msdr_biquad_set_coefficients(msdr_chain *chain, int object, uint32_t ch0, uint32_t nch, uint32_t stage, const int32_t *coef)
@@ -563,12 +720,6 @@ int msdr_biquad_set_coefficients(msdr_chain *chain, int object, uint32_t ch0, ui
 
 namespace {
 
-void free_tc_plan(msdr_chain::TcPlan &pl)
-{
-  cudaFree(pl.d_rowmap); cudaFree(pl.d_wave_rb0); cudaFree(pl.d_rb); cudaFree(pl.d_bmat); cudaFree(pl.d_rowmap32); cudaFree(pl.d_rb32); cudaFree(pl.d_list);
-  pl = msdr_chain::TcPlan{};
-}
-
 // Row plan of the tensor-core chain kernel for the channel range [ch0, ch0 + nch).  All 128 rows of a GEMM tile share the
 // B operand, i.e. one tap table, and a chain wave (W groups of 32 channels, one per CTA) must get its FIR input first; so
 // inside each wave the rows are sorted by table and cut into blocks of 128 (the last block of a table is padded).
@@ -578,20 +729,17 @@ void free_tc_plan(msdr_chain::TcPlan &pl)
 // window leaves room for the second set of chain slots (rings[3]), which is known before any row is sorted — so the wave width
 // is chosen once and an unchanged configuration always hits the cache (256 taps beyond 148 groups used to rebuild twice per update).
 // want_v6: also the group-block plan of the time-folded kernel (msdr_chain_v6.cu), if the window fits that kernel.
-// list != NULL: the rows are the chain channels list[0 .. nch) (ch0 = 0) instead of the range; the plan keeps the list, and a lookup
-// compares its contents.
-int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, uint32_t sms, bool want_dual, bool want_v6,
-                  const msdr_chain::TcPlan **out)
+// A channel list's plan keeps the list, also on the device (ChainParams::chlist).
+int build_tc_plan(msdr_chain *chain, const Rows &sel, uint32_t sms, bool want_dual, bool want_v6, const msdr_chain::TcPlan **out)
 {
   for (const auto &c : chain->plans)
-    if (c.version == chain->meta_version && c.ch0 == ch0 && c.nch == nch && c.sms == sms && c.want_dual == want_dual && c.want_v6 == want_v6 &&
-        c.list.empty() == !list && (!list || std::equal(c.list.begin(), c.list.end(), list))) {
+    if (c.version == chain->meta_version && c.sel.matches(sel) && c.sms == sms && c.want_dual == want_dual && c.want_v6 == want_v6) {
       *out = &c;
       return MSDR_OK;
     }
-  auto chan = [&](uint32_t r) { return list ? list[r] : ch0 + r; }; // chain channel of row r
+  const uint32_t nch = sel.n;
   uint32_t kp_max = 0;
-  for (uint32_t r = 0; r < nch; ++r) kp_max = std::max(kp_max, kp_of_taps(chain->sets[chain->h_set[chan(r)]].T));
+  for (uint32_t r = 0; r < nch; ++r) kp_max = std::max(kp_max, kp_of_taps(chain->sets[chain->h_set[sel.chan(r)]].T));
   const uint32_t K = tc_window_words_kp(kp_max);
   int smem_max = 0;
   CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, chain->device));
@@ -610,7 +758,7 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t 
   free_tc_plan(pl);
   *out = &pl;
   chain->plan_builds++;
-  pl.version = chain->meta_version; pl.ch0 = ch0; pl.nch = nch; pl.sms = sms; pl.want_dual = want_dual; pl.want_v6 = want_v6;
+  pl.version = chain->meta_version; pl.sel.assign(sel); pl.sms = sms; pl.want_dual = want_dual; pl.want_v6 = want_v6;
   std::copy(rings, rings + 4, pl.rings);
   pl.K = K;
   pl.ring_v5 = chain_v5_config(K, smem_max);
@@ -627,7 +775,7 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t 
   for (uint32_t g0 = 0; g0 < NG; g0 += W) {
     const uint32_t g1 = std::min(NG, g0 + W);
     for (auto &b : bucket) b.clear();
-    for (uint32_t r = g0 * kGroup; r < std::min(nch, g1 * (uint32_t)kGroup); ++r) bucket[chain->h_set[chan(r)]].push_back(r);
+    for (uint32_t r = g0 * kGroup; r < std::min(nch, g1 * (uint32_t)kGroup); ++r) bucket[chain->h_set[sel.chan(r)]].push_back(r);
     for (uint32_t sid = 0; sid < n_sets; ++sid) {
       const std::vector<uint32_t> &rows = bucket[sid];
       for (size_t i0 = 0; i0 < rows.size(); i0 += M) {
@@ -650,13 +798,13 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t 
     struct Half { uint32_t sid; size_t i0; bool costly; };
     std::vector<Half> costly, cheap;
     for (auto &b : bucket) b.clear();
-    for (uint32_t r = 0; r < nch; ++r) bucket[chain->h_set[chan(r)]].push_back(r);
+    for (uint32_t r = 0; r < nch; ++r) bucket[chain->h_set[sel.chan(r)]].push_back(r);
     for (uint32_t sid = 0; sid < n_sets; ++sid) {
       const std::vector<uint32_t> &rows = bucket[sid];
       for (size_t i0 = 0; i0 < rows.size(); i0 += HR) {
         bool env = false;
         for (size_t i = i0; i < std::min(rows.size(), i0 + HR); ++i) {
-          const int md = chain->h_mode[chan(rows[i])];
+          const int md = chain->h_mode[sel.chan(rows[i])];
           env |= !(md == MSDR_MODE_LSB || md == MSDR_MODE_USB);
         }
         (env ? costly : cheap).push_back(Half{sid, i0, env});
@@ -705,10 +853,9 @@ int build_tc_plan(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t 
     CK(cudaMemcpyAsync(pl.d_rowmap32, rowmap32.data(), rowmap32.size() * 4, cudaMemcpyHostToDevice, chain->stream));
     CK(cudaMemcpyAsync(pl.d_rb32, rbs32.data(), rbs32.size() * sizeof(uint4), cudaMemcpyHostToDevice, chain->stream));
   }
-  if (list) {
-    pl.list.assign(list, list + nch);
+  if (sel.listed) {
     CK(cudaMalloc(&pl.d_list, (size_t)nch * 4));
-    CK(cudaMemcpyAsync(pl.d_list, pl.list.data(), (size_t)nch * 4, cudaMemcpyHostToDevice, chain->stream));
+    CK(cudaMemcpyAsync(pl.d_list, pl.sel.list.data(), (size_t)nch * 4, cudaMemcpyHostToDevice, chain->stream));
   }
   // On the chain's stream, NOT cudaMemcpy: a synchronous copy from pageable memory returns once the data is staged, its DMA runs in
   // the legacy stream, and the chain's stream is non-blocking - a kernel launched right after could read the plan before it had
@@ -751,33 +898,30 @@ bool side_lane_in_range(msdr_chain *chain, uint32_t ch0, uint32_t nch)
   return it != ch.end() && *it < ch0 + nch;
 }
 
-// list != NULL: the update's rows are the chain channels list[0 .. nch) (ch0 = 0)
-int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, const int16_t *d_in, size_t stride, uint32_t L)
+int syncam_lane_prepare(msdr_chain *chain, const Rows &sel, const int16_t *d_in, size_t stride, uint32_t L)
 {
   msdr_chain::PllLane &ln = chain->pll;
   const bool pll_build = !(chain->flags & MSDR_FLAG_AM_Q31); // Teensy 3.2 arithmetic: SYNCAM is the q31 envelope (.ino:618-620)
-  // The lane's index vectors depend on the range or list, the modes / ANR switches (epoch) and the table bindings (meta_version) only: an
+  // The lane's index vectors depend on the selection, the modes / ANR switches (epoch) and the table bindings (meta_version) only: an
   // update that repeats the last one's configuration re-uses them on the device, and nothing in this function waits for the stream.
-  const bool hit = ln.cached && ln.key_epoch == ln.epoch && ln.key_version == chain->meta_version && ln.key_ch0 == ch0 && ln.key_nch == nch &&
-                   ln.key_list.empty() == !list && (!list || std::equal(ln.key_list.begin(), ln.key_list.end(), list));
-  auto chan = [&](uint32_t r) { return list ? list[r] : ch0 + r; }; // chain channel of row r
+  const bool hit = ln.cached && ln.key_epoch == ln.epoch && ln.key_version == chain->meta_version && ln.key.matches(sel);
   if (!hit) {
     ln.rows.clear();
     ln.any_pll = ln.any_anr = false;
     auto take = [&](uint32_t r) {
-      const bool is_pll = pll_build && chain->h_mode[chan(r)] == MSDR_MODE_SYNCAM;
-      const bool is_anr = chain->n_anr && chain->h_anr[chan(r)] != 0;
-      if (!list || is_pll || is_anr) ln.rows.push_back(r);
+      const bool is_pll = pll_build && chain->h_mode[sel.chan(r)] == MSDR_MODE_SYNCAM;
+      const bool is_anr = chain->n_anr && chain->h_anr[sel.chan(r)] != 0;
+      if (!sel.listed || is_pll || is_anr) ln.rows.push_back(r);
       ln.any_pll |= is_pll; ln.any_anr |= is_anr;
     };
     const std::vector<uint32_t> &lane = side_lane_channels(chain);
-    if (!list)
-      for (auto it = std::lower_bound(lane.begin(), lane.end(), ch0); it != lane.end() && *it < ch0 + nch; ++it) take(*it - ch0);
+    if (!sel.listed)
+      for (auto it = std::lower_bound(lane.begin(), lane.end(), sel.ch0); it != lane.end() && *it < sel.ch0 + sel.n; ++it) take(*it - sel.ch0);
     else if (!lane.empty())
-      for (uint32_t r = 0; r < nch; ++r) take(r);
-    std::stable_sort(ln.rows.begin(), ln.rows.end(), [&](uint32_t a, uint32_t b) { return chain->h_set[chan(a)] < chain->h_set[chan(b)]; });
-    ln.cached = true; ln.key_epoch = ln.epoch; ln.key_version = chain->meta_version; ln.key_ch0 = ch0; ln.key_nch = nch;
-    if (list) ln.key_list.assign(list, list + nch); else ln.key_list.clear();
+      for (uint32_t r = 0; r < sel.n; ++r) take(r);
+    std::stable_sort(ln.rows.begin(), ln.rows.end(), [&](uint32_t a, uint32_t b) { return chain->h_set[sel.chan(a)] < chain->h_set[sel.chan(b)]; });
+    ln.cached = true; ln.key_epoch = ln.epoch; ln.key_version = chain->meta_version;
+    ln.key.assign(sel);
   }
   if (ln.rows.empty()) return MSDR_OK;
   const uint32_t n = (uint32_t)ln.rows.size();
@@ -799,7 +943,7 @@ int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uin
   if (upload) {
     ln.chmap.resize(n); ln.kind.resize(n); ln.amode.resize(n);
     for (uint32_t i = 0; i < n; ++i) {
-      const uint32_t ch = chan(ln.rows[i]);
+      const uint32_t ch = sel.chan(ln.rows[i]);
       ln.chmap[i] = ch;
       const int md = chain->h_mode[ch];
       // demodulation kind of the row (Minimal-SDR.ino:589-628); 255 = the PLL demodulator takes the row
@@ -812,14 +956,14 @@ int syncam_lane_prepare(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uin
     CK(cudaMemcpyAsync(ln.d_kind, ln.kind.data(), n, cudaMemcpyHostToDevice, chain->stream));
     CK(cudaMemcpyAsync(ln.d_anr_mode, ln.amode.data(), n, cudaMemcpyHostToDevice, chain->stream));
   }
-  const uint32_t *d_chmap = list ? ln.d_chmap : nullptr;
-  CK(launch_gather_rows(ln.d_rows, d_chmap, n, ch0, chain->d_hist, chain->H, d_in, stride, ln.d_raw, L, chain->stream));
-  CK(launch_bq_words(0, ln.d_rows, d_chmap, n, ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
+  const uint32_t *d_chmap = sel.listed ? ln.d_chmap : nullptr;
+  CK(launch_gather_rows(ln.d_rows, d_chmap, n, sel.ch0, chain->d_hist, chain->H, d_in, stride, ln.d_raw, L, chain->stream));
+  CK(launch_bq_words(0, ln.d_rows, d_chmap, n, sel.ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
   chain->launches += 2;
   return MSDR_OK;
 }
 
-int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, bool list, int16_t *d_out, size_t stride, uint32_t L)
+int syncam_lane_finish(msdr_chain *chain, const Rows &sel, int16_t *d_out, size_t stride, uint32_t L)
 {
   msdr_chain::PllLane &ln = chain->pll;
   if (ln.rows.empty()) return MSDR_OK;
@@ -831,7 +975,7 @@ int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, bool list, int16_t *d_ou
     uint32_t i1 = i0;
     while (i1 < n && chain->h_set[ln.chmap[i1]] == sid) ++i1;
     const FirSet &fs = chain->sets[sid];
-    const int16_t *taps = chain->d_set_taps + (size_t)sid * 2 * MSDR_MAX_TAPS; // resident since upload_set: no copy, no wait per table
+    const int16_t *taps = chain->d_set_taps + (size_t)sid * 2 * MSDR_MAX_TAPS; // resident since upload_table: no copy, no wait per table
     CK(launch_fir_fast_q15(fs.T, taps, nullptr, nullptr, ln.d_I + i0 * Lp, ln.d_If + i0 * Lp, i1 - i0, (uint32_t)Lp, Lp, chain->stream));
     CK(launch_fir_fast_q15(fs.T, taps + MSDR_MAX_TAPS, nullptr, nullptr, ln.d_Q + i0 * Lp, ln.d_Qf + i0 * Lp, i1 - i0, (uint32_t)Lp, Lp, chain->stream));
     chain->launches += 2;
@@ -846,7 +990,7 @@ int syncam_lane_finish(msdr_chain *chain, uint32_t ch0, bool list, int16_t *d_ou
   CK(launch_biquad(ln.d_defs, audio, n, L, Lp, chain->stream));
   CK(launch_biquad(ln.d_defs + (size_t)n * 32, audio, n, L, Lp, chain->stream));
   CK(launch_scatter_rows(ln.d_rows, n, audio, Lp, d_out, stride, L, chain->stream));
-  CK(launch_bq_words(1, ln.d_rows, list ? ln.d_chmap : nullptr, n, ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
+  CK(launch_bq_words(1, ln.d_rows, sel.listed ? ln.d_chmap : nullptr, n, sel.ch0, chain->d_bq, chain->Cpad, ln.d_defs, chain->stream));
   chain->launches += 6;
   return MSDR_OK;
 }
@@ -871,18 +1015,18 @@ struct Choice {
   uint32_t shape = 0; // v4 (tc_ff): 0 post warps, 1 classic, 2 feed-forward helper warps, 3 two chain sets per SM
 };
 
-// The fused kernel for the range [ch0, ch0 + nch) (or the channel list[0 .. nch)) of NG channel groups on `sms` SMs, and the row plan
-// it runs from.
-int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, uint32_t NG, int sms, Choice &ch)
+// The fused kernel for the selection's NG channel groups on `sms` SMs, and the row plan it runs from.
+int choose_kernel(msdr_chain *chain, const Rows &sel, uint32_t NG, int sms, Choice &ch)
 {
   const int v = chain->variant;
-  if (list) {
+  const uint32_t nch = sel.n;
+  if (sel.listed) {
     // A channel list has no chain kernel v4 form (its chain warps own contiguous 32-channel groups): the time-folded kernel when its
     // group blocks fit one per SM, else the row-block kernels whatever the channel count.  The plan has one wave (sms = NG), and the
     // v6 group blocks are only asked for when the list's channel groups alone fit.
     const int v6_sms = std::max(1, sms - (int)chain->spare_sms);
     const bool want_v6 = !(v & (kNoV6 | kForceV5)) && ((v & kForceV6) || NG <= (uint32_t)v6_sms);
-    const int st = build_tc_plan(chain, 0, nch, list, NG, false, want_v6, &ch.plan);
+    const int st = build_tc_plan(chain, sel, NG, false, want_v6, &ch.plan);
     if (st != MSDR_OK) return st;
     const msdr_chain::TcPlan &pl = *ch.plan;
     if (pl.slots_v6 && ((v & kForceV6) || pl.n_gb <= (uint32_t)v6_sms)) ch.kernel = kV6;
@@ -904,7 +1048,7 @@ int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t 
       if (fs.users) kp_live = std::max(kp_live, kp_of_taps(fs.T));
     const uint32_t K = tc_window_words_kp(kp_live);
     if (chain_v5_config(K, smem_max) || chain_v5l_config(K, smem_max)) { // a plan with ONE wave: rows sorted by table over the range
-      const int st = build_tc_plan(chain, ch0, nch, nullptr, NG, false, false, &ch.plan);
+      const int st = build_tc_plan(chain, sel, NG, false, false, &ch.plan);
       if (st != MSDR_OK) return st;
       const msdr_chain::TcPlan &pl = *ch.plan;
       if (pl.ring_v5 || pl.ring_v5l) { // else no row-block form fits this window: the kernels below
@@ -919,7 +1063,7 @@ int choose_kernel(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t 
   const bool want_v6 = !(v & (kNoV6 | kV4Study)) && (nch <= 8192u || (v & kForceV6));
   // more channel groups than SMs: two chain sets per SM (waves of 2 x SMs groups)
   const bool want_dual = NG > (uint32_t)sms && !(v & kV4Study);
-  const int st = build_tc_plan(chain, ch0, nch, nullptr, (uint32_t)sms, want_dual, want_v6, &ch.plan);
+  const int st = build_tc_plan(chain, sel, (uint32_t)sms, want_dual, want_v6, &ch.plan);
   if (st != MSDR_OK) return st;
   const msdr_chain::TcPlan &pl = *ch.plan;
   if (pl.slots_v6 && ((v & kForceV6) || pl.n_gb <= (uint32_t)std::max(1, sms - (int)chain->spare_sms))) {
@@ -986,37 +1130,18 @@ int prof_dump(msdr_chain *chain, Kernel k, long long *d_prof, uint32_t g, uint32
   return MSDR_OK;
 }
 
-// Refuses a channel list with a channel outside the chain or listed twice (two rows would race on one channel's state).
-int check_list(msdr_chain *chain, const uint32_t *list, uint32_t n)
-{
-  if (chain->list_seen.size() != chain->C) { chain->list_seen.assign(chain->C, 0u); chain->list_stamp = 0; }
-  if (++chain->list_stamp == 0) { std::fill(chain->list_seen.begin(), chain->list_seen.end(), 0u); chain->list_stamp = 1; }
-  for (uint32_t i = 0; i < n; ++i) {
-    const uint32_t c = list[i];
-    if (c >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: channel " + std::to_string(c) + " is not in the chain");
-    if (chain->list_seen[c] == chain->list_stamp) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: channel " + std::to_string(c) + " is listed twice");
-    chain->list_seen[c] = chain->list_stamp;
-  }
-  return MSDR_OK;
-}
-
 // d_adc != NULL: the rows are raw ADC codes for the chain's front end.  Where the int16 input would run the row-block kernels and no
 // channel of the range is on the side lane (which gathers IF samples from `d_in`), the front end runs inside their converters; in
 // every other case K4 conditions the range into a scratch buffer first and the int16 path follows.  Both are bit-exact.
-// list != NULL (ch0 = 0): row r of d_in / d_adc / d_out is chain channel list[r] instead of ch0 + r.  ADC codes of a list always take
-// K4, which reads each row's front-end state through the plan's device copy of the list: a front end fused into the row-block list
-// kernels measured 0.96x of this composition (DESIGN.md §6).
-int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *list, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
-                 size_t stride, const uint16_t *d_adc)
+// Row r of d_in / d_adc / d_out is chain channel sel.chan(r).  ADC codes of a list always take K4, which reads each row's front-end
+// state through the plan's device copy of the list: a front end fused into the row-block list kernels measured 0.96x of this
+// composition (DESIGN.md §6).
+int update_range(msdr_chain *chain, const Rows &sel, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks, size_t stride, const uint16_t *d_adc)
 {
-  if (n_blocks == 0 || nch == 0) return MSDR_OK;
+  if (n_blocks == 0 || sel.n == 0) return MSDR_OK;
   const uint64_t L64 = (uint64_t)n_blocks * MSDR_BLOCK_SAMPLES;
-  if (list) {
-    const int st = check_list(chain, list, nch);
-    if (st != MSDR_OK) return st;
-  } else if (!range_ok(chain, ch0, nch)) {
-    return fail(chain, MSDR_ERR_ARGUMENT, "update: bad channel range");
-  }
+  int st = check_rows(chain, sel, true, "update");
+  if (st != MSDR_OK) return st;
   const void *src_rows = d_adc ? static_cast<const void *>(d_adc) : static_cast<const void *>(d_in);
   if (!src_rows || !d_out || L64 > stride || L64 > 0x7FFFFF00ull) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
   if (((uintptr_t)src_rows & 15u) || ((uintptr_t)d_out & 15u) || (stride & 7u))
@@ -1026,23 +1151,16 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
 
   int sms = 0;
   CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, chain->device));
-  const uint32_t NG = (nch + kGroup - 1) / kGroup;
+  const uint32_t NG = (sel.n + kGroup - 1) / kGroup;
   Choice ch;
-  int st = choose_kernel(chain, ch0, nch, list, NG, sms, ch);
-  if (st != MSDR_OK) return st;
+  if ((st = choose_kernel(chain, sel, NG, sms, ch)) != MSDR_OK) return st;
   const msdr_chain::TcPlan &pl = *ch.plan;
-  const bool fe_composed = d_adc && (list || (ch.kernel != kV5 && ch.kernel != kV5l) || side_lane_in_range(chain, ch0, nch));
+  const bool fe_composed = d_adc && (sel.listed || (ch.kernel != kV5 && ch.kernel != kV5l) || side_lane_in_range(chain, sel.ch0, sel.n));
   if (fe_composed) {
-    // K4 over the range or list into the scratch rows (same stride as `d_out`), then the int16 path reads them
-    const size_t need = (size_t)nch * stride;
-    if (need > chain->fe_if_samples) {
-      CK(cudaStreamSynchronize(chain->stream));
-      cudaFree(chain->d_fe_if);
-      chain->d_fe_if = nullptr; chain->fe_if_samples = 0;
-      CK(cudaMalloc(&chain->d_fe_if, need * sizeof(int16_t)));
-      chain->fe_if_samples = need;
-    }
-    CK(launch_frontend(d_adc, chain->d_fe_if, stride, nch, n_blocks, chain->d_fe + ch0, chain->fe_agc_max, chain->fe_agc_on, 0, chain->stream, pl.d_list));
+    // K4 over the selection into the scratch rows (same stride as `d_out`), then the int16 path reads them
+    if ((st = grow(chain, chain->d_fe_if, chain->fe_if_samples, (size_t)sel.n * stride)) != MSDR_OK) return st;
+    CK(launch_frontend(d_adc, chain->d_fe_if, stride, sel.n, n_blocks, chain->d_fe + sel.ch0, chain->fe_agc_max, chain->fe_agc_on, 0, chain->stream,
+                       pl.d_list));
     chain->launches++;
     d_in = chain->d_fe_if;
     d_adc = nullptr;
@@ -1050,7 +1168,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
 
   ChainParams p{};
   p.in = d_in; p.out = d_out; p.stride = stride;
-  p.C = nch; p.ch0 = ch0; p.Cpad = chain->Cpad; p.L = (uint32_t)L64; p.H = chain->H;
+  p.C = sel.n; p.ch0 = sel.ch0; p.Cpad = chain->Cpad; p.L = (uint32_t)L64; p.H = chain->H;
   p.hist = chain->d_hist; p.bq = chain->d_bq; p.mode = chain->d_mode; p.setid = chain->d_set;
   p.am_q31 = (chain->flags & MSDR_FLAG_AM_Q31) ? 1u : 0u;
   p.spare_sms = chain->spare_sms;
@@ -1078,13 +1196,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
     p.tc_ring = pl.rings[ch.shape]; p.tc_ff = ch.shape;
     p.NU = p.L / chain_v4_unit_samples();
     const size_t n_cnt = (size_t)NG * p.NU;
-    if (n_cnt > chain->tile_cnt_len) {
-      CK(cudaStreamSynchronize(chain->stream));
-      cudaFree(chain->d_tile_cnt);
-      chain->d_tile_cnt = nullptr; chain->tile_cnt_len = 0;
-      CK(cudaMalloc(&chain->d_tile_cnt, (n_cnt + 1024) * sizeof(int)));
-      chain->tile_cnt_len = n_cnt + 1024;
-    }
+    if ((st = grow(chain, chain->d_tile_cnt, chain->tile_cnt_len, n_cnt, 1024)) != MSDR_OK) return st;
     CK(cudaMemsetAsync(chain->d_ctrl, 0, 2 * sizeof(int), chain->stream));
     CK(cudaMemsetAsync(chain->d_tile_cnt, 0, n_cnt * sizeof(int), chain->stream));
     p.ctrl = chain->d_ctrl; p.tile_cnt = chain->d_tile_cnt;
@@ -1096,7 +1208,7 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
     if ((st = usage_resolve(chain)) != MSDR_OK) return st; // the event pair is reused: fold the previous update in first
     CK(cudaEventRecord(chain->ev0, chain->stream));
   }
-  if ((st = syncam_lane_prepare(chain, ch0, nch, list, d_in, stride, p.L)) != MSDR_OK) return st;
+  if ((st = syncam_lane_prepare(chain, sel, d_in, stride, p.L)) != MSDR_OK) return st;
   static const bool prof_on = getenv("MSDR_PROF") != nullptr; // developer aid: per-role cycle counters on stderr
   long long *d_prof = nullptr;
   if (prof_on) {
@@ -1114,9 +1226,9 @@ int update_range(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint32_t *
   chain->last_kernel = std::string("msdr::") + kNames[ch.kernel].ns + "::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; " +
                        (ch.kernel == kV4 ? kV4ShapeNames[ch.shape] : kNames[ch.kernel].form) + ")";
   if (p.fe) chain->last_kernel += "; front end fused into the converters";
-  if (list) chain->last_kernel += "; channel list";
+  if (sel.listed) chain->last_kernel += "; channel list";
   if (fe_composed) chain->last_kernel = "msdr::fe::frontend_kernel (front end), then " + chain->last_kernel;
-  if ((st = syncam_lane_finish(chain, ch0, list != nullptr, d_out, stride, p.L)) != MSDR_OK) return st;
+  if ((st = syncam_lane_finish(chain, sel, d_out, stride, p.L)) != MSDR_OK) return st;
   if (chain->timed) {
     CK(cudaEventRecord(chain->ev1, chain->stream));
     chain->usage_pending = true;
@@ -1133,7 +1245,7 @@ int msdr_chain_update_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch
                                    size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
-  return update_range(chain, ch0, nch, nullptr, d_in, d_out, n_blocks, stride, nullptr);
+  return update_range(chain, Rows{ch0, nch}, d_in, d_out, n_blocks, stride, nullptr);
 }
 
 int msdr_chain_update_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks,
@@ -1141,13 +1253,13 @@ int msdr_chain_update_list_device(msdr_chain *chain, const uint32_t *channels, u
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: NULL channel list");
-  return update_range(chain, 0, n, channels, d_in, d_out, n_blocks, stride, nullptr);
+  return update_range(chain, Rows{0, n, channels, true}, d_in, d_out, n_blocks, stride, nullptr);
 }
 
 int msdr_chain_update_device(msdr_chain *chain, const int16_t *d_in, int16_t *d_out, uint32_t n_blocks, size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
-  return msdr_chain_update_range_device(chain, 0, chain->C, d_in, d_out, n_blocks, stride);
+  return update_range(chain, Rows{0, chain->C}, d_in, d_out, n_blocks, stride, nullptr);
 }
 
 namespace {
@@ -1155,11 +1267,13 @@ namespace {
 // Host buffers: channels are cut into chunks that flow through a 3-slot device ring — H2D copy (stream copy_in),
 // fused kernel (chain stream), D2H copy (stream copy_out) — so PCIe traffic in both directions overlaps the kernels.
 // adc: `in` holds uint16 ADC codes (2 bytes a sample like int16 IF samples) for the chain's front end.
-// list != NULL: the rows of `in` / `out` are the n chain channels list[0 .. n), cut into chunks of the list instead of the chain.
-int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride, bool adc, const uint32_t *list = nullptr,
-                  uint32_t n = 0)
+// Row r of `in` / `out` is chain channel sel.chan(r); a list is cut into chunks of the list instead of the chain.
+int host_pipeline(msdr_chain *chain, const Rows &sel, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride, bool adc)
 {
-  const uint32_t rows = list ? n : chain->C;
+  if (sel.n == 0 || n_blocks == 0) return MSDR_OK;
+  int st = check_rows(chain, sel, true, "update"); // the whole selection before the first chunk is queued
+  if (st != MSDR_OK) return st;
+  const uint32_t rows = sel.n;
   const size_t L = (size_t)n_blocks * MSDR_BLOCK_SAMPLES;
   if (!in || !out || L > stride) return fail(chain, MSDR_ERR_ARGUMENT, "update: bad buffers / stride < n_blocks*128");
   if (chain->n_uninit) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update: some channels have no FIR bound (call msdr_fir_init_q15)");
@@ -1181,8 +1295,9 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
   nbk = std::min(nbk, n_blocks);
   const size_t Lc = (size_t)nbk * MSDR_BLOCK_SAMPLES; // device row pitch of a chunk
   const size_t slot_samples = (size_t)Cc * Lc;
-  int st = ensure_stage(chain, slot_samples * kSlots);
-  if (st != MSDR_OK) return st;
+  if ((st = grow(chain, chain->d_in, chain->in_samples, slot_samples * kSlots)) != MSDR_OK ||
+      (st = grow(chain, chain->d_out, chain->out_samples, slot_samples * kSlots)) != MSDR_OK)
+    return st;
   if (chain->pipe_ev.empty()) {
     chain->pipe_ev.resize(3 * kSlots);
     for (auto &ev : chain->pipe_ev) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
@@ -1205,11 +1320,7 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
       CK(cudaMemcpy2DAsync(din, Lc * 2, in + hoff, stride * 2, w, nc, cudaMemcpyHostToDevice, chain->copy_in));
       CK(cudaEventRecord(ev_h2d[slot], chain->copy_in));
       CK(cudaStreamWaitEvent(chain->stream, ev_h2d[slot], 0));
-      const uint16_t *dadc = reinterpret_cast<const uint16_t *>(din);
-      st = list ? (adc ? msdr_chain_update_adc_list_device(chain, list + c0, nc, dadc, dout, nb, Lc)
-                       : msdr_chain_update_list_device(chain, list + c0, nc, din, dout, nb, Lc))
-           : adc ? msdr_chain_update_adc_range_device(chain, c0, nc, dadc, dout, nb, Lc)
-                 : msdr_chain_update_range_device(chain, c0, nc, din, dout, nb, Lc);
+      st = update_range(chain, sel.sub(c0, nc), adc ? nullptr : din, dout, nb, Lc, adc ? reinterpret_cast<const uint16_t *>(din) : nullptr);
       if (st != MSDR_OK) return st;
       CK(cudaEventRecord(ev_k[slot], chain->stream));
       CK(cudaStreamWaitEvent(chain->copy_out, ev_k[slot], 0));
@@ -1227,18 +1338,14 @@ int host_pipeline(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n
 int msdr_chain_update(msdr_chain *chain, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
-  if (n_blocks == 0) return MSDR_OK;
-  return host_pipeline(chain, in, out, n_blocks, stride, false);
+  return host_pipeline(chain, Rows{0, chain->C}, in, out, n_blocks, stride, false);
 }
 
 int msdr_chain_update_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, const int16_t *in, int16_t *out, uint32_t n_blocks, size_t stride)
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_list: NULL channel list");
-  if (n == 0 || n_blocks == 0) return MSDR_OK;
-  const int st = check_list(chain, channels, n); // the whole list before the first chunk is queued
-  if (st != MSDR_OK) return st;
-  return host_pipeline(chain, in, out, n_blocks, stride, false, channels, n);
+  return host_pipeline(chain, Rows{0, n, channels, true}, in, out, n_blocks, stride, false);
 }
 
 // ---- ADC-code input: the front end of msdr_frontend.cu per chain channel, in front of the chain ------------------------------------
@@ -1246,55 +1353,23 @@ int msdr_chain_enable_frontend(msdr_chain *chain, float agc_start, float agc_max
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   CK(cudaSetDevice(chain->device));
-  CK(cudaStreamSynchronize(chain->stream));
   if (!chain->d_fe) CK(cudaMalloc(&chain->d_fe, (size_t)chain->C * sizeof(fe::State)));
+  int st = staging_wait(chain); // fe0 is the source of the copies below
+  if (st != MSDR_OK) return st;
   chain->fe_agc_start = agc_start; chain->fe_agc_max = agc_max; chain->fe_agc_on = agc_on ? 1 : 0;
-  fe::State s{};
-  s.agc_idx = fe::kAgcBuf;                // .ino:451
-  s.agc_val = agc_start;                  // .ino:104
-  s.mult = fe::amp_multiplier(agc_start); // .ino:385
-  std::vector<fe::State> h(chain->C, s);
-  CK(cudaMemcpy(chain->d_fe, h.data(), h.size() * sizeof(fe::State), cudaMemcpyHostToDevice));
-  CK(cudaDeviceSynchronize()); // legacy-stream copy vs the chain's non-blocking stream
-  return MSDR_OK;
+  chain->fe0 = fe::initial_state(agc_start);
+  if ((st = replicate(chain, chain->d_fe, sizeof(fe::State), chain->C, &chain->fe0)) != MSDR_OK) return st;
+  return staging_uploaded(chain);
 }
 
-/* AudioInputAnalog::init (input_adc.cpp:59-63): x1 = first reading << 14, y1 = 0 */
 int msdr_chain_frontend_preset(msdr_chain *chain, uint32_t ch0, uint32_t nch, uint16_t first_reading)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if (!range_ok(chain, ch0, nch)) return fail(chain, MSDR_ERR_ARGUMENT, "frontend_preset: bad channel range");
-  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "frontend_preset: call msdr_chain_enable_frontend first");
-  if (nch == 0) return MSDR_OK;
-  CK(cudaSetDevice(chain->device));
-  CK(cudaStreamSynchronize(chain->stream));
-  std::vector<fe::State> h(nch);
-  CK(cudaMemcpy(h.data(), chain->d_fe + ch0, nch * sizeof(fe::State), cudaMemcpyDeviceToHost));
-  for (auto &s : h) { s.hpf_x1 = (int32_t)((uint32_t)first_reading << 14); s.hpf_y1 = 0; }
-  CK(cudaMemcpy(chain->d_fe + ch0, h.data(), nch * sizeof(fe::State), cudaMemcpyHostToDevice));
-  CK(cudaDeviceSynchronize());
-  return MSDR_OK;
+  return chain ? frontend_preset(chain, Rows{ch0, nch}, first_reading) : MSDR_ERR_ARGUMENT;
 }
 
 int msdr_chain_frontend_preset_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, uint16_t first_reading)
 {
-  if (!chain) return MSDR_ERR_ARGUMENT;
-  if (!channels && n) return fail(chain, MSDR_ERR_ARGUMENT, "frontend_preset_list: NULL channel list");
-  for (uint32_t i = 0; i < n; ++i)
-    if (channels[i] >= chain->C) return fail(chain, MSDR_ERR_ARGUMENT, "frontend_preset_list: channel out of range");
-  if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "frontend_preset_list: call msdr_chain_enable_frontend first");
-  if (n == 0) return MSDR_OK;
-  CK(cudaSetDevice(chain->device));
-  uint32_t *d_list = nullptr;
-  CK(cudaMalloc(&d_list, (size_t)n * 4));
-  // pageable source: staged before the call returns; the stream order puts the preset after every update already queued
-  cudaError_t e = cudaMemcpyAsync(d_list, channels, (size_t)n * 4, cudaMemcpyHostToDevice, chain->stream);
-  if (e == cudaSuccess) e = launch_frontend_preset(chain->d_fe, d_list, n, first_reading, chain->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(chain->stream);
-  cudaFree(d_list);
-  if (e != cudaSuccess) return cuda_fail(chain, e, "frontend_preset_list");
-  chain->launches++;
-  return MSDR_OK;
+  return chain ? frontend_preset(chain, Rows{0, n, channels, true}, first_reading) : MSDR_ERR_ARGUMENT;
 }
 
 int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks,
@@ -1302,7 +1377,7 @@ int msdr_chain_update_adc_range_device(msdr_chain *chain, uint32_t ch0, uint32_t
 {
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
-  return update_range(chain, ch0, nch, nullptr, nullptr, d_out, n_blocks, stride, d_adc);
+  return update_range(chain, Rows{ch0, nch}, nullptr, d_out, n_blocks, stride, d_adc);
 }
 
 int msdr_chain_update_adc_device(msdr_chain *chain, const uint16_t *d_adc, int16_t *d_out, uint32_t n_blocks, size_t stride)
@@ -1316,7 +1391,7 @@ int msdr_chain_update_adc(msdr_chain *chain, const uint16_t *adc, int16_t *out, 
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (n_blocks == 0) return MSDR_OK;
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc: call msdr_chain_enable_frontend first");
-  return host_pipeline(chain, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true);
+  return host_pipeline(chain, Rows{0, chain->C}, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true);
 }
 
 int msdr_chain_update_adc_list_device(msdr_chain *chain, const uint32_t *channels, uint32_t n, const uint16_t *d_adc, int16_t *d_out,
@@ -1325,7 +1400,7 @@ int msdr_chain_update_adc_list_device(msdr_chain *chain, const uint32_t *channel
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_adc_list: NULL channel list");
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc_list: call msdr_chain_enable_frontend first");
-  return update_range(chain, 0, n, channels, nullptr, d_out, n_blocks, stride, d_adc);
+  return update_range(chain, Rows{0, n, channels, true}, nullptr, d_out, n_blocks, stride, d_adc);
 }
 
 int msdr_chain_update_adc_list(msdr_chain *chain, const uint32_t *channels, uint32_t n, const uint16_t *adc, int16_t *out, uint32_t n_blocks,
@@ -1334,10 +1409,7 @@ int msdr_chain_update_adc_list(msdr_chain *chain, const uint32_t *channels, uint
   if (!chain) return MSDR_ERR_ARGUMENT;
   if (n && !channels) return fail(chain, MSDR_ERR_ARGUMENT, "update_adc_list: NULL channel list");
   if (!chain->d_fe) return fail(chain, MSDR_ERR_NOT_INITIALISED, "update_adc_list: call msdr_chain_enable_frontend first");
-  if (n == 0 || n_blocks == 0) return MSDR_OK;
-  const int st = check_list(chain, channels, n); // the whole list before the first chunk is queued
-  if (st != MSDR_OK) return st;
-  return host_pipeline(chain, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true, channels, n);
+  return host_pipeline(chain, Rows{0, n, channels, true}, reinterpret_cast<const int16_t *>(adc), out, n_blocks, stride, true);
 }
 
 int msdr_chain_get_frontend_state(msdr_chain *chain, uint32_t ch, msdr_frontend_state *out)
@@ -1358,9 +1430,8 @@ int msdr_chain_set_frontend_state(msdr_chain *chain, uint32_t ch, const msdr_fro
   // agc_idx indexes the 25-entry history after a pre-decrement (Minimal-SDR.ino:481): anything outside 0..25 would be an out-of-bounds store
   if (in->agc_idx < 0 || in->agc_idx > fe::kAgcBuf) return fail(chain, MSDR_ERR_ARGUMENT, "set_frontend_state: agc_idx outside [0, 25]");
   CK(cudaSetDevice(chain->device));
-  CK(cudaStreamSynchronize(chain->stream));
-  CK(cudaMemcpy(chain->d_fe + ch, in, sizeof(*in), cudaMemcpyHostToDevice));
-  CK(cudaDeviceSynchronize());
+  CK(cudaMemcpyAsync(chain->d_fe + ch, in, sizeof(*in), cudaMemcpyHostToDevice, chain->stream));
+  CK(cudaStreamSynchronize(chain->stream)); // the caller may free `in` on return
   return MSDR_OK;
 }
 
@@ -1437,18 +1508,17 @@ int msdr_chain_set_state(msdr_chain *chain, uint32_t ch, const msdr_channel_stat
   const uint8_t sid = chain->h_set[ch];
   if (sid == 0xFF || chain->sets[sid].T != in->num_taps)
     return fail(chain, MSDR_ERR_ARGUMENT, "set_state: bind the FIR (msdr_fir_init_q15) with the same tap count first");
-  CK(cudaSetDevice(chain->device));
-  CK(cudaStreamSynchronize(chain->stream));
-  int st = msdr_chain_set_mode(chain, ch, 1, in->mode);
+  int st = set_mode(chain, Rows{ch, 1}, in->mode);
   if (st != MSDR_OK) return st;
   std::vector<int16_t> h(chain->H, 0);
   const uint32_t n = in->num_taps - 1;
   memcpy(h.data() + (chain->H - n), in->fir_history, n * sizeof(int16_t));
-  CK(cudaMemcpy(chain->d_hist + (size_t)ch * chain->H, h.data(), chain->H * sizeof(int16_t), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy2D(chain->d_bq + ch, (size_t)chain->Cpad * sizeof(int32_t), in->biquad_definition, sizeof(int32_t), sizeof(int32_t), kBqWords,
-                  cudaMemcpyHostToDevice));
-  CK(cudaMemcpy2D(chain->d_pll + ch, (size_t)chain->Cpad * sizeof(float), in->syncam_pll, sizeof(float), sizeof(float), 3, cudaMemcpyHostToDevice));
-  CK(cudaDeviceSynchronize()); // legacy-stream copies vs the chain's non-blocking stream
+  cudaStream_t s = chain->stream;
+  CK(cudaMemcpyAsync(chain->d_hist + (size_t)ch * chain->H, h.data(), chain->H * sizeof(int16_t), cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpy2DAsync(chain->d_bq + ch, (size_t)chain->Cpad * sizeof(int32_t), in->biquad_definition, sizeof(int32_t), sizeof(int32_t), kBqWords,
+                       cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpy2DAsync(chain->d_pll + ch, (size_t)chain->Cpad * sizeof(float), in->syncam_pll, sizeof(float), sizeof(float), 3, cudaMemcpyHostToDevice, s));
+  CK(cudaStreamSynchronize(s)); // `h` and the caller's `in` are read until the copies have run
   return MSDR_OK;
 }
 
@@ -1529,22 +1599,6 @@ int snap_parse_header(const void *buf, size_t bytes, SnapHeader &h, const char *
   return MSDR_OK;
 }
 
-// before writing the staging vectors again, the uploads that read them must have run
-int snap_wait(msdr_chain *chain)
-{
-  if (!chain->snap_ev) CK(cudaEventCreateWithFlags(&chain->snap_ev, cudaEventDisableTiming));
-  if (chain->snap_pending) CK(cudaEventSynchronize(chain->snap_ev));
-  chain->snap_pending = false;
-  return MSDR_OK;
-}
-
-int snap_uploaded(msdr_chain *chain)
-{
-  CK(cudaEventRecord(chain->snap_ev, chain->stream));
-  chain->snap_pending = true;
-  return MSDR_OK;
-}
-
 // header, tables and meta of channels [ch0, ch0+nch) into chain->snap_host (the first l.off[kOffHist] bytes of the snapshot)
 void snap_build_prefix(msdr_chain *chain, uint32_t ch0, uint32_t nch, const SnapLayout &l)
 {
@@ -1611,32 +1665,7 @@ int snap_begin(msdr_chain *chain, uint32_t ch0, uint32_t nch, size_t bytes, cons
   l = snap_layout(nch, chain->H, chain_sections(chain));
   if (bytes < l.total) return fail(chain, MSDR_ERR_ARGUMENT, "snapshot: buffer smaller than msdr_chain_snapshot_bytes");
   CK(cudaSetDevice(chain->device));
-  return snap_wait(chain);
-}
-
-// `count` copies of the element at host address `elem` (which outlives the copies) from d on: one upload, then doubling copies
-int replicate(msdr_chain *chain, void *d, size_t elem_bytes, size_t count, const void *elem)
-{
-  if (!count) return MSDR_OK;
-  uint8_t *p = static_cast<uint8_t *>(d);
-  CK(cudaMemcpyAsync(p, elem, elem_bytes, cudaMemcpyHostToDevice, chain->stream));
-  for (size_t done = 1; done < count; done *= 2)
-    CK(cudaMemcpyAsync(p + done * elem_bytes, p, std::min(done, count - done) * elem_bytes, cudaMemcpyDeviceToDevice, chain->stream));
-  return MSDR_OK;
-}
-
-const float kAnrLidx0 = 120.0f, kAnrNgamma0 = 0.001f; // Minimal-SDR.ino:715,718
-
-// initial LMS state (msdr_chain_set_anr's) for channels [ch0, ch0+n)
-int anr_initial(msdr_chain *chain, uint32_t ch0, uint32_t n)
-{
-  const size_t cp = (size_t)chain->Cpad * 4, w = (size_t)n * 4;
-  CK(cudaMemset2DAsync(chain->d_anr_d + ch0, cp, 0, w, 512, chain->stream));
-  CK(cudaMemset2DAsync(chain->d_anr_w + ch0, cp, 0, w, 64, chain->stream));
-  CK(cudaMemsetAsync(chain->d_anr_idx + ch0, 0, w, chain->stream));
-  int st = replicate(chain, chain->d_anr_lidx + ch0, 4, n, &kAnrLidx0);
-  if (st == MSDR_OK) st = replicate(chain, chain->d_anr_ngamma + ch0, 4, n, &kAnrNgamma0);
-  return st;
+  return staging_wait(chain);
 }
 
 // Restore channels [ch0, ch0+n) from snapshot channels [first, first+n).  `pre` is a host copy of the snapshot from byte 0 through
@@ -1679,77 +1708,55 @@ int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre
       if (idx < 0 || idx >= 512) return fail(chain, MSDR_ERR_ARGUMENT, "restore: ANR in_idx outside [0, 512)");
     }
   }
-  // table slots: the range gives its bindings back (release_sole_sets frees tables only it used), then the snapshot's tables are
-  // interned; count the live tables that would need before anything changes
-  auto same = [&](const FirSet &s, const SnapTable &t) {
-    return s.T == t.T && !memcmp(s.cI.data(), t.cI, t.T * 2) && !memcmp(s.cQ.data(), t.cQ, t.T * 2);
-  };
-  auto same_tab = [](const SnapTable &a, const SnapTable &b) { return a.T == b.T && !memcmp(a.cI, b.cI, a.T * 2) && !memcmp(a.cQ, b.cQ, a.T * 2); };
+  // table slots: the range gives its bindings back, then the snapshot's tables are interned in order, each bound to its channels at
+  // once; a dry run of that on a copy of the tables finds out whether they fit before anything changes
   {
-    uint32_t left[MSDR_MAX_FIR_SETS] = {0};
-    for (size_t s = 0; s < chain->sets.size(); ++s) left[s] = chain->sets[s].users;
+    std::vector<FirSet> sets = chain->sets;
     for (uint32_t c = ch0; c < ch0 + n; ++c)
-      if (chain->h_set[c] != kNoTable) left[chain->h_set[c]]--;
-    uint32_t live = 0;
-    for (size_t s = 0; s < chain->sets.size(); ++s) live += left[s] > 0;
+      if (chain->h_set[c] != kNoTable) sets[chain->h_set[c]].users--;
+    bool fresh;
     for (uint32_t k = 0; k < h.n_tables; ++k) {
       if (!used[k]) continue;
-      bool found = false;
-      for (size_t s = 0; s < chain->sets.size() && !found; ++s) found = left[s] > 0 && same(chain->sets[s], tab[k]);
-      for (uint32_t j = 0; j < k && !found; ++j) found = used[j] && same_tab(tab[j], tab[k]);
-      live += !found;
+      const int id = find_or_add_table(sets, tab[k].T, tab[k].cI, tab[k].cQ, &fresh);
+      if (id < 0) return fail(chain, MSDR_ERR_NOMEM, "restore: more than MSDR_MAX_FIR_SETS distinct FIR tables in one chain");
+      sets[id].users += used[k];
     }
-    if (live > MSDR_MAX_FIR_SETS) return fail(chain, MSDR_ERR_NOMEM, "restore: more than MSDR_MAX_FIR_SETS distinct FIR tables in one chain");
   }
 
   // ---- from here on the chain changes
   CK(cudaSetDevice(chain->device));
-  if ((st = snap_wait(chain)) != MSDR_OK) return st;
-  release_sole_sets(chain, [&](auto &&f) { for (uint32_t c = ch0; c < ch0 + n; ++c) f(c); });
-  for (uint32_t c = ch0; c < ch0 + n; ++c)
-    if (chain->h_set[c] != kNoTable) { chain->sets[chain->h_set[c]].users--; chain->h_set[c] = kNoTable; chain->n_uninit++; }
-  uint8_t map[MSDR_MAX_FIR_SETS];
-  chain->snap_taps.resize((size_t)MSDR_MAX_FIR_SETS * 2 * MSDR_MAX_TAPS);
-  for (uint32_t k = 0; k < h.n_tables; ++k) {
-    if (!used[k]) continue;
-    const SnapTable &t = tab[k];
-    size_t slot = chain->sets.size();
-    for (size_t s = 0; s < chain->sets.size() && slot == chain->sets.size(); ++s)
-      if (chain->sets[s].users > 0 && same(chain->sets[s], t)) slot = s;
-    if (slot == chain->sets.size()) { // a new table: first free slot, uploaded from the staging vectors
-      for (size_t s = 0; s < chain->sets.size(); ++s)
-        if (chain->sets[s].users == 0) { slot = s; break; }
-      if (slot == chain->sets.size()) chain->sets.emplace_back();
-      FirSet &fs = chain->sets[slot];
-      fs.T = t.T;
-      fs.cI.assign(t.cI, t.cI + t.T);
-      fs.cQ.assign(t.cQ, t.cQ + t.T);
-      int16_t *tp = chain->snap_taps.data() + slot * 2 * MSDR_MAX_TAPS;
-      std::copy(t.cI, t.cI + t.T, tp);
-      std::copy(t.cQ, t.cQ + t.T, tp + MSDR_MAX_TAPS);
-      CK(cudaMemcpyAsync(chain->d_set_taps + slot * 2 * MSDR_MAX_TAPS, tp, 2 * MSDR_MAX_TAPS * 2, cudaMemcpyHostToDevice, chain->stream));
+  if ((st = staging_wait(chain)) != MSDR_OK) return st;
+  unbind_rows(chain, Rows{ch0, n});
+  {
+    uint32_t at[MSDR_MAX_FIR_SETS + 1] = {0}; // the channels grouped by snapshot table: table k's are by_table[at[k] .. at[k+1])
+    for (uint32_t k = 0; k < h.n_tables; ++k) at[k + 1] = at[k] + used[k];
+    std::vector<uint32_t> &by_table = chain->snap_rows;
+    by_table.resize(at[h.n_tables]);
+    uint32_t fill[MSDR_MAX_FIR_SETS];
+    std::copy(at, at + MSDR_MAX_FIR_SETS, fill);
+    for (uint32_t i = 0; i < n; ++i)
+      if (meta[4 * i + 1] != kNoTable) by_table[fill[meta[4 * i + 1]]++] = ch0 + i;
+    for (uint32_t k = 0; k < h.n_tables; ++k) {
+      if (!used[k]) continue;
+      const int id = intern_table(chain, tab[k].T, tab[k].cI, tab[k].cQ);
+      if (id < 0) return id;
+      bind_rows(chain, Rows{0, used[k], by_table.data() + at[k], true}, (uint32_t)id);
     }
-    chain->sets[slot].users += used[k]; // counted at once: an identical later entry finds this slot
-    map[k] = (uint8_t)slot;
   }
-  // host mirrors, then the device copies of mode and table id
+  if ((st = upload_bindings(chain, Rows{ch0, n})) != MSDR_OK) return st;
+  // host mirrors, then the device copy of the modes
   if (has_anr && chain->h_anr.empty()) chain->h_anr.assign(chain->C, 0);
   std::vector<uint8_t> &hb = chain->snap_host;
-  hb.resize(2 * (size_t)n);
+  hb.resize(n);
   for (uint32_t i = 0; i < n; ++i) {
     const uint8_t *m = meta + 4 * i;
     const uint32_t c = ch0 + i;
-    chain->h_mode[c] = m[0];
-    if (m[1] != kNoTable) { chain->h_set[c] = map[m[1]]; chain->n_uninit--; }
+    chain->h_mode[c] = hb[i] = m[0];
     if (!chain->h_anr.empty()) { chain->n_anr += (m[2] != 0) - (chain->h_anr[c] != 0); chain->h_anr[c] = m[2]; }
-    hb[i] = chain->h_mode[c];
-    hb[n + i] = chain->h_set[c];
   }
-  chain->meta_version++;
   chain->pll.dirty = true; chain->pll.epoch++;
   cudaStream_t s = chain->stream;
   CK(cudaMemcpyAsync(chain->d_mode + ch0, hb.data(), n, cudaMemcpyHostToDevice, s));
-  CK(cudaMemcpyAsync(chain->d_set + ch0, hb.data() + n, n, cudaMemcpyHostToDevice, s));
 
   // state sections: one (2D) copy each; the snapshot side has pitch nch, the chain side Cpad
   const size_t H = chain->H, Hs = h.hist_len, m = std::min(H, Hs), cp = (size_t)chain->Cpad * 4, sp = (size_t)h.nch * 4, w = (size_t)n * 4;
@@ -1769,11 +1776,7 @@ int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre
       CK(cudaMalloc(&chain->d_fe, (size_t)chain->C * sizeof(fe::State)));
       chain->fe_agc_start = h.agc_start; chain->fe_agc_max = h.agc_max; chain->fe_agc_on = h.agc_on ? 1 : 0;
     }
-    fe::State &s0 = chain->snap_fe0;
-    s0 = fe::State{};
-    s0.agc_idx = fe::kAgcBuf;                          // .ino:451
-    s0.agc_val = chain->fe_agc_start;                  // .ino:104
-    s0.mult = fe::amp_multiplier(chain->fe_agc_start); // .ino:385
+    const fe::State &s0 = chain->fe0 = fe::initial_state(chain->fe_agc_start);
     if (fe_new) st = replicate(chain, chain->d_fe, sizeof(fe::State), chain->C, &s0);
     if (st == MSDR_OK && has_fe)
       CK(cudaMemcpyAsync(chain->d_fe + ch0, src + h.off[kOffFe] + (size_t)first * sizeof(fe::State), (size_t)n * sizeof(fe::State), kind, s));
@@ -1782,12 +1785,7 @@ int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre
     if (st != MSDR_OK) return st;
   }
 
-  if (has_anr && !chain->d_anr_d) { // LMS arrays on first need, as msdr_chain_set_anr allocates them; every channel starts at the initial state
-    const size_t cpb = (size_t)chain->Cpad * 4;
-    CK(cudaMalloc(&chain->d_anr_d, 512 * cpb)); CK(cudaMalloc(&chain->d_anr_w, 64 * cpb));
-    CK(cudaMalloc(&chain->d_anr_lidx, cpb)); CK(cudaMalloc(&chain->d_anr_ngamma, cpb)); CK(cudaMalloc(&chain->d_anr_idx, cpb));
-    if ((st = anr_initial(chain, 0, chain->Cpad)) != MSDR_OK) return st;
-  }
+  if (has_anr && (st = anr_alloc(chain)) != MSDR_OK) return st;
   if (has_anr) {
     CK(cudaMemcpy2DAsync(chain->d_anr_d + ch0, cp, src + h.off[kOffAnrD] + 4 * (size_t)first, sp, w, 512, kind, s));
     CK(cudaMemcpy2DAsync(chain->d_anr_w + ch0, cp, src + h.off[kOffAnrW] + 4 * (size_t)first, sp, w, 64, kind, s));
@@ -1797,7 +1795,7 @@ int snap_restore(msdr_chain *chain, uint32_t ch0, const uint8_t *pre, size_t pre
   } else if (chain->d_anr_d) {
     if ((st = anr_initial(chain, ch0, n)) != MSDR_OK) return st;
   }
-  return snap_uploaded(chain);
+  return staging_uploaded(chain);
 }
 
 } // namespace
@@ -1831,7 +1829,7 @@ int msdr_chain_snapshot_device(msdr_chain *chain, uint32_t ch0, uint32_t nch, vo
   uint8_t *d = static_cast<uint8_t *>(d_buf);
   CK(cudaMemcpyAsync(d, chain->snap_host.data(), chain->snap_host.size(), cudaMemcpyHostToDevice, chain->stream));
   if ((st = snap_copy_state_out(chain, ch0, nch, d, l, cudaMemcpyDeviceToDevice)) != MSDR_OK) return st;
-  return snap_uploaded(chain);
+  return staging_uploaded(chain);
 }
 
 int msdr_chain_restore(msdr_chain *chain, uint32_t ch0, const void *buf, size_t bytes, uint32_t first, uint32_t n)

@@ -109,21 +109,22 @@ __global__ void frontend_kernel(const Params p)
   if (active) p.state[srow] = s;
 }
 
-// AudioInputAnalog::init (input_adc.cpp:59-63) for the states state[channels[i]], i < n: x1 = first reading << 14, y1 = 0
-__global__ void preset_kernel(State *state, const uint32_t *channels, uint32_t n, int32_t x1)
+// AudioInputAnalog::init (input_adc.cpp:59-63) for the states state[channels[i]] (channels == NULL: state[ch0 + i]), i < n:
+// x1 = first reading << 14, y1 = 0
+__global__ void preset_kernel(State *state, const uint32_t *channels, uint32_t ch0, uint32_t n, int32_t x1)
 {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  State &s = state[channels[i]];
+  State &s = state[channels ? channels[i] : ch0 + i];
   s.hpf_x1 = x1;
   s.hpf_y1 = 0;
 }
 
 } // namespace fe
 
-cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t n, uint16_t first_reading, cudaStream_t s)
+cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t ch0, uint32_t n, uint16_t first_reading, cudaStream_t s)
 {
-  fe::preset_kernel<<<(n + 255) / 256, 256, 0, s>>>(state, channels, n, (int32_t)((uint32_t)first_reading << 14));
+  fe::preset_kernel<<<(n + 255) / 256, 256, 0, s>>>(state, channels, ch0, n, (int32_t)((uint32_t)first_reading << 14));
   return cudaGetLastError();
 }
 
@@ -191,13 +192,7 @@ int msdr_frontend_create(msdr_frontend **out, int device, uint32_t n_channels, f
   if (e == cudaSuccess) e = cudaMalloc(&fe->d_state, (size_t)n_channels * sizeof(msdr::fe::State));
   if (e != cudaSuccess) { g_fe_error = std::string("frontend_create: ") + cudaGetErrorString(e); delete fe; return MSDR_ERR_CUDA; }
   fe->stream = fe->own_stream;
-  std::vector<msdr::fe::State> h(n_channels);
-  for (auto &s : h) {
-    s = msdr::fe::State{};
-    s.agc_idx = msdr::fe::kAgcBuf;                    // .ino:451
-    s.agc_val = agc_start;                            // .ino:104
-    s.mult = msdr::fe::amp_multiplier(agc_start);     // .ino:385
-  }
+  std::vector<msdr::fe::State> h(n_channels, msdr::fe::initial_state(agc_start));
   e = cudaMemcpy(fe->d_state, h.data(), h.size() * sizeof(msdr::fe::State), cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaDeviceSynchronize(); // legacy-stream copy vs this object's non-blocking stream
   if (e != cudaSuccess) { g_fe_error = std::string("frontend_create: ") + cudaGetErrorString(e); cudaFree(fe->d_state); delete fe; return MSDR_ERR_CUDA; }
@@ -234,14 +229,9 @@ int msdr_frontend_synchronize(msdr_frontend *fe)
 int msdr_frontend_preset(msdr_frontend *fe, uint32_t ch0, uint32_t nch, uint16_t first_reading)
 {
   if (!fe || (uint64_t)ch0 + nch > fe->C) return fe_fail(fe, MSDR_ERR_ARGUMENT, "frontend_preset: bad channel range");
-  FCK(cudaSetDevice(fe->device));
-  FCK(cudaStreamSynchronize(fe->stream));
-  std::vector<msdr::fe::State> h(nch);
   if (nch == 0) return MSDR_OK;
-  FCK(cudaMemcpy(h.data(), fe->d_state + ch0, nch * sizeof(msdr::fe::State), cudaMemcpyDeviceToHost));
-  for (auto &s : h) { s.hpf_x1 = (int32_t)((uint32_t)first_reading << 14); s.hpf_y1 = 0; }
-  FCK(cudaMemcpy(fe->d_state + ch0, h.data(), nch * sizeof(msdr::fe::State), cudaMemcpyHostToDevice));
-  FCK(cudaDeviceSynchronize()); // the copies ran in the legacy stream; this object's stream is non-blocking
+  FCK(cudaSetDevice(fe->device));
+  FCK(msdr::launch_frontend_preset(fe->d_state, nullptr, ch0, nch, first_reading, fe->stream));
   return MSDR_OK;
 }
 

@@ -36,6 +36,16 @@ __host__ __device__ inline int32_t amp_multiplier(float n) // AudioAmplifier::ga
 #endif
 }
 
+// a channel before its first block: high-pass at rest, empty AGC history, gain agc_start
+inline State initial_state(float agc_start)
+{
+  State s{};
+  s.agc_idx = kAgcBuf;                // .ino:451
+  s.agc_val = agc_start;              // .ino:104
+  s.mult = amp_multiplier(agc_start); // .ino:385
+  return s;
+}
+
 // ARMv7E-M SSUB16 (sets APSR.GE[1:0] / [3:2] when the low / high halfword difference is >= 0) and SEL (bytes of `a` where GE is set)
 __device__ __forceinline__ uint32_t ssub16(int a, int b, uint32_t &ge)
 {

@@ -10,6 +10,7 @@ namespace fe { struct State; } // msdr_frontend.cuh
 
 constexpr int kGroup = 32;            // channels per work group (one biquad lane each)
 constexpr int kBqWords = 64;          // 2 objects x 4 stages x 8 words (filter_biquad.h:152)
+constexpr float kAnrLidx0 = 120.0f, kAnrNgamma0 = 0.001f; // initial LMS leak index and noise gain (Minimal-SDR.ino:715,718)
 
 // taps per polyphase sub-filter, padded: KP = roundup4(T/2 + 1)
 inline __host__ __device__ uint32_t kp_of_taps(uint32_t T) { return ((T / 2u + 1u) + 3u) & ~3u; }
@@ -68,8 +69,9 @@ bool chain_v4_config(uint32_t K, int smem_max, uint32_t rings[4]);
 // K4 (msdr_frontend.cu) over C rows: raw codes -> conditioned int16 IF samples; state = the first row's front-end state, or with
 // map != NULL the state array that row r indexes at map[r] (the rows' codes and outputs stay row r).
 // sms > 0 packs the channel groups into about that many CTAs.
-// launch_frontend_preset: hpf_x1 = first_reading << 14, hpf_y1 = 0 in state[channels[i]] for the n device-resident channels.
-cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t n, uint16_t first_reading, cudaStream_t s);
+// launch_frontend_preset: hpf_x1 = first_reading << 14, hpf_y1 = 0 in state[channels[i]] for the n device-resident channels, or with
+// channels == NULL in state[ch0 + i].
+cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t ch0, uint32_t n, uint16_t first_reading, cudaStream_t s);
 cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, uint32_t C, uint32_t n_blocks, fe::State *state, float agc_max,
                             int agc_on, int sms, cudaStream_t s, const uint32_t *map = nullptr);
 // row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config (0 = does not fit);
