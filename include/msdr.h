@@ -195,8 +195,8 @@ int msdr_snapshot_info(const void *header, size_t bytes, uint32_t *n_channels, u
 /* Options.  "variant" selects the shape of the fused kernel for studies and cross-checks (all shapes are bit-exact, DESIGN.md 6):
  *   0    default, by channel count: the time-folded kernel (msdr_chain_v6.cu) up to one 32-channel group block per SM; tensor-core
  *        FIR producers (tcgen05 kind::i8) + pinned biquad chains (msdr_chain_v4.cu: feed-forward helper warps up to 148 channel
- *        groups, two chain sets per SM beyond) up to one wave of those (9472 channels on 148 SMs); the row-block kernels
- *        (msdr_chain_v5.cu / v5l.cu) from there
+ *        groups, two chain sets per SM beyond) up to one wave of those (9472 channels on 148 SMs); the row-block kernel
+ *        (msdr_chain_v5.cu, whole tiles, or half tiles for the 256-tap window) from there
  *   16384  never the time-folded kernel;  65536  the time-folded kernel for any channel count;  +2 there: feed-forward products as DFMA
  *   8192   never the row-block kernel;    4096   the row-block kernel for any channel count;    32768  its half-tile form for any window
  *          (+1, +2, +4, +8, +12 there: the stage's products as IMAD.WIDE instead of IMAD.HI (the half-tile form: the other way round) /

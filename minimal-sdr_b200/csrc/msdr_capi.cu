@@ -101,8 +101,8 @@ struct msdr_chain {
     RowsKey sel;
     uint32_t sms = 0, W = 0, K = 0, rings[4] = {0, 0, 0, 0}, n_rb = 0, n_waves = 0;
     bool want_dual = false, want_v6 = false, dual = false;
-    uint32_t ring_v5 = 0;  // msdr_chain_v5.cu: operand ring depth, 0 = the window does not fit that kernel
-    uint32_t ring_v5l = 0; // msdr_chain_v5l.cu (half-tile hand-offs, for the 256-tap window)
+    uint32_t ring_v5 = 0;  // msdr_chain_v5.cu, whole-tile form: operand ring depth, 0 = the window does not fit that form
+    uint32_t ring_v5l = 0; // its half-tile form (for the 256-tap window)
     uint32_t slots_v6 = 0, n_gb = 0; // msdr_chain_v6.cu: sub-tile slots (0 = the window does not fit), group blocks of 32 same-table rows
     uint32_t *d_rowmap32 = nullptr;
     uint4 *d_rb32 = nullptr;
@@ -761,8 +761,8 @@ int build_tc_plan(msdr_chain *chain, const Rows &sel, uint32_t sms, bool want_du
   pl.version = chain->meta_version; pl.sel.assign(sel); pl.sms = sms; pl.want_dual = want_dual; pl.want_v6 = want_v6;
   std::copy(rings, rings + 4, pl.rings);
   pl.K = K;
-  pl.ring_v5 = chain_v5_config(K, smem_max);
-  pl.ring_v5l = chain_v5l_config(K, smem_max);
+  pl.ring_v5 = chain_v5_config(K, smem_max, false);
+  pl.ring_v5l = chain_v5_config(K, smem_max, true);
   pl.slots_v6 = want_v6 ? chain_v6_config(K, smem_max) : 0u;
   pl.dual = want_dual && pl.rings[3] != 0;
   const uint32_t W = pl.W = sms * (pl.dual ? 2u : 1u);
@@ -1047,7 +1047,7 @@ int choose_kernel(msdr_chain *chain, const Rows &sel, uint32_t NG, int sms, Choi
     for (const FirSet &fs : chain->sets)
       if (fs.users) kp_live = std::max(kp_live, kp_of_taps(fs.T));
     const uint32_t K = tc_window_words_kp(kp_live);
-    if (chain_v5_config(K, smem_max) || chain_v5l_config(K, smem_max)) { // a plan with ONE wave: rows sorted by table over the range
+    if (chain_v5_config(K, smem_max, false) || chain_v5_config(K, smem_max, true)) { // a plan with ONE wave: rows sorted by table over the range
       const int st = build_tc_plan(chain, sel, NG, false, false, &ch.plan);
       if (st != MSDR_OK) return st;
       const msdr_chain::TcPlan &pl = *ch.plan;
@@ -1220,8 +1220,8 @@ int update_range(msdr_chain *chain, const Rows &sel, const int16_t *d_in, int16_
   switch (ch.kernel) {
   case kV6: CK(launch_chain_v6(p, chain->stream, chain->variant, std::max(1, sms - (int)chain->spare_sms), &chain->last_info)); break;
   case kV4: CK(launch_chain_v4(p, chain->stream, chain->variant, &chain->last_info)); break;
-  case kV5: CK(launch_chain_v5(p, chain->stream, chain->variant, sms, &chain->last_info)); break;
-  case kV5l: CK(launch_chain_v5l(p, chain->stream, chain->variant, sms, &chain->last_info)); break;
+  case kV5:
+  case kV5l: CK(launch_chain_v5(p, chain->stream, chain->variant, sms, ch.kernel == kV5l, &chain->last_info)); break;
   }
   chain->last_kernel = std::string("msdr::") + kNames[ch.kernel].ns + "::chain_kernel (fused mix + tensor-core FIR pair + demod + biquad cascade; " +
                        (ch.kernel == kV4 ? kV4ShapeNames[ch.shape] : kNames[ch.kernel].form) + ")";

@@ -1,6 +1,5 @@
-// msdr_chain_v5_common.cuh — helpers shared by the row-block kernels (msdr_chain_v5.cu: windows up to 128 words, msdr_chain_v5l.cu: the
-// 256-tap window): epilogue drain and demodulation on registers, the biquad tile loop, the developer profile, the front end of the
-// ADC-code input.
+// msdr_chain_v5_common.cuh — helpers of the row-block kernel (msdr_chain_v5.cu, whole- and half-tile forms): epilogue drain and
+// demodulation on registers, the biquad tile loop, the developer profile, the front end of the ADC-code input.
 #pragma once
 #include "msdr_chain_common.cuh"
 #include "msdr_frontend.cuh"

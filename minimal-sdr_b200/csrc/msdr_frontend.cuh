@@ -1,5 +1,5 @@
 // msdr_frontend.cuh — the front-end arithmetic (SURVEY 8f rank 1), shared by K4 (msdr_frontend.cu) and the ADC-code instantiations of
-// the row-block chain kernels (msdr_chain_v5.cu, msdr_chain_v5l.cu):
+// the row-block chain kernel (msdr_chain_v5.cu, both forms):
 //   raw unsigned ADC codes -> 1-pole DC-blocking high-pass in S1.30 (AudioInputAnalog::update, input_adc.cpp:198-212)
 //   -> AudioAmplifier gain with SSAT16 (mixer.cpp:34-47,134-159, mixer.h:75-79) -> int16 IF samples,
 //   and per 128-sample block the AGC of the sketch (Minimal-SDR.ino:445-515): block maximum of |x| through the halfword SIMD

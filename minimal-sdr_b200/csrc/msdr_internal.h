@@ -74,18 +74,16 @@ bool chain_v4_config(uint32_t K, int smem_max, uint32_t rings[4]);
 cudaError_t launch_frontend_preset(fe::State *state, const uint32_t *channels, uint32_t ch0, uint32_t n, uint16_t first_reading, cudaStream_t s);
 cudaError_t launch_frontend(const uint16_t *adc, int16_t *out, size_t stride, uint32_t C, uint32_t n_blocks, fe::State *state, float agc_max,
                             int agc_on, int sms, cudaStream_t s, const uint32_t *map = nullptr);
-// row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config (0 = does not fit);
+// row-block kernel for many channels (msdr_chain_v5.cu): p.n_items = number of row blocks, p.tc_ring from chain_v5_config of the same
+// form (0 = does not fit).  half_tile: the form with half-tile hand-offs, for windows too long for whole tiles (256 taps).
 // p.fe != NULL selects the ADC-code instantiation (default biquad form only), p.chlist != NULL the channel-list one (the same)
-cudaError_t launch_chain_v5(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
-uint32_t chain_v5_config(uint32_t K, int smem_max);
+cudaError_t launch_chain_v5(const ChainParams &p, cudaStream_t stream, int variant, int sms, bool half_tile, ChainLaunchInfo *info);
+uint32_t chain_v5_config(uint32_t K, int smem_max, bool half_tile);
 // pinned 32-channel group blocks with the tile rows folded over time (msdr_chain_v6.cu): p.tc_rowmap = [n_items][32] rows,
 // p.tc_rb[i].x / .y = the tables of its two half blocks, p.tc_ring = sub-tile slots from chain_v6_config (0 = the window does not fit)
 cudaError_t launch_chain_v6(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
 uint32_t chain_v6_config(uint32_t K, int smem_max);
 uint32_t chain_v6_group_rows();
-// the same kernel with half-tile hand-offs for windows too long for it (256 taps; msdr_chain_v5l.cu)
-cudaError_t launch_chain_v5l(const ChainParams &p, cudaStream_t stream, int variant, int sms, ChainLaunchInfo *info);
-uint32_t chain_v5l_config(uint32_t K, int smem_max);
 
 // stage-level kernels on device buffers
 cudaError_t launch_mix_fs4(const int16_t *in, int16_t *I, int16_t *Q, uint32_t rows, uint32_t n, size_t stride, cudaStream_t s);

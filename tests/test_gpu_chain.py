@@ -170,7 +170,7 @@ def test_inplace_coefficient_rewrite_and_mode_change(msdr, orc, K):
 @pytest.mark.parametrize("variant", [0, 4096, 4097])
 def test_long_taps_256(msdr, orc, K, variant):
     """BASELINE config 4 shape: 255 taps + one zero (arm_fir_init_q15.c:55-64), 256-tap delay line.  variant 0: the chain kernel (few
-    channels); 4096 / 4097: the row-block kernel in its half-tile form for the long window (msdr_chain_v5l.cu), both stage forms."""
+    channels); 4096 / 4097: the row-block kernel in its half-tile form for the long window (msdr_chain_v5.cu), both stage forms."""
     rng = np.random.default_rng(44)
     modes = [AM, USB, LSB, CW] * 5
     c255 = rng.integers(-600, 600, 255).astype(np.int16)

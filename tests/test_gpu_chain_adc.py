@@ -1,5 +1,5 @@
-"""Receive chain from raw ADC codes (msdr_chain_update_adc*): the front end fused into the converters of the row-block kernels
-(csrc/msdr_chain_v5.cu, msdr_chain_v5l.cu), or the front-end kernel followed by the int16 path.  Every comparison is byte for byte
+"""Receive chain from raw ADC codes (msdr_chain_update_adc*): the front end fused into the converters of the row-block kernel
+(csrc/msdr_chain_v5.cu, both forms), or the front-end kernel followed by the int16 path.  Every comparison is byte for byte
 against the CPU oracles run one after the other: the front end (frontend_lib.Orc) feeding the chain (oracle_lib)."""
 import ctypes as C
 

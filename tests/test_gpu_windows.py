@@ -51,7 +51,7 @@ def history(max_taps):
 
 # ---- the windows and what fits them -----------------------------------------------------------------------------------------
 # Which kernels fit each window (in words): what chain_v6_config, chain_v4_config (its rings: post-warp, classic, helper-warp, two
-# sets), chain_v5_config and chain_v5l_config (csrc/msdr_chain_v*.cu) return for that window with the B200's opt-in shared memory of
+# sets) and chain_v5_config in both forms (csrc/msdr_chain_v*.cu) return for that window with the B200's opt-in shared memory of
 # 232 448 bytes per block, evaluated on the host from the same sources.  The cases below check on the device that update_range picks
 # accordingly: a change of a shared-memory budget that moves a fit fails them, and this table changes with it.
 # taps: the tables of a chain in that window, the upper edge (the longest) first: both edges of the window, every padding class

@@ -8,7 +8,8 @@ mkdir -p variants
 NV="/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC --expt-relaxed-constexpr"
 $NV "$@" -c -o variants/${file%.cu}_$tag.o $file
 objs=""
-for f in msdr_chain_v3 msdr_chain_v4 msdr_chain_v5 msdr_chain_v5l msdr_chain_v6 msdr_fir_tc msdr_frontend msdr_anr msdr_syncam msdr_stage_kernels msdr_capi; do
+for f in $(sed -n 's/^SRCS *:= *//p' Makefile); do # the library's sources, as the Makefile lists them
+  f=${f%.cu}
   if [ "$f.cu" = "$file" ]; then objs="$objs variants/${f}_$tag.o"; else objs="$objs $f.o"; fi
 done
 /usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -shared -o variants/libmsdr_$tag.so $objs
